@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- k-mers/s over insert + traverse (the timed region of kmer_hash.cpp:129-137).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: empty table ->
 insert every k-mer + find the start nodes -> walk every contig -> contig text materialised.
@@ -14,6 +14,9 @@ One JSON line on stdout (rank 0); see README/DESIGN.md for the keys.  `value` ha
 records resident in HBM when the clock starts (as the reference has them resident in host RAM);
 `e2e` runs the same step through the host-buffer C ABI calls (kh_insert_pairs / kh_assemble) with
 the H2D of the records and the D2H of the contigs inside the timed region.
+
+--dump-outputs DIR writes what the last timed step of the main workload produced (see dump_outputs) as .npy files, so
+that two builds can be compared output for output: the inputs are generated from a fixed seed.
 """
 from __future__ import annotations
 
@@ -77,6 +80,41 @@ def alg_bytes_per_kmer(k: int) -> dict:
     pb = (k + 3) // 4 + 2
     # SURVEY.md 8(d): record read + insert sector read+write-back + successor sector read + output byte
     return {"record": pb, "insert": 64, "lookup": 32, "output": 1, "total": pb + 97}
+
+
+DUMP_BLOCK = 4096                                       # elements per sampled block
+DUMP_CAP = {"contigs": 8 << 20, "offsets": 2 << 20}     # elements kept per array: 32 MB as float32 + 16 MB as float64
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_sample(n: int, cap: int, seed: int = SEED):
+    """Which blocks of an n-element output to keep: None (every element) when n <= cap, else the sorted numbers of a
+    fixed, seeded choice of DUMP_BLOCK-element blocks, at most cap elements in all."""
+    if n <= cap:
+        return None
+    n_blocks = (n + DUMP_BLOCK - 1) // DUMP_BLOCK
+    return np.sort(np.random.default_rng(seed).choice(n_blocks, cap // DUMP_BLOCK, replace=False))
+
+
+def dump_outputs(out_dir: str, contigs: np.ndarray, offsets: np.ndarray, n_nodes: int) -> dict:
+    """What kh_assemble_device hands its caller: the contig text (ASCII codes of '\\n'-terminated contigs) as contigs.npy
+    (float32), the n_contigs + 1 byte offsets into it as offsets.npy (float64), and counts.npy (float64: n_contigs,
+    contig bytes, nodes).  An array longer than its DUMP_CAP is replaced by a seeded sample of whole blocks, and
+    <name>_blocks.npy holds the numbers of the blocks kept (element i of block b is element b * DUMP_BLOCK + i).
+    Returns {file name: bytes written}."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"counts": np.array([offsets.size - 1, contigs.size, n_nodes], dtype=np.float64)}
+    for name, a, dtype in (("contigs", contigs, np.float32), ("offsets", offsets, np.float64)):
+        blocks = dump_sample(a.size, DUMP_CAP[name])
+        if blocks is not None:
+            idx = (blocks[:, None] * DUMP_BLOCK + np.arange(DUMP_BLOCK)).ravel()
+            a = a[idx[idx < a.size]]
+            arrays[name + "_blocks"] = blocks.astype(np.float64)
+        arrays[name] = a.astype(dtype)
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name + ".npy": int(a.nbytes) for name, a in arrays.items()}
 
 
 class ClockSampler:
@@ -175,7 +213,7 @@ def run_reference_arm(args, k: int, workload: str) -> dict:
         raise RuntimeError(f"oracle/_ref/kmer_hash_ref_{k} missing: run `make -C oracle` where /root/reference exists")
     mean_nodes = n_full / c_full
     runs = args.steps + args.warmup
-    work = tempfile.mkdtemp(prefix="kh_ref_", dir=os.path.join(ROOT, ".scratch") if os.path.isdir(os.path.join(ROOT, ".scratch")) else None)
+    work = tempfile.mkdtemp(prefix="kh_ref_")
 
     def make(n):
         d = kmergen.Dataset(k, n, max(1, int(round(n / mean_nodes))), seed=SEED)
@@ -259,8 +297,10 @@ def ncu_traffic_for(kernel_substr: str, workload: str):
     return None, None
 
 
-def measure_shape_n1(args, workload: str, steps: int, warmup: int, local_rank: int, full: bool) -> dict:
-    """One workload on one GPU: `steps` timed steps with the records resident in HBM, then the host-buffer leg."""
+def measure_shape_n1(args, workload: str, steps: int, warmup: int, local_rank: int, full: bool,
+                     dump_dir: str | None = None) -> dict:
+    """One workload on one GPU: `steps` timed steps with the records resident in HBM, then the host-buffer leg.
+    With `dump_dir`, the last timed step's output is written there (dump_outputs)."""
     import torch
 
     import cs267_hw3_b200 as kh
@@ -324,8 +364,16 @@ def measure_shape_n1(args, workload: str, steps: int, warmup: int, local_rank: i
     clocks = sampler.stop()
     ms = [a.elapsed_time(b) for a, b in evs]
     ms_per_step = float(np.mean(ms))
-    _, _, n_contigs, contig_bytes, n_nodes = out
+    contigs_dev, offsets_dev, n_contigs, contig_bytes, n_nodes = out
     st_last = tab.stats()
+    dumped = None
+    if dump_dir:
+        contigs_h = np.empty(contig_bytes, dtype=np.uint8)
+        offsets_h = np.empty(n_contigs + 1, dtype=np.uint64)
+        tab._check(kh.lib().kh_copy_to_host(tab._h, contigs_h.ctypes.data, contigs_dev, contigs_h.nbytes))
+        tab._check(kh.lib().kh_copy_to_host(tab._h, offsets_h.ctypes.data, offsets_dev, offsets_h.nbytes))
+        dumped = dump_outputs(dump_dir, contigs_h, offsets_h, n_nodes)
+        del contigs_h, offsets_h
 
     # correctness gate: re-run the traversal into host memory and compare the contig set with the generator's own
     # solution (order-independent digest) + node/contig counts
@@ -416,7 +464,7 @@ def measure_shape_n1(args, workload: str, steps: int, warmup: int, local_rank: i
                               "note": "N x B_alg / t(insert+traverse), SURVEY.md 8(d)"},
                      "probes_per_s": 2 * n / (ms_per_step * 1e-3),
                      "sector_ceiling_per_s": peak * 1e9 / 32},
-        "e2e": e2e, "pack_lines": pack, "gpu_launches": int(launches), "clocks": clocks,
+        "e2e": e2e, "pack_lines": pack, "gpu_launches": int(launches), "clocks": clocks, "dumped": dumped,
     }
     tab.close()
     host.free()
@@ -452,7 +500,7 @@ def run_b200_arm(args, workload: str) -> dict | None:
         sharded.shutdown()
         return line if rank == 0 else None
 
-    m = measure_shape_n1(args, workload, args.steps, args.warmup, local_rank, full=True)
+    m = measure_shape_n1(args, workload, args.steps, args.warmup, local_rank, full=True, dump_dir=args.dump_outputs)
     k = WORKLOADS[workload][0]
     line = {
         "metric": METRIC, "value": m["value"], "unit": UNIT, "n_gpus": 1,
@@ -462,6 +510,8 @@ def run_b200_arm(args, workload: str) -> dict | None:
     for key in ("ms_per_step_median", "ms_per_step_best", "config", "stages_ms", "n_segments", "rank_rounds", "assembly_time_s",
                 "wall_s_timed_loop", "gen_s", "verified", "roofline", "e2e", "pack_lines", "gpu_launches", "clocks"):
         line[key] = m[key]
+    if m["dumped"]:
+        line["dumped"] = {"dir": os.path.abspath(args.dump_outputs), "files": m["dumped"]}
     if second:
         line["shapes"] = {}
         for w in second:
@@ -521,7 +571,13 @@ def main():
                     help="further workloads measured in the same run and reported under \"shapes\" (default: chr14_k19)")
     ap.add_argument("--scaling", default="strong", choices=["strong", "weak"],
                     help="N>1 only: strong = the N=1 file split over the GPUs (default); weak = one such file per GPU (K>=31)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's output (contigs, offsets, counts) to DIR/<name>.npy (--gpus 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "b200"):
+        ap.error("--dump-outputs needs --gpus 1 and --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     # BASELINE.json configs[2]/[3]: the reference's real chr14 shape is K=51 (results/results_parallel_kmer51.txt);
     # the same file at every N (strong scaling over the sharded table).  configs[1] (K=19) rides along as a sub-record.
@@ -541,4 +597,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the tree may be read-only: the bench writes nothing into it
     main()
