@@ -24,7 +24,7 @@ $(LIB): $(CSRC) include/kh_capi.h
 kmer_hash_%: src/kmer_hash.cpp $(HDRS) $(LIB)
 	$(CXX) $(CXXFLAGS) -DKMER_LEN=$* -Iinclude $< -L$(PKG) -lkh_b200 -Wl,-rpath,$(abspath $(PKG)) -o $@
 
-kmer_count: src/kmer_count.cpp include/kh_capi.h include/kh/kmer_counter.hpp $(LIB)
+kmer_count: src/kmer_count.cpp include/kh_capi.h include/kh/kmer_counter.hpp include/kh/sharded_counter.hpp include/kh/sharded_host.hpp $(LIB)
 	$(CXX) $(CXXFLAGS) -Iinclude $< -L$(PKG) -lkh_b200 -Wl,-rpath,$(abspath $(PKG)) -o $@
 
 tools/gen_kmers: tools/kmer_gen.cpp

@@ -37,6 +37,7 @@ ABI_SYMBOLS = [
     # k-mer analysis (reads -> k-mers with extensions), the stage before this one
     "kh_count_create", "kh_count_destroy", "kh_count_clear", "kh_count_reads", "kh_count_reads_device",
     "kh_count_extract", "kh_count_extract_device", "kh_count_extract_lines", "kh_count_lookup", "kh_count_get_stats", "kh_count_last_error",
+    "kh_count_record_bytes", "kh_count_partition", "kh_count_merge_device",
 ]
 
 
@@ -132,6 +133,10 @@ def lib() -> C.CDLL:
     L.kh_count_get_stats.argtypes = [vp, C.POINTER(CountStats)]
     L.kh_count_last_error.argtypes = [vp]
     L.kh_count_last_error.restype = C.c_char_p
+    L.kh_count_record_bytes.argtypes = [i32]
+    L.kh_count_record_bytes.restype = u64
+    L.kh_count_partition.argtypes = [vp, i32, C.POINTER(vp), pu64]
+    L.kh_count_merge_device.argtypes = [vp, vp, u64]
     _lib = L
     return L
 
@@ -384,3 +389,26 @@ class KmerCounter:
         s = CountStats()
         self._check(lib().kh_count_get_stats(self._h, C.byref(s)))
         return s.as_dict()
+
+    # -- merging counters (sharded counting, kh_count_partition / kh_count_merge_device) --
+    def partition(self, world: int) -> tuple[int, np.ndarray]:
+        """Every k-mer of this counter grouped by owner rank: (device pointer to the records, uint64 offsets[world + 1]).
+        Group o holds records offsets[o] .. offsets[o+1] of record_bytes(k) bytes; the buffer belongs to the counter."""
+        p = C.c_void_p()
+        offs = np.zeros(world + 1, dtype=np.uint64)
+        self._check(lib().kh_count_partition(self._h, world, C.byref(p), offs.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return p.value or 0, offs
+
+    def merge_device(self, dev_ptr: int, n: int) -> None:
+        """Add n records (a group of another counter's partition, on any device) to this counter."""
+        self._check(lib().kh_count_merge_device(self._h, dev_ptr, n))
+
+    def merge(self, other: "KmerCounter") -> None:
+        """Add all k-mers of `other` (same K) to this counter: its counters become those of one counter over both inputs."""
+        ptr, offs = other.partition(1)
+        self.merge_device(ptr, int(offs[1]))
+
+
+def record_bytes(k: int) -> int:
+    """Bytes of one record of kh_count_partition: a counter slot, 16 (K <= 31) or 32."""
+    return 16 if k <= 31 else 32

@@ -63,7 +63,8 @@ def build_count_cli(force: bool = False) -> str:
     """kmer_count: reads -> the reference's k-mer file (or straight to contigs); K is a run-time argument."""
     build_lib()
     src = os.path.join(ROOT, "src", "kmer_count.cpp")
-    hdrs = [os.path.join(ROOT, "include", "kh_capi.h"), os.path.join(ROOT, "include", "kh", "kmer_counter.hpp")]
+    hdrs = [os.path.join(ROOT, "include", "kh_capi.h")] + [os.path.join(ROOT, "include", "kh", f) for f in
+                                                            ("kmer_counter.hpp", "sharded_counter.hpp", "sharded_host.hpp")]
     out = os.path.join(ROOT, "kmer_count")
     if force or _stale(out, [src, LIB, *hdrs]):
         _run(["g++", "-O2", "-std=c++17", "-pthread", "-I" + os.path.join(ROOT, "include"), src,

@@ -168,6 +168,74 @@ kc_extract_kernel(const u64* __restrict__ table, u64 n_slots, int k, u32 min_cou
     }
 }
 
+// Sharded counting, step 1: the occupied slots grouped by owner rank (kc_owner).  Two launches over the table, the same
+// block-wise pattern as kc_extract_kernel: a warp aggregates the slots of one owner with __match_any_sync, the block
+// collects per-owner counts in shared memory and reserves its run in each owner's segment with ONE global atomicAdd per
+// owner.  scatter = false: cursor[o] ends as owner o's slot count (the histogram); scatter = true: cursor[o] starts at
+// owner o's segment offset and the slots are copied there verbatim (order within a segment is arbitrary).
+template <int W>
+__global__ void __launch_bounds__(kKcExtThreads)
+kc_partition_kernel(const u64* __restrict__ table, u64 n_slots, u32 world, bool scatter, u64* __restrict__ cursor, u64* __restrict__ out) {
+    __shared__ u32 s_cnt[kKcMaxWorld];
+    __shared__ u64 s_base[kKcMaxWorld];
+    for (u32 o = threadIdx.x; o < world; o += kKcExtThreads) s_cnt[o] = 0;
+    __syncthreads();
+    const u64 first = (u64)blockIdx.x * (kKcExtThreads * kKcExtPer);
+    const u32 lane = threadIdx.x & 31u;
+    u32 own[kKcExtPer], at[kKcExtPer];
+#pragma unroll
+    for (int r = 0; r < kKcExtPer; ++r) {
+        const u64 i = first + (u64)r * kKcExtThreads + threadIdx.x;
+        own[r] = i < n_slots ? kc_slot_owner<W>(table, i, world) : world;
+        const u32 peers = __match_any_sync(kFull, own[r]);
+        const u32 leader = (u32)__ffs(peers) - 1u;
+        u32 base = 0;
+        if (lane == leader && own[r] < world) base = atomicAdd(&s_cnt[own[r]], (u32)__popc(peers));
+        at[r] = __shfl_sync(kFull, base, leader) + (u32)__popc(peers & ((1u << lane) - 1u));
+    }
+    __syncthreads();
+    for (u32 o = threadIdx.x; o < world; o += kKcExtThreads)
+        if (s_cnt[o]) s_base[o] = atomicAdd(&cursor[o], (u64)s_cnt[o]);
+    if (!scatter) return;
+    __syncthreads();
+#pragma unroll
+    for (int r = 0; r < kKcExtPer; ++r) {
+        if (own[r] >= world) continue;
+        const u64 i = first + (u64)r * kKcExtThreads + threadIdx.x;
+        const u64* src = table + i * (u64)KcSlot<W>::kWords;
+        u64* dst = out + (s_base[own[r]] + at[r]) * (u64)KcSlot<W>::kWords;
+#pragma unroll
+        for (int j = 0; j < KcSlot<W>::kWords; ++j) dst[j] = src[j];
+    }
+}
+
+// Sharded counting, step 2: records (slots of other tables of the same K) merged into this table, one per thread
+template <int W>
+__global__ void __launch_bounds__(256)
+kc_merge_kernel(const u64* __restrict__ recs, u64 n, u64* __restrict__ table, u64 n_slots, KcCounters* ctr) {
+    __shared__ u32 s_fresh, s_fail;
+    if (threadIdx.x == 0) { s_fresh = 0; s_fail = 0; }
+    __syncthreads();
+    const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    u32 fresh = 0, fail = 0;
+    if (i < n) {
+        bool f = false;
+        if (kc_merge_slot<W>(table, n_slots, recs + i * (u64)KcSlot<W>::kWords, f)) fresh = f ? 1u : 0u;
+        else fail = 1u;
+    }
+    fresh = __reduce_add_sync(kFull, fresh);
+    fail = __reduce_add_sync(kFull, fail);
+    if ((threadIdx.x & 31u) == 0) {
+        if (fresh) atomicAdd(&s_fresh, fresh);
+        if (fail) atomicAdd(&s_fail, fail);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        if (s_fresh) atomicAdd(&ctr->n_distinct, (u64)s_fresh);
+        if (s_fail) atomicOr(&ctr->errors, kKcErrFull);
+    }
+}
+
 template <int W>
 __global__ void __launch_bounds__(256)
 kc_lookup_kernel(const u64* __restrict__ table, u64 n_slots, int k, const unsigned char* __restrict__ pkmers, u64 n, u32* __restrict__ counts_out) {
@@ -213,6 +281,13 @@ struct kh_counter {
     size_t out_cap = 0;
     void* scratch = nullptr;
     size_t scratch_cap = 0;
+    void* outbox = nullptr;           // kh_count_partition: the slots grouped by owner
+    size_t outbox_cap = 0;
+    void* inbox = nullptr;            // kh_count_merge_device: records copied over from another device
+    size_t inbox_cap = 0;
+    void* cursor = nullptr;           // kh_count_partition: per-owner counts / write cursors
+    size_t cursor_cap = 0;
+    u64 peers_enabled = 0;            // bit d: this counter's device reads device d's memory directly
     u64 n_bytes = 0;
     u32 n_launches = 0;
     float ms_count = 0.f, ms_extract = 0.f;
@@ -381,6 +456,7 @@ int kh_count_destroy(kh_counter* c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     cudaFree(c->table); cudaFree(c->d_ctr); cudaFree(c->stage[0]); cudaFree(c->stage[1]); cudaFree(c->out); cudaFree(c->scratch);
+    cudaFree(c->outbox); cudaFree(c->inbox); cudaFree(c->cursor);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     if (c->ev2) cudaEventDestroy(c->ev2);
@@ -538,6 +614,84 @@ int kh_count_extract_lines(kh_counter* c, uint32_t min_count, uint32_t min_ext, 
         KC_CUDA(c, cudaStreamSynchronize(c->stream));
     }
     return KH_OK;
+}
+
+uint64_t kh_count_record_bytes(int k) { return k < 2 || k > 61 ? 0ull : (kc_slot_words(k) == 1 ? 16ull : 32ull); }
+
+int kh_count_partition(kh_counter* c, int world, const void** records_dev_out, uint64_t* offsets_host_out) {
+    if (!c || !records_dev_out || !offsets_host_out) return KH_ERR_ARG;
+    *records_dev_out = nullptr;
+    if (world < 1 || world > (int)kKcMaxWorld) return kc_fail(c, KH_ERR_ARG, "kh_count_partition: 1 <= world <= 64");
+    KC_CUDA(c, cudaSetDevice(c->device));
+    KC_TRY(kc_settle(c));                                   // a table that overflowed while counting is reported here
+    const u64 n = c->h_ctr.n_distinct, rb = c->W == 1 ? 16 : 32;
+    KC_TRY(kc_grow(c, &c->outbox, &c->outbox_cap, (size_t)(std::max<u64>(n, 1) * rb)));
+    KC_TRY(kc_grow(c, &c->cursor, &c->cursor_cap, kKcMaxWorld * sizeof(u64)));
+    u64* cur = static_cast<u64*>(c->cursor);
+    const u64 blocks = (c->n_slots + kKcExtThreads * kKcExtPer - 1) / (kKcExtThreads * kKcExtPer);
+    auto launch = [&](bool scatter) -> int {
+        if (c->W == 1)
+            kc_partition_kernel<1><<<(unsigned)blocks, kKcExtThreads, 0, c->stream>>>(c->table, c->n_slots, (u32)world, scatter, cur, static_cast<u64*>(c->outbox));
+        else
+            kc_partition_kernel<2><<<(unsigned)blocks, kKcExtThreads, 0, c->stream>>>(c->table, c->n_slots, (u32)world, scatter, cur, static_cast<u64*>(c->outbox));
+        KC_CUDA(c, cudaGetLastError());
+        ++c->n_launches;
+        return KH_OK;
+    };
+    u64 h[kKcMaxWorld + 1] = {};
+    KC_CUDA(c, cudaMemsetAsync(cur, 0, (size_t)world * sizeof(u64), c->stream));
+    KC_TRY(launch(false));
+    KC_CUDA(c, cudaMemcpyAsync(h + 1, cur, (size_t)world * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    for (int o = 0; o < world; ++o) h[o + 1] += h[o];      // per-owner counts -> segment offsets
+    if (h[world] != n) return kc_fail(c, KH_ERR_CUDA, "k-mer counter: occupied slots differ from the distinct count (internal)");
+    KC_CUDA(c, cudaMemcpyAsync(cur, h, (size_t)world * sizeof(u64), cudaMemcpyHostToDevice, c->stream));
+    KC_TRY(launch(true));
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    for (int o = 0; o <= world; ++o) offsets_host_out[o] = h[o];
+    *records_dev_out = c->outbox;
+    return KH_OK;
+}
+
+int kh_count_merge_device(kh_counter* c, const void* records_dev, uint64_t n) {
+    if (!c || (n && !records_dev)) return KH_ERR_ARG;
+    if (n == 0) return KH_OK;
+    KC_CUDA(c, cudaSetDevice(c->device));
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, records_dev) != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)) {
+        cudaGetLastError();
+        return kc_fail(c, KH_ERR_ARG, "kh_count_merge_device: records_dev is not device memory");
+    }
+    const u64 rb = c->W == 1 ? 16 : 32;
+    const u64* src = static_cast<const u64*>(records_dev);
+    if (a.type == cudaMemoryTypeDevice && a.device != c->device) {
+        // another GPU's records: one copy into this counter's inbox, peer to peer where the devices allow it
+        if (a.device >= 0 && a.device < 64 && !((c->peers_enabled >> a.device) & 1ull)) {
+            int can = 0;
+            if (cudaDeviceCanAccessPeer(&can, c->device, a.device) == cudaSuccess && can) {
+                const cudaError_t e = cudaDeviceEnablePeerAccess(a.device, 0);
+                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) KC_CUDA(c, e);
+                cudaGetLastError();
+            }
+            c->peers_enabled |= 1ull << a.device;
+        }
+        KC_TRY(kc_grow(c, &c->inbox, &c->inbox_cap, (size_t)(n * rb)));
+        KC_CUDA(c, cudaMemcpyAsync(c->inbox, records_dev, (size_t)(n * rb), cudaMemcpyDefault, c->stream));
+        src = static_cast<const u64*>(c->inbox);
+    }
+    for (u64 done = 0; done < n;) {                        // like kh_count_reads: every record may be a new k-mer
+        u64 take = 0;
+        KC_TRY(kc_reserve(c, n - done, &take));
+        const u64 blocks = (take + 255) / 256;
+        const u64* r = src + done * (rb / 8);
+        if (c->W == 1) kc_merge_kernel<1><<<(unsigned)blocks, 256, 0, c->stream>>>(r, take, c->table, c->n_slots, c->d_ctr);
+        else kc_merge_kernel<2><<<(unsigned)blocks, 256, 0, c->stream>>>(r, take, c->table, c->n_slots, c->d_ctr);
+        KC_CUDA(c, cudaGetLastError());
+        ++c->n_launches;
+        c->distinct_ub += take;
+        done += take;
+    }
+    return kc_settle(c);
 }
 
 int kh_count_lookup(kh_counter* c, const void* pkmers_host, uint64_t n, uint32_t* counts_host_out) {

@@ -318,6 +318,84 @@ __host__ __device__ __forceinline__ bool kc_move_slot(const u64* old_table, u64 
     return false;
 }
 
+// ---- merging tables (sharded counting: one table per rank, every k-mer reduced at its owner rank) ----------------
+// Every field of the counter word saturates, and min(cap, min(cap, a) + min(cap, b)) = min(cap, a + b): adding the words
+// of per-rank tables field by field with saturation gives exactly the word one table over all reads would hold, in any
+// order and grouping -- provided nothing was dropped before the merge and no k-mer or observation straddles two ranks.
+constexpr u32 kKcMaxWorld = 64;
+
+// Owner rank of a k-mer: a second mix of kc_hash, independent of its top bits (kc_home takes those).  Were the owner
+// drawn from the top bits too, the keys of one owner would all have their home slot in 1/world of its table.  Depends
+// on the key and world only, never on a table size.
+__host__ __device__ __forceinline__ u32 kc_owner(u64 key_hi, u64 key_lo, u32 world) {
+    return (u32)kc_mulhi64(fmix64(kc_hash(key_hi, key_lo) ^ 0xD6E8FEB86659FD93ull), (u64)world);
+}
+// per-field saturating sum of two counter words (occurrences at 255, each of the 8 observation counts at 127); no carry
+// crosses a field border
+__host__ __device__ __forceinline__ u64 kc_add(u64 a, u64 b) {
+    u64 t = (a & 0xFFull) + (b & 0xFFull);
+    u64 r = t > kKcCountCap ? kKcCountCap : t;
+#pragma unroll
+    for (u32 f = 0; f < 8u; ++f) {
+        const u32 s = 8u + 7u * f;
+        t = ((a >> s) & 127ull) + ((b >> s) & 127ull);
+        r |= (t > kKcExtCap ? (u64)kKcExtCap : t) << s;
+    }
+    return r;
+}
+__host__ __device__ __forceinline__ void kc_tag_key(int W, u64 t0, u64 t1, u64& key_hi, u64& key_lo) {
+    key_lo = W == 1 ? t0 >> 1 : t0;
+    key_hi = W == 1 ? 0ull : t1 & ~(1ull << 63);
+}
+// slot i: its owner rank, or `world` when the slot is empty
+template <int W>
+__host__ __device__ __forceinline__ u32 kc_slot_owner(const u64* table, u64 i, u32 world) {
+    const u64* p = table + i * (u64)KcSlot<W>::kWords;
+    const u64 q[4] = {p[0], p[1], 0ull, 0ull};
+    if (kc_slot_empty<W>(q)) return world;
+    u64 kh_, kl_;
+    kc_tag_key(W, q[0], q[1], kh_, kl_);
+    return kc_owner(kh_, kl_, world);
+}
+// One record -- a slot of another table of the same K, copied verbatim -- merged into this table: find or claim the key's
+// slot (as kc_move_slot / kc_upsert do), then add the counter word with kc_add in a CAS loop: one launch may carry the
+// same key from several source tables.  Returns false when the table is full.
+template <int W>
+__host__ __device__ __forceinline__ bool kc_merge_slot(u64* table, u64 n_slots, const u64* rec, bool& fresh) {
+    const u64 t0 = rec[0], t1 = W == 1 ? 0ull : rec[1], add = rec[W == 1 ? 1 : 2];
+    u64 key_hi, key_lo;
+    kc_tag_key(W, t0, t1, key_hi, key_lo);
+    u64 s = kc_home(key_hi, key_lo, n_slots);
+    fresh = false;
+    for (u64 tries = 0, lim = n_slots < kKcMaxProbes ? n_slots : kKcMaxProbes; tries < lim; ++tries) {
+        u64* p = table + s * (u64)KcSlot<W>::kWords;
+        u64 q[4];
+        kc_load_slot<W>(p, q);
+        if (kc_slot_empty<W>(q)) {
+            if (W == 1) {
+                const u64 old = kc_cas64(p, 0ull, t0);
+                if (old == 0ull) { fresh = true; q[0] = t0; } else q[0] = old;
+            } else {
+                const u128 old = kc_cas128(p, u128{0ull, 0ull}, u128{t0, t1});
+                if (old.lo == 0ull && old.hi == 0ull) { fresh = true; q[0] = t0; q[1] = t1; } else { q[0] = old.lo; q[1] = old.hi; }
+            }
+        }
+        if (kc_slot_is<W>(q, t0, t1)) {
+            u64* w = p + (W == 1 ? 1 : 2);
+            u64 c = kc_slot_counters<W>(q);
+            for (;;) {
+                const u64 n = kc_add(c, add);
+                if (n == c) return true;
+                const u64 old = kc_cas64(w, c, n);
+                if (old == c) return true;
+                c = old;
+            }
+        }
+        s = (s + 1 == n_slots) ? 0ull : s + 1;
+    }
+    return false;
+}
+
 // ---- k-mer <-> the reference's packed bytes (packing.hpp:77-92: first base in bits 7..6 of byte 0, A-padded tail) ---
 __host__ __device__ __forceinline__ void kc_key_to_packed(u64 key_hi, u64 key_lo, int k, unsigned char* out) {
     const int pl = (k + 3) >> 2, sh = 8 * pl - 2 * k;       // 0, 2, 4 or 6 bits of padding

@@ -27,7 +27,8 @@ class KmerCounter {
     }
 
   public:
-    // n_distinct_expected counts every distinct k-mer of the reads (erroneous ones too); the table does not grow.
+    // n_distinct_expected counts every distinct k-mer of the reads (erroneous ones too).  count_reads doubles the table
+    // when it runs short (kh_count_create), so a good estimate only saves the rehashes.
     KmerCounter(int k, uint64_t n_distinct_expected, double load_factor = 0.5, int device = 0) : k_(k) {
         if (kh_device_count() <= 0) throw std::runtime_error("KmerCounter: no CUDA device (libkh_b200 has no CPU fallback)");
         check(kh_count_create(k, n_distinct_expected, load_factor, device, &c_), "kh_count_create");

@@ -222,7 +222,15 @@ int kh_shard_result(kh_table* t, const char** contigs_dev, const uint64_t** offs
  * (1..255); an extension is the base that alone reaches min_ext (1..127) on its side, 'F' when none does
  * (a contig begins / ends: README.md:37) or several do (a fork).  No reverse complements, like the reference
  * (kmer_t.hpp:51-57).  Records come out in table order (arbitrary, as k-mer counters' output is).
- * One GPU per counter; supported K: 2..61.
+ * Supported K: 2..61.
+ *
+ * One GPU per counter, several counters per analysis: every counter field saturates, and saturating sums are
+ * associative, so counters that counted disjoint pieces of the reads (cut at a non-base byte) merge field by field
+ * into exactly the counters one table over all reads would hold.  kh_count_partition groups a counter's k-mers by
+ * owner rank, kh_count_merge_device adds such a group into another counter (on any device of the process): P
+ * ranks count their pieces, every owner merges the group addressed to it from every rank, and the union of the
+ * owners' extracts is the single-counter result (include/kh/sharded_counter.hpp drives that flow).  Thresholds
+ * apply to the merged counters only -- nothing may be dropped before the merge.
  * ------------------------------------------------------------------------------------------- */
 typedef struct kh_counter kh_counter;
 typedef struct kh_count_stats {
@@ -264,6 +272,19 @@ int kh_count_extract_lines(kh_counter* c, uint32_t min_count, uint32_t min_ext, 
 int kh_count_lookup(kh_counter* c, const void* pkmers_host, uint64_t n, uint32_t* counts_host_out);
 int kh_count_get_stats(kh_counter* c, kh_count_stats* out);
 const char* kh_count_last_error(kh_counter* c);
+/* Merging counters.  A record is one k-mer with its counters, kh_count_record_bytes(k) = 16 or 32 bytes; the format is
+ * opaque and meaningful only to a counter of the same K.  The owner rank of a k-mer depends on the k-mer and world only.
+ * kh_count_partition: every k-mer of this counter, grouped by owner rank (0..world-1), in a counter-owned device buffer
+ * valid until the next partition or destroy; offsets_host_out: world+1 record offsets (group o = records
+ * [offsets[o], offsets[o+1])).  1 <= world <= 64.  Host-synchronous; returns KH_ERR_TABLE_FULL after a count that
+ * overflowed the table.
+ * kh_count_merge_device: saturating merge of n records into this counter.  records_dev may live on any device of this
+ * process: if it is not the counter's, it is first copied into a counter-owned inbox (peer to peer where possible).
+ * Grows the table like kh_count_reads (KH_COUNT_GROW=0 -> KH_ERR_TABLE_FULL).  Host-synchronous.  Adds the newly seen
+ * k-mers to n_distinct; n_occurrences and n_bytes keep counting only what kh_count_reads* consumed here. */
+uint64_t kh_count_record_bytes(int k);
+int kh_count_partition(kh_counter* c, int world, const void** records_dev_out, uint64_t* offsets_host_out);
+int kh_count_merge_device(kh_counter* c, const void* records_dev, uint64_t n);
 
 /* Introspection for tests and debugging: device pointer and capacity of an internal buffer of a chunk table
  * ("link", "meta", "chunk_base", "seg_base", "chunk_cursor", "counters", ...; "caps" returns HOST numbers). */

@@ -13,6 +13,14 @@
 // the host).  Bases are upper-case ACGT; anything else (N, ...) splits a read.  Defaults: min_count = min_ext = 2.
 // Environment: KH_DEVICE, KH_LOAD_FACTOR (0.5), KH_COUNT_DISTINCT = distinct k-mers to size the table for, erroneous
 // ones included (default: half the input bytes).
+//
+// KH_RANKS=P (2..8): the analysis on P ranks (GPU r % visible GPUs, KH_DEVICE is not used), kh_sharded::CountCluster:
+// the pieces of the file are dealt to the ranks in turn, every rank counts its pieces, and reduce() merges all counts at
+// the k-mers' owner ranks -- whenever a rank has counted KH_COUNT_BATCH_BYTES since the last reduce (then pieces are
+// that size too; default: no intermediate reduce) and once at the end.  The k-mer file is the ranks' k-mers in rank
+// order; with --contigs, every rank's records go on its GPU into kh_sharded::Cluster (17 <= K <= 54) and rank r writes
+// PREFIX_r.dat.  Same k-mers, counters and contigs as P = 1, in another order.
+#include <algorithm>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -22,6 +30,8 @@
 #include <vector>
 
 #include "kh/kmer_counter.hpp"
+#include "kh/sharded_counter.hpp"
+#include "kh/sharded_host.hpp"
 
 namespace {
 
@@ -34,6 +44,96 @@ void must(int status, kh_table* t, const char* what) {
 int usage() {
     fprintf(stderr, "Usage: kmer_count K reads_file (kmer_file_out | --contigs PREFIX) [min_count [min_ext]]\n");
     return 1;
+}
+
+// The file goes through in pieces of about `buffer` bytes that end on a line boundary (FASTA: before a header); each
+// piece's sequence lines (kh::sequence_lines) go to sink(text, n).
+template <class Sink> void read_pieces(FILE* f, size_t buffer, Sink sink) {
+    std::vector<char> buf(buffer);
+    size_t carry = 0;
+    char format = 0;
+    unsigned state = 0;
+    for (;;) {
+        if (carry == buf.size()) buf.resize(buf.size() * 2);                  // a single line longer than the buffer
+        const size_t got = fread(buf.data() + carry, 1, buf.size() - carry, f);
+        const size_t have = carry + got;
+        if (have == 0) break;
+        if (format == 0) format = buf[0] == '>' ? 'a' : (buf[0] == '@' ? 'q' : 'p');
+        size_t cut = have;
+        if (got != 0) {                                                       // not at the end of the file: stop where a new read starts
+            cut = kh::sequence_cut(buf.data(), have, format);
+            if (cut == 0) { carry = have; continue; }
+        }
+        size_t len = cut;
+        kh::sequence_lines(buf.data(), len, format, state);
+        sink(buf.data(), len);
+        carry = have - cut;
+        memmove(buf.data(), buf.data() + cut, carry);
+        if (got == 0) break;
+    }
+}
+
+int count_sharded(FILE* f, int k, int ranks, uint64_t distinct, double lf, bool contigs, const std::string& out_name,
+                  uint32_t min_count, uint32_t min_ext) {
+    using clock = std::chrono::high_resolution_clock;
+    const uint64_t batch = getenv("KH_COUNT_BATCH_BYTES") ? strtoull(getenv("KH_COUNT_BATCH_BYTES"), nullptr, 10) : 0;
+    const size_t buffer = batch ? (size_t)std::min<uint64_t>(128u << 20, std::max<uint64_t>(batch, 4096)) : (128u << 20) + (1u << 20);
+    const auto t0 = clock::now();
+    kh_sharded::CountCluster cluster(k, ranks, distinct, lf);
+    int next = 0;
+    read_pieces(f, buffer, [&](const char* p, size_t n) {
+        const int r = next;
+        next = (next + 1) % ranks;
+        cluster.count(r, p, n);
+        if (batch && cluster.batch_bytes(r) >= batch) cluster.reduce();
+    });
+    fclose(f);
+    cluster.reduce();
+    const auto t1 = clock::now();
+    printf("Counted %llu k-mer occurrences, %llu distinct %d-mers, from %llu bytes of reads in %lf s\n",
+           (unsigned long long)cluster.n_occurrences(), (unsigned long long)cluster.n_distinct(), k,
+           (unsigned long long)cluster.n_bytes(), std::chrono::duration<double>(t1 - t0).count());
+
+    if (!contigs) {
+        FILE* o = fopen(out_name.c_str(), "wb");
+        if (o == nullptr) throw std::runtime_error("kmer_count: could not open " + out_name);
+        uint64_t lines = 0;
+        for (int r = 0; r < ranks; ++r) {
+            const std::string text = cluster.extract_lines(r, min_count, min_ext);
+            if (fwrite(text.data(), 1, text.size(), o) != text.size()) throw std::runtime_error("kmer_count: short write to " + out_name);
+            lines += text.size() / (size_t)(k + 4);
+        }
+        fclose(o);
+        printf("Wrote %llu k-mers (count >= %u, extensions seen >= %u times) to %s\n", (unsigned long long)lines, min_count,
+               min_ext, out_name.c_str());
+        return 0;
+    }
+    std::vector<const void*> recs(ranks);
+    std::vector<uint64_t> n(ranks);
+    for (int r = 0; r < ranks; ++r) recs[r] = cluster.extract_device(r, min_count, min_ext, n[r]);
+    uint64_t n_local_max = 1, n_total = 0;
+    for (uint64_t x : n) { n_local_max = std::max(n_local_max, x); n_total += x; }
+    const auto t2 = clock::now();
+    kh_sharded::Cluster tables(k, ranks, n_local_max, std::max<uint64_t>(n_total, 1), lf);
+    tables.begin();
+    tables.insert(recs, n);
+    const std::vector<kh_sharded::RankOutput> outs = tables.assemble();
+    const auto t3 = clock::now();
+    uint64_t nc = 0, nodes = 0;
+    for (int r = 0; r < ranks; ++r) {
+        const std::string dat = out_name + "_" + std::to_string(r) + ".dat";
+        FILE* o = fopen(dat.c_str(), "wb");
+        if (o == nullptr) throw std::runtime_error("kmer_count: could not open " + dat);
+        const std::vector<char>& text = outs[r].text;
+        if (!text.empty() && fwrite(text.data(), 1, text.size(), o) != text.size()) throw std::runtime_error("kmer_count: short write to " + dat);
+        fclose(o);
+        nc += outs[r].n_contigs;
+        nodes += outs[r].n_nodes;
+    }
+    printf("Assembled %llu k-mers into %llu contigs with %llu nodes in %lf s; wrote %s_0.dat .. %s_%d.dat\n",
+           (unsigned long long)n_total, (unsigned long long)nc, (unsigned long long)nodes,
+           std::chrono::duration<double>(t3 - t2).count(), out_name.c_str(), out_name.c_str(), ranks - 1);
+    return 0;
 }
 
 }  // namespace
@@ -59,33 +159,14 @@ int main(int argc, char** argv) {
     fseek(f, 0, SEEK_SET);
     const uint64_t distinct = getenv("KH_COUNT_DISTINCT") ? strtoull(getenv("KH_COUNT_DISTINCT"), nullptr, 10)
                                                           : (file_bytes / 2 > 1024 ? file_bytes / 2 : 1024);
+    const int ranks = getenv("KH_RANKS") ? atoi(getenv("KH_RANKS")) : 1;
+    if (ranks < 1 || ranks > 8) { fprintf(stderr, "kmer_count: KH_RANKS must be 1..8\n"); return 1; }
+    if (ranks > 1 && contigs && (k < 17 || k > 54)) { fprintf(stderr, "kmer_count: --contigs with KH_RANKS > 1 needs 17 <= K <= 54\n"); return 1; }
+    if (ranks > 1) return count_sharded(f, k, ranks, distinct, lf, contigs, out_name, min_count, min_ext);
     const auto t0 = std::chrono::high_resolution_clock::now();
     kh::KmerCounter counter(k, distinct, lf, device);
 
-    // the file goes through in pieces that end on a line boundary
-    const size_t piece = 128u << 20;
-    std::vector<char> buf(piece + (1u << 20));
-    size_t carry = 0;
-    char format = 0;
-    unsigned state = 0;
-    for (;;) {
-        if (carry == buf.size()) buf.resize(buf.size() * 2);                  // a single line longer than the buffer
-        const size_t got = fread(buf.data() + carry, 1, buf.size() - carry, f);
-        const size_t have = carry + got;
-        if (have == 0) break;
-        if (format == 0) format = buf[0] == '>' ? 'a' : (buf[0] == '@' ? 'q' : 'p');
-        size_t cut = have;
-        if (got != 0) {                                                       // not at the end of the file: stop where a new read starts
-            cut = kh::sequence_cut(buf.data(), have, format);
-            if (cut == 0) { carry = have; continue; }
-        }
-        size_t len = cut;
-        kh::sequence_lines(buf.data(), len, format, state);
-        counter.count_reads(buf.data(), len);
-        carry = have - cut;
-        memmove(buf.data(), buf.data() + cut, carry);
-        if (got == 0) break;
-    }
+    read_pieces(f, (128u << 20) + (1u << 20), [&](const char* p, size_t n) { counter.count_reads(p, n); });
     fclose(f);
     const auto t1 = std::chrono::high_resolution_clock::now();
     kh_count_stats st = counter.stats();
