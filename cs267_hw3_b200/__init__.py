@@ -37,7 +37,7 @@ ABI_SYMBOLS = [
     # k-mer analysis (reads -> k-mers with extensions), the stage before this one
     "kh_count_create", "kh_count_destroy", "kh_count_clear", "kh_count_reads", "kh_count_reads_device",
     "kh_count_extract", "kh_count_extract_device", "kh_count_extract_lines", "kh_count_lookup", "kh_count_get_stats", "kh_count_last_error",
-    "kh_count_record_bytes", "kh_count_partition", "kh_count_merge_device",
+    "kh_count_record_bytes", "kh_count_partition", "kh_count_merge_device", "kh_count_histogram", "kh_count_auto_min_count",
 ]
 
 
@@ -137,6 +137,9 @@ def lib() -> C.CDLL:
     L.kh_count_record_bytes.restype = u64
     L.kh_count_partition.argtypes = [vp, i32, C.POINTER(vp), pu64]
     L.kh_count_merge_device.argtypes = [vp, vp, u64]
+    L.kh_count_histogram.argtypes = [vp, pu64]
+    L.kh_count_auto_min_count.argtypes = [pu64]
+    L.kh_count_auto_min_count.restype = u32
     _lib = L
     return L
 
@@ -385,6 +388,12 @@ class KmerCounter:
         self._check(lib().kh_count_lookup(self._h, q.ctypes.data, n, out.ctypes.data))
         return out
 
+    def histogram(self) -> np.ndarray:
+        """The k-mer spectrum, uint64[256]: [c] = distinct k-mers seen exactly c times, [255] = 255 times or more, [0] = 0."""
+        h = np.zeros(HIST_BINS, dtype=np.uint64)
+        self._check(lib().kh_count_histogram(self._h, h.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return h
+
     def stats(self) -> dict:
         s = CountStats()
         self._check(lib().kh_count_get_stats(self._h, C.byref(s)))
@@ -407,6 +416,20 @@ class KmerCounter:
         """Add all k-mers of `other` (same K) to this counter: its counters become those of one counter over both inputs."""
         ptr, offs = other.partition(1)
         self.merge_device(ptr, int(offs[1]))
+
+
+HIST_BINS = 256
+
+
+def auto_min_count(hist) -> int:
+    """min_count at the valley of a k-mer spectrum (256 bins, KmerCounter.histogram()): kh_count_auto_min_count.
+    None gives the default, 2."""
+    if hist is None:
+        return int(lib().kh_count_auto_min_count(None))
+    h = np.ascontiguousarray(hist, dtype=np.uint64)
+    if h.shape != (HIST_BINS,):
+        raise ValueError(f"a spectrum has {HIST_BINS} bins, got shape {h.shape}")
+    return int(lib().kh_count_auto_min_count(h.ctypes.data_as(C.POINTER(C.c_uint64))))
 
 
 def record_bytes(k: int) -> int:

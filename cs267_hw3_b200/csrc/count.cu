@@ -8,6 +8,7 @@
 //                      sector read + one CAS on the counter word
 //   kc_extract_kernel  table scan -> kmer_pair records of the k-mers with enough occurrences (block-wise compaction)
 //   kc_lookup_kernel   counters of given k-mers
+//   kc_histogram_kernel  table scan -> the k-mer spectrum (distinct k-mers per occurrence count)
 //
 // HBM-bound integer work like the rest of the library: what an occurrence costs is one random 32-byte sector (the slot)
 // read and written back.  Algorithmic bytes per occurrence = 1 (the character) + 64.
@@ -236,6 +237,33 @@ kc_merge_kernel(const u64* __restrict__ recs, u64 n, u64* __restrict__ table, u6
     }
 }
 
+// The k-mer spectrum (kc_slot_total per slot, binned): one read of the table, grid-stride with a few blocks per SM so the
+// global flush stays at about blocks x 256 atomics.  The bins are very skewed -- half the slots are empty at load 0.5 and
+// most k-mers of error-rich reads sit in bin 1 -- so a warp aggregates its equal values with __match_any_sync before
+// the shared atomic, as kc_partition_kernel does.  Empty slots (value 0) are not binned.
+constexpr int kKcHistThreads = 256;
+constexpr int kKcHistBlocksPerSm = 4;
+
+template <int W>
+__global__ void __launch_bounds__(kKcHistThreads)
+kc_histogram_kernel(const u64* __restrict__ table, u64 n_slots, u64* __restrict__ hist) {
+    __shared__ u32 s_bin[kKcHistBins];
+    for (u32 b = threadIdx.x; b < kKcHistBins; b += kKcHistThreads) s_bin[b] = 0;
+    __syncthreads();
+    const u32 lane = threadIdx.x & 31u;
+    const u64 stride = (u64)gridDim.x * kKcHistThreads;
+    // the bound is block-uniform: every lane reaches __match_any_sync
+    for (u64 first = (u64)blockIdx.x * kKcHistThreads; first < n_slots; first += stride) {
+        const u64 i = first + threadIdx.x;
+        const u32 v = i < n_slots ? kc_slot_total<W>(table, i) : 0u;
+        const u32 peers = __match_any_sync(kFull, v);
+        if (v && lane == (u32)__ffs(peers) - 1u) atomicAdd(&s_bin[v], (u32)__popc(peers));
+    }
+    __syncthreads();
+    for (u32 b = threadIdx.x; b < kKcHistBins; b += kKcHistThreads)
+        if (s_bin[b]) atomicAdd(&hist[b], (u64)s_bin[b]);
+}
+
 template <int W>
 __global__ void __launch_bounds__(256)
 kc_lookup_kernel(const u64* __restrict__ table, u64 n_slots, int k, const unsigned char* __restrict__ pkmers, u64 n, u32* __restrict__ counts_out) {
@@ -287,6 +315,8 @@ struct kh_counter {
     size_t inbox_cap = 0;
     void* cursor = nullptr;           // kh_count_partition: per-owner counts / write cursors
     size_t cursor_cap = 0;
+    void* hist = nullptr;             // kh_count_histogram: 256 x u64 bins
+    size_t hist_cap = 0;
     u64 peers_enabled = 0;            // bit d: this counter's device reads device d's memory directly
     u64 n_bytes = 0;
     u32 n_launches = 0;
@@ -456,7 +486,7 @@ int kh_count_destroy(kh_counter* c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     cudaFree(c->table); cudaFree(c->d_ctr); cudaFree(c->stage[0]); cudaFree(c->stage[1]); cudaFree(c->out); cudaFree(c->scratch);
-    cudaFree(c->outbox); cudaFree(c->inbox); cudaFree(c->cursor);
+    cudaFree(c->outbox); cudaFree(c->inbox); cudaFree(c->cursor); cudaFree(c->hist);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     if (c->ev2) cudaEventDestroy(c->ev2);
@@ -693,6 +723,33 @@ int kh_count_merge_device(kh_counter* c, const void* records_dev, uint64_t n) {
     }
     return kc_settle(c);
 }
+
+int kh_count_histogram(kh_counter* c, uint64_t* hist_host_out) {
+    if (!c || !hist_host_out) return KH_ERR_ARG;
+    KC_CUDA(c, cudaSetDevice(c->device));
+    KC_TRY(kc_settle(c));                                   // a table that overflowed while counting is reported here
+    KC_TRY(kc_grow(c, &c->hist, &c->hist_cap, kKcHistBins * sizeof(u64)));
+    int sms = 0;
+    KC_CUDA(c, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    const u64 blocks = std::max<u64>(1, std::min<u64>((c->n_slots + kKcHistThreads - 1) / kKcHistThreads, (u64)std::max(sms, 1) * kKcHistBlocksPerSm));
+    u64* d = static_cast<u64*>(c->hist);
+    KC_CUDA(c, cudaMemsetAsync(d, 0, kKcHistBins * sizeof(u64), c->stream));
+    if (c->W == 1) kc_histogram_kernel<1><<<(unsigned)blocks, kKcHistThreads, 0, c->stream>>>(c->table, c->n_slots, d);
+    else kc_histogram_kernel<2><<<(unsigned)blocks, kKcHistThreads, 0, c->stream>>>(c->table, c->n_slots, d);
+    KC_CUDA(c, cudaGetLastError());
+    ++c->n_launches;
+    u64 h[kKcHistBins];
+    KC_CUDA(c, cudaMemcpyAsync(h, d, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    u64 total = 0;
+    for (u32 b = 0; b < kKcHistBins; ++b) total += h[b];
+    if (h[0] != 0 || total != c->h_ctr.n_distinct)
+        return kc_fail(c, KH_ERR_CUDA, "k-mer counter: spectrum bins differ from the distinct count (internal)");
+    memcpy(hist_host_out, h, sizeof h);
+    return KH_OK;
+}
+
+uint32_t kh_count_auto_min_count(const uint64_t* hist) { return kc_auto_min_count(reinterpret_cast<const u64*>(hist)); }
 
 int kh_count_lookup(kh_counter* c, const void* pkmers_host, uint64_t n, uint32_t* counts_host_out) {
     if (!c || (n && (!pkmers_host || !counts_host_out))) return KH_ERR_ARG;

@@ -423,6 +423,33 @@ __host__ __device__ __forceinline__ bool kc_slot_reported(const u64* table, u64 
     const u64 q[4] = {p[0], p[1], W == 1 ? 0ull : p[2], 0ull};
     return !kc_slot_empty<W>(q) && kc_total(kc_slot_counters<W>(q)) >= min_count;
 }
+// slot i of the finished table: the occurrences of its k-mer (saturated at 255), 0 for an empty slot -- its spectrum bin
+template <int W>
+__host__ __device__ __forceinline__ u32 kc_slot_total(const u64* table, u64 i) {
+    const u64* p = table + i * (u64)KcSlot<W>::kWords;
+    const u64 q[4] = {p[0], p[1], W == 1 ? 0ull : p[2], 0ull};
+    return kc_slot_empty<W>(q) ? 0u : kc_total(kc_slot_counters<W>(q));
+}
+
+// ---- the k-mer spectrum -----------------------------------------------------------------------------------------
+// hist[c] (c = 1..254): distinct k-mers counted exactly c times; hist[255]: those seen 255 times or more; hist[0] = 0.
+constexpr u32 kKcHistBins = 256;
+constexpr u32 kKcDefaultMinCount = 2;
+// The valley rule: reads with sequencing errors give a falling slope of erroneous k-mers (count 1, 2, ...) that meets the
+// coverage peak of the true ones; the first c where the spectrum stops falling (hist[c+1] >= hist[c]) separates them.
+// That c is the threshold when it is >= 2 and k-mers remain at or above it; otherwise (no falling slope -- error-free reads,
+// an empty table -- or a spectrum that falls to zero with no second peak) the default 2.
+inline u32 kc_auto_min_count(const u64* hist) {
+    if (!hist) return kKcDefaultMinCount;
+    for (u32 c = 1; c + 1 < kKcHistBins; ++c) {
+        if (hist[c + 1] < hist[c]) continue;
+        if (c < 2) return kKcDefaultMinCount;
+        u64 above = 0;
+        for (u32 d = c; d < kKcHistBins; ++d) above += hist[d];
+        return above > 0 ? c : kKcDefaultMinCount;
+    }
+    return kKcDefaultMinCount;
+}
 template <int W>
 __host__ __device__ __forceinline__ void kc_slot_record(const u64* table, u64 i, int k, u32 min_ext, unsigned char* rec) {
     const u64* p = table + i * (u64)KcSlot<W>::kWords;

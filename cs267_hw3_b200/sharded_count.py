@@ -150,6 +150,11 @@ class ShardedCounter:
     def extract_lines(self, rank: int, min_count: int = 2, min_ext: int = 2) -> np.ndarray:
         return self.owned[rank].extract_lines(min_count, min_ext)
 
+    def histogram(self) -> np.ndarray:
+        """After reduce(): the k-mer spectrum of everything reduced so far, uint64[256] (KmerCounter.histogram()).  Every
+        k-mer has one owner and the owned counters equal one counter's, so the sum of the owners' spectra is exact."""
+        return np.sum([c.histogram() for c in self.owned], axis=0, dtype=np.uint64)
+
     def lookup(self, rank: int, pkmers) -> np.ndarray:
         return self.owned[rank].lookup(pkmers)
 

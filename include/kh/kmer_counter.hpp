@@ -7,6 +7,7 @@
 // quality lines contain letters that would read as bases).
 #pragma once
 
+#include <array>
 #include <cstdint>
 #include <stdexcept>
 #include <string>
@@ -64,6 +65,13 @@ class KmerCounter {
         const void* p = nullptr;
         check(kh_count_extract_device(c_, min_count, min_ext, &p, &n), "extract_device");
         return p;
+    }
+    // the k-mer spectrum: [c] = distinct k-mers seen exactly c times, [255] = 255 times or more (kh_count_histogram);
+    // kh_count_auto_min_count(h.data()) picks min_count at its valley
+    std::array<uint64_t, 256> histogram() {
+        std::array<uint64_t, 256> h{};
+        check(kh_count_histogram(c_, h.data()), "histogram");
+        return h;
     }
     kh_count_stats stats() {
         kh_count_stats s{};

@@ -16,6 +16,7 @@
 #pragma once
 
 #include <algorithm>
+#include <array>
 #include <cstdint>
 #include <exception>
 #include <stdexcept>
@@ -150,6 +151,19 @@ class CountCluster {
         std::string out(n * (uint64_t)(k_ + 4), '\0');
         count_must(kh_count_extract_lines(owned_[rank], min_count, min_ext, &out[0], n, &n), owned_[rank], "extract_lines");
         return out;
+    }
+
+    // After reduce(): the k-mer spectrum of everything reduced so far (kh_count_histogram).  Every k-mer has exactly one
+    // owner and the owned counters are bit-identical to one counter's, so the bin-by-bin sum of the owners' spectra is
+    // exact.  Reads counted since the last reduce are not in it.
+    std::array<uint64_t, 256> histogram() {
+        std::array<uint64_t, 256> sum{};
+        for (int r = 0; r < world_; ++r) {
+            std::array<uint64_t, 256> h{};
+            count_must(kh_count_histogram(owned_[r], h.data()), owned_[r], "histogram");
+            for (size_t c = 0; c < h.size(); ++c) sum[c] += h[c];
+        }
+        return sum;
     }
 
     // totals over all ranks: occurrences and read bytes counted (reduced or not), distinct k-mers reduced so far

@@ -285,6 +285,20 @@ const char* kh_count_last_error(kh_counter* c);
 uint64_t kh_count_record_bytes(int k);
 int kh_count_partition(kh_counter* c, int world, const void** records_dev_out, uint64_t* offsets_host_out);
 int kh_count_merge_device(kh_counter* c, const void* records_dev, uint64_t n);
+/* The k-mer spectrum, for choosing min_count (the two-column histogram `jellyfish histo` / GenomeScope use).
+ * hist[c], c = 1..254: the number of distinct k-mers counted exactly c times; hist[255]: those seen 255 times or more
+ * (the occurrence counter saturates there); hist[0] = 0.  So sum(hist) = n_distinct, and for every m the sum of
+ * hist[c] over c >= m is the number of records kh_count_extract*(m, any min_ext) reports.  Counters merged from other
+ * counters are covered like counted ones, so the spectrum of a sharded analysis is the bin-by-bin sum of its owners'.
+ * kh_count_histogram: hist_host_out has room for 256 uint64; one scan of the table.  Host-synchronous; returns
+ * KH_ERR_TABLE_FULL after a count that overflowed the table.
+ * kh_count_auto_min_count: the valley rule, a pure function of the 256 bins that needs no device.  Let v be the
+ * smallest c in 1..254 with hist[c+1] >= hist[c] (where the falling slope of erroneous k-mers stops).  The result is v
+ * when v >= 2 and some k-mer is counted v times or more; otherwise 2 (no falling slope, as for error-free reads or an
+ * empty table; or a spectrum that falls to zero without a second peak).  hist = NULL gives 2.  kh_count_extract* take
+ * the result like any other min_count. */
+int kh_count_histogram(kh_counter* c, uint64_t* hist_host_out);
+uint32_t kh_count_auto_min_count(const uint64_t* hist);
 
 /* Introspection for tests and debugging: device pointer and capacity of an internal buffer of a chunk table
  * ("link", "meta", "chunk_base", "seg_base", "chunk_cursor", "counters", ...; "caps" returns HOST numbers). */

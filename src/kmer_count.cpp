@@ -1,7 +1,8 @@
 // kmer_count -- reads -> the reference's k-mer file, or straight to contigs, on the B200 library.
 //
-//   kmer_count K reads_file kmer_file_out   [min_count [min_ext]]
-//   kmer_count K reads_file --contigs PREFIX [min_count [min_ext]]
+//   kmer_count K reads_file [--histo HISTO_FILE] kmer_file_out   [min_count [min_ext]]
+//   kmer_count K reads_file [--histo HISTO_FILE] --contigs PREFIX [min_count [min_ext]]
+//   kmer_count K reads_file --histo HISTO_FILE
 //
 // The first form writes what the reference's read_kmers parses (read_kmers.hpp:64-76: K bases, a blank, backward and
 // forward extension, '\n' per unique k-mer) -- the output of "the first preprocessing stage" the assignment assumes done
@@ -11,6 +12,11 @@
 //
 // reads_file: one read per line, FASTA or FASTQ (detected from the first byte; header / quality lines are blanked on
 // the host).  Bases are upper-case ACGT; anything else (N, ...) splits a read.  Defaults: min_count = min_ext = 2.
+//
+// --histo HISTO_FILE writes the k-mer spectrum (kh_count_histogram) in the two-column format of `jellyfish histo`, which
+// GenomeScope reads: "c n" per line for every count c in 1..255 with n > 0 distinct k-mers, ascending; 255 stands for
+// 255 or more.  With --histo alone nothing else is written.  min_count may be the word `auto`: the valley of the
+// spectrum (kh_count_auto_min_count).  Whenever the spectrum is computed, one more stdout line reports it.
 // Environment: KH_DEVICE, KH_LOAD_FACTOR (0.5), KH_COUNT_DISTINCT = distinct k-mers to size the table for, erroneous
 // ones included (default: half the input bytes).
 //
@@ -21,6 +27,7 @@
 // order; with --contigs, every rank's records go on its GPU into kh_sharded::Cluster (17 <= K <= 54) and rank r writes
 // PREFIX_r.dat.  Same k-mers, counters and contigs as P = 1, in another order.
 #include <algorithm>
+#include <array>
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -42,8 +49,27 @@ void must(int status, kh_table* t, const char* what) {
 }
 
 int usage() {
-    fprintf(stderr, "Usage: kmer_count K reads_file (kmer_file_out | --contigs PREFIX) [min_count [min_ext]]\n");
+    fprintf(stderr, "Usage: kmer_count K reads_file [--histo HISTO_FILE] [kmer_file_out | --contigs PREFIX] [min_count|auto [min_ext]]\n"
+                    "       (the output may be left out only with --histo)\n");
     return 1;
+}
+
+// The spectrum once counting is done: written to `histo` (if named), min_count resolved when it is `auto`, one line on
+// stdout.
+void spectrum(const std::array<uint64_t, 256>& hist, int k, const std::string& histo, bool auto_min_count, uint32_t& min_count) {
+    if (!histo.empty()) {
+        FILE* o = fopen(histo.c_str(), "wb");
+        if (o == nullptr) throw std::runtime_error("kmer_count: could not open " + histo);
+        for (size_t c = 1; c < hist.size(); ++c)
+            if (hist[c] && fprintf(o, "%zu %llu\n", c, (unsigned long long)hist[c]) < 0) throw std::runtime_error("kmer_count: short write to " + histo);
+        if (fclose(o) != 0) throw std::runtime_error("kmer_count: short write to " + histo);
+    }
+    uint64_t distinct = 0;
+    for (uint64_t n : hist) distinct += n;
+    const uint32_t valley = kh_count_auto_min_count(hist.data());
+    if (auto_min_count) min_count = valley;
+    printf("Spectrum of %llu distinct %d-mers%s%s: min_count %u, auto min_count %u\n", (unsigned long long)distinct, k,
+           histo.empty() ? "" : " written to ", histo.c_str(), min_count, valley);
 }
 
 // The file goes through in pieces of about `buffer` bytes that end on a line boundary (FASTA: before a header); each
@@ -74,7 +100,7 @@ template <class Sink> void read_pieces(FILE* f, size_t buffer, Sink sink) {
 }
 
 int count_sharded(FILE* f, int k, int ranks, uint64_t distinct, double lf, bool contigs, const std::string& out_name,
-                  uint32_t min_count, uint32_t min_ext) {
+                  const std::string& histo, bool auto_min_count, uint32_t min_count, uint32_t min_ext) {
     using clock = std::chrono::high_resolution_clock;
     const uint64_t batch = getenv("KH_COUNT_BATCH_BYTES") ? strtoull(getenv("KH_COUNT_BATCH_BYTES"), nullptr, 10) : 0;
     const size_t buffer = batch ? (size_t)std::min<uint64_t>(128u << 20, std::max<uint64_t>(batch, 4096)) : (128u << 20) + (1u << 20);
@@ -93,6 +119,8 @@ int count_sharded(FILE* f, int k, int ranks, uint64_t distinct, double lf, bool 
     printf("Counted %llu k-mer occurrences, %llu distinct %d-mers, from %llu bytes of reads in %lf s\n",
            (unsigned long long)cluster.n_occurrences(), (unsigned long long)cluster.n_distinct(), k,
            (unsigned long long)cluster.n_bytes(), std::chrono::duration<double>(t1 - t0).count());
+    if (!histo.empty() || auto_min_count) spectrum(cluster.histogram(), k, histo, auto_min_count, min_count);
+    if (out_name.empty()) return 0;
 
     if (!contigs) {
         FILE* o = fopen(out_name.c_str(), "wb");
@@ -143,10 +171,18 @@ int main(int argc, char** argv) {
     const int k = atoi(argv[1]);
     const std::string reads_file = argv[2];
     int a = 3;
-    const bool contigs = std::string(argv[a]) == "--contigs";
+    std::string histo;
+    if (std::string(argv[a]) == "--histo") {
+        if (++a >= argc) return usage();
+        histo = argv[a++];
+    }
+    if (histo.empty() && a >= argc) return usage();
+    const bool contigs = a < argc && std::string(argv[a]) == "--contigs";
     if (contigs && ++a >= argc) return usage();
-    const std::string out_name = argv[a++];
-    const uint32_t min_count = a < argc ? (uint32_t)atoi(argv[a++]) : 2u;
+    const std::string out_name = a < argc ? argv[a++] : "";              // empty: --histo alone
+    const bool auto_min_count = a < argc && std::string(argv[a]) == "auto";
+    uint32_t min_count = a < argc ? (auto_min_count ? 0u : (uint32_t)atoi(argv[a])) : 2u;
+    if (a < argc) ++a;
     const uint32_t min_ext = a < argc ? (uint32_t)atoi(argv[a++]) : 2u;
     if (k < 2 || k > 61) { fprintf(stderr, "kmer_count: K must be 2..61\n"); return 1; }
     const int device = getenv("KH_DEVICE") ? atoi(getenv("KH_DEVICE")) : 0;
@@ -162,7 +198,7 @@ int main(int argc, char** argv) {
     const int ranks = getenv("KH_RANKS") ? atoi(getenv("KH_RANKS")) : 1;
     if (ranks < 1 || ranks > 8) { fprintf(stderr, "kmer_count: KH_RANKS must be 1..8\n"); return 1; }
     if (ranks > 1 && contigs && (k < 17 || k > 54)) { fprintf(stderr, "kmer_count: --contigs with KH_RANKS > 1 needs 17 <= K <= 54\n"); return 1; }
-    if (ranks > 1) return count_sharded(f, k, ranks, distinct, lf, contigs, out_name, min_count, min_ext);
+    if (ranks > 1) return count_sharded(f, k, ranks, distinct, lf, contigs, out_name, histo, auto_min_count, min_count, min_ext);
     const auto t0 = std::chrono::high_resolution_clock::now();
     kh::KmerCounter counter(k, distinct, lf, device);
 
@@ -173,6 +209,8 @@ int main(int argc, char** argv) {
     printf("Counted %llu k-mer occurrences, %llu distinct %d-mers, from %llu bytes of reads in %lf s\n",
            (unsigned long long)st.n_occurrences, (unsigned long long)st.n_distinct, k, (unsigned long long)st.n_bytes,
            std::chrono::duration<double>(t1 - t0).count());
+    if (!histo.empty() || auto_min_count) spectrum(counter.histogram(), k, histo, auto_min_count, min_count);
+    if (out_name.empty()) return 0;
 
     if (!contigs) {
         const std::string lines = counter.extract_lines(min_count, min_ext);
