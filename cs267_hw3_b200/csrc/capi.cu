@@ -36,8 +36,6 @@ enum { EV_INS0, EV_INS1, EV_AS0, EV_WALK, EV_RANK, EV_AS1, EV_PACK0, EV_PACK1, E
 
 struct kh_table {
     int k = 0, W = 1, device = 0, pl = 0, pb = 0, slot_bytes = 8, per_bucket = 4;
-    int mlen = 0;                     // minimizer length of the in-table placement (0 = plain key hash; KH_LOCALITY=1 turns it on)
-    int olen = 0;                     // minimizer length of the owner-GPU function (0 = plain key hash; KH_OWNER_LOCALITY=0)
     double lf = 0.5;
     u64 n_expected = 0, nbuckets = 0;
     cudaStream_t stream = nullptr, own_stream = nullptr, copy_stream = nullptr;
@@ -53,10 +51,7 @@ struct kh_table {
     bool chunk_attr_set = false;
     int debug_cap_pct = 100;          // KH_DEBUG_CAP_PCT: scale the grouping buffers' capacities (tests force the overflow paths)
     int partition_mode = -1;          // -1 auto, 0 never, 1 always (KH_PARTITION)
-    u64 part_bytes = 16ull << 20;     // table bytes per partition (KH_PART_MB)
     bool part_attr_set = false;
-    int ins_mode = 1;                 // KH_INS_MODE: 0 read-then-CAS, 1 CAS-first
-    int warm_ahead = 1;               // KH_WARM_AHEAD: table regions prefetched ahead of the inserts (0 = off)
     Counters* d_ctr = nullptr;
     Counters* h_ctr = nullptr;
     DevBuf link, seglen, tmp, contig_len, contig_pre, contig_off, out;
@@ -204,11 +199,11 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
     u32 part_shift = 0, nparts = 1, bpp = 1;
     u64 part_cap = 0;
     if (part) {
-        while ((32ull << part_shift) < t->part_bytes) ++part_shift;
+        while ((32ull << part_shift) < kPartBytes) ++part_shift;
         while (((t->nbuckets - 1) >> part_shift) + 1 > (u64)kMaxParts) ++part_shift;
         nparts = (u32)(((t->nbuckets - 1) >> part_shift) + 1);
-        // a partition's expected share of n plus slack (supermers move as a unit, so the spread is a few times
-        // the binomial sigma), rounded to whole insert tiles; overflow falls back to a direct insert
+        // a partition's expected share of n plus slack (24 binomial sigmas), rounded to whole insert tiles; overflow
+        // falls back to a direct insert
         const double share = (double)n * (double)std::min<u64>(t->nbuckets, 1ull << part_shift) / (double)t->nbuckets;
         part_cap = (u64)(share + 24.0 * std::sqrt(share + 1.0) + 64.0) * t->debug_cap_pct / 100;
         part_cap = (part_cap + kInsTile - 1) / kInsTile * kInsTile;
@@ -247,15 +242,14 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
         KH_TRY(ensure(t, t->chunk_cursor, nchunks * sizeof(u32)));
         KH_TRY(ensure(t, t->overflow, (u64)overflow_cap * sizeof(V)));
         if (!t->chunk_attr_set) {
-            KH_CUDA(t, cudaFuncSetAttribute(build_chunks_kernel<W, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kChunkBuckets * 32)));
-            KH_CUDA(t, cudaFuncSetAttribute(build_chunks_kernel<W, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kChunkBuckets * 32)));
+            KH_CUDA(t, cudaFuncSetAttribute(build_chunks_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kChunkBuckets * 32)));
             t->chunk_attr_set = true;
         }
     }
     if (record_start) KH_CUDA(t, cudaEventRecord(t->ev[EV_INS0], t->stream));
     if (!part) {
         insert_kernel<W><<<(unsigned)ntiles, kInsThreads, (size_t)kInsTile * t->pb + kStageSlack, t->stream>>>(
-            recs, n, t->k, t->mlen, static_cast<V*>(t->table), t->nbuckets, static_cast<u32*>(t->mask.p),
+            recs, n, t->k, static_cast<V*>(t->table), t->nbuckets, static_cast<u32*>(t->mask.p),
             static_cast<u32*>(t->tile_counts.p), t->d_ctr);
     } else if (chunked) {
         KH_CUDA(t, cudaMemsetAsync(t->part_cursor.p, 0, kMaxParts * sizeof(u32), t->stream));
@@ -263,40 +257,32 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
         KH_CUDA(t, cudaMemsetAsync(&t->d_ctr->n_outbox, 0, sizeof(u32), t->stream));
         const u64 pblocks = (n + kPartTile - 1) / kPartTile;
         partition_kernel<W><<<(unsigned)pblocks, kPartThreads, partition_smem(W, nparts, t->pb), t->stream>>>(
-            recs, n, t->k, t->mlen, t->nbuckets, part_shift, nparts, part_cap, static_cast<u32*>(t->part_cursor.p),
+            recs, n, t->k, t->nbuckets, part_shift, nparts, part_cap, static_cast<u32*>(t->part_cursor.p),
             static_cast<V*>(t->grouped.p), static_cast<V*>(t->table), static_cast<u32*>(t->mask.p),
             static_cast<u32*>(t->tile_counts.p), static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
         subpartition_kernel<W><<<nparts * bpp2, kSubThreads, sub_smem, t->stream>>>(
-            static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), 0, part_cap, bpp2, kChunkShift,
-            1u << (part_shift - kChunkShift), t->k, t->mlen, t->nbuckets, chunk_cap, static_cast<u32*>(t->chunk_cursor.p), static_cast<V*>(t->fine.p),
+            static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), part_cap, bpp2, kChunkShift,
+            1u << (part_shift - kChunkShift), t->nbuckets, chunk_cap, static_cast<u32*>(t->chunk_cursor.p), static_cast<V*>(t->fine.p),
             static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
-        build_chunks_kernel<W, false><<<(unsigned)nchunks, kBuildThreads, kChunkBuckets * 32, t->stream>>>(
+        build_chunks_kernel<W><<<(unsigned)nchunks, kBuildThreads, kChunkBuckets * 32, t->stream>>>(
             static_cast<const V*>(t->fine.p), static_cast<const u32*>(t->chunk_cursor.p), chunk_cap, static_cast<V*>(t->table),
-            t->nbuckets, t->k, t->mlen, t->table_dirty ? 1 : 0, static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr, BoundaryReg{});
-        insert_overflow_kernel<W><<<64, 256, 0, t->stream>>>(static_cast<const V*>(t->overflow.p), overflow_cap, t->k, t->mlen,
+            t->nbuckets, t->table_dirty ? 1 : 0, static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
+        insert_overflow_kernel<W><<<64, 256, 0, t->stream>>>(static_cast<const V*>(t->overflow.p), overflow_cap,
                                                             static_cast<V*>(t->table), t->nbuckets, t->d_ctr);
     } else {
         KH_CUDA(t, cudaMemsetAsync(t->part_cursor.p, 0, kMaxParts * sizeof(u32), t->stream));
-        const u32 ahead = (u32)std::max(0, t->warm_ahead);
-        if (ahead) {
-            const u64 warm_buckets = std::min<u64>(t->nbuckets, (u64)ahead << part_shift);
-            warm_kernel<<<(unsigned)t->sm_count * 4, 256, 0, t->stream>>>(static_cast<const char*>(t->table),
-                                                                         (warm_buckets * 32 + 127) >> 7);
-        }
+        const u64 warm_buckets = std::min<u64>(t->nbuckets, (u64)kWarmAhead << part_shift);
+        warm_kernel<<<(unsigned)t->sm_count * 4, 256, 0, t->stream>>>(static_cast<const char*>(t->table),
+                                                                     (warm_buckets * 32 + 127) >> 7);
         const u64 pblocks = (n + kPartTile - 1) / kPartTile;
         partition_kernel<W><<<(unsigned)pblocks, kPartThreads, partition_smem(W, nparts, t->pb), t->stream>>>(
-            recs, n, t->k, t->mlen, t->nbuckets, part_shift, nparts, part_cap, static_cast<u32*>(t->part_cursor.p),
+            recs, n, t->k, t->nbuckets, part_shift, nparts, part_cap, static_cast<u32*>(t->part_cursor.p),
             static_cast<V*>(t->grouped.p), static_cast<V*>(t->table), static_cast<u32*>(t->mask.p),
             static_cast<u32*>(t->tile_counts.p), static_cast<V*>(nullptr), 0u, t->d_ctr);
         const unsigned iblocks = nparts * bpp;
-        if (t->ins_mode == 0)
-            insert_slots_kernel<W, 0><<<iblocks, kInsThreads, 0, t->stream>>>(
-                static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), part_cap, bpp, nparts,
-                part_shift, ahead, t->k, t->mlen, static_cast<V*>(t->table), t->nbuckets, t->d_ctr);
-        else
-            insert_slots_kernel<W, 1><<<iblocks, kInsThreads, 0, t->stream>>>(
-                static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), part_cap, bpp, nparts,
-                part_shift, ahead, t->k, t->mlen, static_cast<V*>(t->table), t->nbuckets, t->d_ctr);
+        insert_slots_kernel<W><<<iblocks, kInsThreads, 0, t->stream>>>(
+            static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), part_cap, bpp, nparts,
+            part_shift, static_cast<V*>(t->table), t->nbuckets, t->d_ctr);
     }
     t->table_dirty = true;
     t->n_launches += !part ? 1 : (chunked ? 4 : 3);
@@ -388,7 +374,7 @@ int assemble_impl(kh_table* t) {
     wp.link = static_cast<u64*>(t->link.p); wp.seglen = static_cast<unsigned char*>(t->seglen.p);
     wp.tmp = static_cast<unsigned char*>(t->tmp.p); wp.ctr = t->d_ctr;
     wp.n_starts = (u32)n_starts; wp.n_split = (u32)n_split; wp.split_shift = t->split_shift;
-    wp.seg_chars = t->seg_chars; wp.seg_cap = (u32)seg_cap; wp.k = t->k; wp.m = t->mlen;
+    wp.seg_chars = t->seg_chars; wp.seg_cap = (u32)seg_cap; wp.k = t->k;
     walk_kernel<W><<<walk_blocks, kWalkThreads, 0, t->stream>>>(wp);
     KH_CUDA(t, cudaGetLastError());
     KH_CUDA(t, cudaEventRecord(t->ev[EV_WALK], t->stream));
@@ -1026,7 +1012,9 @@ int kh_create(int k, uint64_t n_expected, double load_factor, int device, kh_tab
 
     const long double slots = (long double)std::max<uint64_t>(n_expected, 1) / (long double)load_factor;
     t->nbuckets = std::max<u64>(16, (u64)(slots / t->per_bucket) + 1);
-    t->nbuckets = (t->nbuckets + 15) / 16 * 16;       // whole placement regions (slot.cuh RegionOf)
+    // Rounded up to a multiple of 16 buckets.  The size is visible to callers (kh_stats n_buckets / n_slots, the slot
+    // layout behind kh_get_device_view), so this rounding stays part of the sizing rule.
+    t->nbuckets = (t->nbuckets + 15) / 16 * 16;
     t->table_bytes = use_ct ? 0 : (size_t)t->nbuckets * 32;       // a chunk table is allocated by ct_setup
     int rc = KH_OK;
     auto ck = [&](cudaError_t e) { if (e != cudaSuccess && rc == KH_OK) { rc = e == cudaErrorMemoryAllocation ? KH_ERR_NOMEM : KH_ERR_CUDA; t->err = cudaGetErrorString(e); } };
@@ -1049,18 +1037,11 @@ int kh_create(int k, uint64_t n_expected, double load_factor, int device, kh_tab
     memset(t->h_ctr, 0, sizeof(Counters));
     int v = env_int("KH_SPLIT_BUCKETS", 0);
     if (v > 0 && set_option(t, "split_buckets", v) != KH_OK) fprintf(stderr, "libkh_b200: ignoring KH_SPLIT_BUCKETS=%d\n", v);
-    t->mlen = env_int("KH_LOCALITY", 0) ? minimizer_len(k) : 0;
-    t->olen = env_int("KH_OWNER_LOCALITY", 1) ? owner_minimizer_len(k) : 0;
-    if (env_int("KH_OWNER_MLEN", 0) > 0) t->olen = std::min(k, env_int("KH_OWNER_MLEN", 0));
     t->partition_mode = env_int("KH_PARTITION", -1);
     // measured: the shared-memory build wins for 64-bit slots (2.85 vs 3.03 ms) and loses for 128-bit slots
     // (4.6 vs 4.1 ms: twice the bytes through the two grouping passes), so it is the default only for K <= 29
     t->build_mode = env_int("KH_BUILD", t->W == 1 ? 1 : 0);
     t->debug_cap_pct = std::max(1, env_int("KH_DEBUG_CAP_PCT", 100));
-    t->ins_mode = env_int("KH_INS_MODE", 1);
-    t->warm_ahead = env_int("KH_WARM_AHEAD", 1);
-    v = env_int("KH_PART_MB", 0);
-    if (v > 0) t->part_bytes = (u64)v << 20;
     v = env_int("KH_SEG_CHARS", 0);
     if (v > 0 && set_option(t, "seg_chars", v) != KH_OK) fprintf(stderr, "libkh_b200: ignoring KH_SEG_CHARS=%d\n", v);
     if (use_ct) {
@@ -1259,10 +1240,10 @@ int kh_find_device(kh_table* t, const void* pkmers_dev, uint64_t n, void* pairs_
         return KH_OK;
     }
     if (t->W == 1)
-        find_kernel<1><<<blocks, 256, 0, t->stream>>>(static_cast<const u64*>(t->table), t->nbuckets, t->k, t->mlen,
+        find_kernel<1><<<blocks, 256, 0, t->stream>>>(static_cast<const u64*>(t->table), t->nbuckets, t->k,
             static_cast<const unsigned char*>(pkmers_dev), n, static_cast<unsigned char*>(pairs_dev_out), found_dev_out);
     else
-        find_kernel<2><<<blocks, 256, 0, t->stream>>>(static_cast<const u128*>(t->table), t->nbuckets, t->k, t->mlen,
+        find_kernel<2><<<blocks, 256, 0, t->stream>>>(static_cast<const u128*>(t->table), t->nbuckets, t->k,
             static_cast<const unsigned char*>(pkmers_dev), n, static_cast<unsigned char*>(pairs_dev_out), found_dev_out);
     KH_CUDA(t, cudaGetLastError());
     return KH_OK;
@@ -1421,7 +1402,7 @@ int kh_get_device_view(kh_table* t, kh_device_view* out) {
     if (!t || !out) return KH_ERR_ARG;
     if (t->ct.on) return fail(t, KH_ERR_ARG, "kh_get_device_view: a chunk table has no single-record device interface (KH_CT=0 forces a plain table)");
     out->table = t->table; out->n_buckets = t->nbuckets; out->k = t->k; out->slot_bytes = t->slot_bytes;
-    out->placement_m = t->mlen; out->device = t->device;
+    out->placement_m = 0; out->device = t->device;
     t->table_dirty = true;              // the caller may insert behind our back: the next bulk insert must not assume an empty table
     return KH_OK;
 }

@@ -33,10 +33,11 @@ constexpr u64 kKcMinLaunch = 4ull << 20;                    // grow rather than 
 
 // Pass 1 compacts the tile's positions that hold a k-mer into a list (reads end every ~150 characters and K - 1
 // positions before every end hold none: a third of the lanes would idle through the table code otherwise); pass 2 runs
-// over the list with full warps (2.22 -> 1.69 ms for 52.7 M occurrences of 51-mers).  PF (off by default): the slot of a
-// thread's next occurrence is prefetched into L2 one iteration ahead -- measured, no gain: the kernel is issue-bound.
-template <int W, bool PF, int MINB>
-__global__ void __launch_bounds__(kKcThreads, MINB)
+// over the list with full warps (2.22 -> 1.69 ms for 52.7 M occurrences of 51-mers).  A software prefetch of a thread's
+// next occurrence one iteration ahead, and 6 instead of 8 blocks per SM for 128-bit keys, were measured with no gain:
+// the kernel is issue-bound.
+template <int W>
+__global__ void __launch_bounds__(kKcThreads, 8)
 kc_count_kernel(const unsigned char* __restrict__ buf, u64 n, u64 p_begin, u64 p_end, u64* __restrict__ table, u64 n_slots, int k,
                 KcCounters* ctr) {
     __shared__ u32 s_code[kKcWords], s_inv[kKcWords];
@@ -63,38 +64,12 @@ kc_count_kernel(const unsigned char* __restrict__ buf, u64 n, u64 p_begin, u64 p
     // a table that has overflowed stays wrong whatever follows: later blocks do not probe it slot by slot any more
     const u32 cnt = *reinterpret_cast<volatile u32*>(&ctr->errors) ? 0u : s_n;
     u32 fresh = 0, fail = 0;
-    if (!PF) {
 #pragma unroll 1
-        for (u32 i = threadIdx.x; i < cnt; i += kKcThreads) {
-            const KcOcc o = kc_position(s_code, s_inv, s_list[i], k);
-            bool f;
-            if (kc_upsert<W>(table, n_slots, o, kc_home(o.key_hi, o.key_lo, n_slots), f)) fresh += f ? 1u : 0u;
-            else ++fail;
-        }
-    } else {
-        u32 i = threadIdx.x;
-        KcOcc o = {};
-        u64 home = 0;
-        if (i < cnt) {
-            o = kc_position(s_code, s_inv, s_list[i], k);
-            home = kc_home(o.key_hi, o.key_lo, n_slots);
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(table + home * (u64)KcSlot<W>::kWords));
-        }
-#pragma unroll 1
-        while (i < cnt) {
-            const u32 i2 = i + kKcThreads;
-            KcOcc o2 = {};
-            u64 home2 = 0;
-            if (i2 < cnt) {
-                o2 = kc_position(s_code, s_inv, s_list[i2], k);
-                home2 = kc_home(o2.key_hi, o2.key_lo, n_slots);
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(table + home2 * (u64)KcSlot<W>::kWords));
-            }
-            bool f;
-            if (kc_upsert<W>(table, n_slots, o, home, f)) fresh += f ? 1u : 0u;
-            else ++fail;
-            o = o2; home = home2; i = i2;
-        }
+    for (u32 i = threadIdx.x; i < cnt; i += kKcThreads) {
+        const KcOcc o = kc_position(s_code, s_inv, s_list[i], k);
+        bool f;
+        if (kc_upsert<W>(table, n_slots, o, kc_home(o.key_hi, o.key_lo, n_slots), f)) fresh += f ? 1u : 0u;
+        else ++fail;
     }
     __syncwarp();
     fresh = __reduce_add_sync(kFull, fresh);
@@ -322,12 +297,10 @@ struct kh_counter {
     u32 n_launches = 0;
     float ms_count = 0.f, ms_extract = 0.f;
     bool have_count = false;
-    bool prefetch = false;            // KH_COUNT_PREFETCH=1: software prefetch of the next occurrence's slot (measured: no gain, the kernel is issue-bound)
     bool may_grow = true;             // KH_COUNT_GROW=0: a full table is an error instead of a reason to grow
     double lf = 0.5;
     u32 n_grows = 0;
     u64 distinct_ub = 0;              // host-side upper bound of the distinct count: every launched position counted as new
-    int min_blocks = 8;               // KH_COUNT_BLOCKS=6: 128-bit keys at 40 registers / 6 blocks per SM instead of 32 / 8
     std::string err;
 };
 
@@ -417,15 +390,8 @@ int kc_launch_count(kh_counter* c, const unsigned char* buf, u64 n, u64 p_begin,
     const u64 blocks = (span + kKcTile - 1) / kKcTile;
     if (blocks > 0x7FFFFFFFull) return kc_fail(c, KH_ERR_ARG, "kh_count_reads_device: at most 2^42 bytes per call");
     const unsigned g = (unsigned)blocks;
-#define KC_LAUNCH(W_, PF_, MB_) kc_count_kernel<W_, PF_, MB_><<<g, kKcThreads, 0, c->stream>>>(buf, n, p_begin, p_end, c->table, c->n_slots, c->k, c->d_ctr)
-    if (c->W == 1) {
-        if (c->prefetch) KC_LAUNCH(1, true, 8); else KC_LAUNCH(1, false, 8);
-    } else if (c->min_blocks == 8) {                        // 32 registers (a few spilled bytes), 8 blocks per SM
-        if (c->prefetch) KC_LAUNCH(2, true, 8); else KC_LAUNCH(2, false, 8);
-    } else {                                                // 40 registers, 6 blocks per SM
-        if (c->prefetch) KC_LAUNCH(2, true, 6); else KC_LAUNCH(2, false, 6);
-    }
-#undef KC_LAUNCH
+    if (c->W == 1) kc_count_kernel<1><<<g, kKcThreads, 0, c->stream>>>(buf, n, p_begin, p_end, c->table, c->n_slots, c->k, c->d_ctr);
+    else kc_count_kernel<2><<<g, kKcThreads, 0, c->stream>>>(buf, n, p_begin, p_end, c->table, c->n_slots, c->k, c->d_ctr);
     KC_CUDA(c, cudaGetLastError());
     ++c->n_launches;
     return KH_OK;
@@ -446,8 +412,6 @@ int kh_count_create(int k, uint64_t n_distinct_expected, double load_factor, int
     }
     kh_counter* c = new kh_counter();
     c->k = k; c->W = kc_slot_words(k); c->device = device; c->pb = (k + 3) / 4 + 2;
-    if (const char* e = getenv("KH_COUNT_PREFETCH")) c->prefetch = atoi(e) != 0;
-    if (const char* e = getenv("KH_COUNT_BLOCKS")) c->min_blocks = atoi(e) == 6 ? 6 : 8;
     if (const char* e = getenv("KH_COUNT_GROW")) c->may_grow = atoi(e) != 0;
     c->lf = load_factor;
     const double want = (double)std::max<uint64_t>(n_distinct_expected, 1) / load_factor;

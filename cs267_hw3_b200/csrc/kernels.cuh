@@ -11,8 +11,8 @@
 //      rank_kernel            pointer jumping over the segment list (cooperative launch)
 //   K6 emit_segments_kernel / emit_heads_kernel   contig text             (read_kmers.hpp:81-92)
 //
-// All of it is HBM-bound integer work: no tensor cores, no floating point.  The multi-GPU kernels are in
-// sharded.cuh.
+// All of it is HBM-bound integer work: no tensor cores, no floating point.  The multi-GPU path uses the chunk
+// table (ctable.cuh).
 #pragma once
 #include <cooperative_groups.h>
 
@@ -159,7 +159,7 @@ __device__ __forceinline__ int insert_one(typename Slot<W>::value_t* table, u64 
 
 template <int W>
 __global__ void __launch_bounds__(kInsThreads)
-insert_kernel(const unsigned char* __restrict__ recs, u64 n, int k, int m,
+insert_kernel(const unsigned char* __restrict__ recs, u64 n, int k,
               typename Slot<W>::value_t* table, u64 nbuckets,
               u32* __restrict__ start_mask, u32* __restrict__ tile_starts, Counters* ctr) {
     typedef Slot<W> S;
@@ -186,7 +186,7 @@ insert_kernel(const unsigned char* __restrict__ recs, u64 n, int k, int m,
         v[r] = S::zero();
         if (live[r]) v[r] = S::from_record_staged(s_rec + j * pb, k, pl, ok);
         if (!ok) { err |= kErrBadInput; live[r] = false; }
-        b[r] = live[r] ? place_bucket<W>(v[r], k, m, nbuckets) : 0;
+        b[r] = live[r] ? place_bucket<W>(v[r], nbuckets) : 0;
         if (live[r]) load256_cg(table + b[r] * S::kPerBucket, q[r]);      // 4 independent sector reads in flight
         // kmer_hash.cpp:27-31: remember which records start a contig, by position in the input
         const u32 bal = __ballot_sync(kFullMask, live[r] && S::back(v[r]) == kExtF);
@@ -260,6 +260,7 @@ __device__ __forceinline__ u64 block_exclusive_scan(u64 x, u64* s_warp, u64& blo
 // counting-sort pass; the insert kernel then sweeps the grouped array front to back, and the blocks
 // in flight at any moment touch only a couple of regions.  The table semantics are unchanged
 // (same buckets, same probing) -- only the order of insertion differs.
+constexpr u64 kPartBytes = 16ull << 20;    // table bytes per partition (more when the table needs over kMaxParts of them)
 constexpr int kMaxParts = 1024;
 constexpr int kPartThreads = 256;
 constexpr int kPartPerThread = 8;
@@ -275,7 +276,7 @@ constexpr int kPartTile = kPartThreads * kPartPerThread;     // 2048 records per
 #endif
 template <int W>
 __global__ void __launch_bounds__(kPartThreads, KH_PART_MIN_BLOCKS)
-partition_kernel(const unsigned char* __restrict__ recs, u64 n, int k, int m, u64 nbuckets, u32 part_shift, u32 nparts,
+partition_kernel(const unsigned char* __restrict__ recs, u64 n, int k, u64 nbuckets, u32 part_shift, u32 nparts,
                  u64 part_cap, u32* __restrict__ cursor, typename Slot<W>::value_t* __restrict__ grouped,
                  typename Slot<W>::value_t* table, u32* __restrict__ start_mask, u32* __restrict__ tile_starts,
                  typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap, Counters* ctr) {
@@ -313,7 +314,7 @@ partition_kernel(const unsigned char* __restrict__ recs, u64 n, int k, int m, u6
         if (live) v[r] = S::from_record_staged(s_rec + j * pb, k, pl, ok);
         if (!ok) { err |= kErrBadInput; live = false; }
         if (live) {
-            pid[r] = (u32)(place_bucket<W>(v[r], k, m, nbuckets) >> part_shift);
+            pid[r] = (u32)(place_bucket<W>(v[r], nbuckets) >> part_shift);
             rk[r] = atomicAdd(&s_hist[pid[r]], 1u);
         }
         // kmer_hash.cpp:27-31: which records start a contig, by position in the input
@@ -370,7 +371,7 @@ partition_kernel(const unsigned char* __restrict__ recs, u64 n, int k, int m, u6
             else atomicOr(&s_err, kErrInternal);
         } else {                                           // partition buffer full: insert right here
             const V val = s_sorted[pos];
-            const u64 b = place_bucket<W>(val, k, m, nbuckets);
+            const u64 b = place_bucket<W>(val, nbuckets);
             u64 q[4];
             load256_cg(table + b * S::kPerBucket, q);
             const int rc = insert_one<W>(table, nbuckets, b, val, q);
@@ -410,13 +411,11 @@ constexpr int kSubTile = kSubThreads * kSubPerThread;  // 2048 slot values per b
 // After the block-wide rank/reserve each thread writes its values straight to their destination run (L2 merges
 // the sector writes); staging a sorted copy in shared memory first was measured slower (2.71 vs 2.52 ms insert).
 // The kernel splits input partition `part` (values whose home lies in units [part*nsub, (part+1)*nsub), a unit being
-// 2^unit_shift buckets) into one buffer per unit.  Level 2 of the chunked build uses it with unit = chunk; the sharded
-// path also uses it as level 1 on the flat array of received slot values (part_cursor == nullptr: one input
-// "partition" of n_flat values, unit = 8 MB table region).
+// 2^unit_shift buckets) into one buffer per unit.  Level 2 of the chunked build uses it with unit = chunk.
 template <int W>
 __global__ void __launch_bounds__(kSubThreads, 4)
-subpartition_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const u32* __restrict__ part_cursor, u64 n_flat,
-                    u64 part_cap, u32 blocks_per_part, u32 unit_shift, u32 nsub, int k, int m, u64 nbuckets,
+subpartition_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const u32* __restrict__ part_cursor,
+                    u64 part_cap, u32 blocks_per_part, u32 unit_shift, u32 nsub, u64 nbuckets,
                     u32 chunk_cap, u32* __restrict__ chunk_cursor, typename Slot<W>::value_t* __restrict__ fine,
                     typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap, Counters* ctr) {
     typedef Slot<W> S;
@@ -425,7 +424,7 @@ subpartition_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const
     u32* s_hist = reinterpret_cast<u32*>(s_raw);                       // nsub <= 1024 units per input partition
     u32* s_gbase = s_hist + nsub;
     const u32 part = blockIdx.x / blocks_per_part, jblk = blockIdx.x % blocks_per_part;
-    const u64 n = part_cursor ? min((u64)part_cursor[part], part_cap) : n_flat;
+    const u64 n = min((u64)part_cursor[part], part_cap);
     const u64 base = (u64)jblk * kSubTile;
     if (base >= n) return;
     const V* __restrict__ src = grouped + (u64)part * part_cap;
@@ -443,7 +442,7 @@ subpartition_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const
     for (int r = 0; r < kSubPerThread; ++r) {
         sid[r] = 0xFFFFFFFFu;
         if (!S::empty(v[r])) {
-            const u64 chunk = place_bucket<W>(v[r], k, m, nbuckets) >> unit_shift;
+            const u64 chunk = place_bucket<W>(v[r], nbuckets) >> unit_shift;
             sid[r] = min((u32)(chunk - first_chunk), nsub - 1u);
             rk[r] = atomicAdd(&s_hist[sid[r]], 1u);
         }
@@ -501,27 +500,16 @@ __device__ __forceinline__ int build_insert_one(typename Slot<W>::value_t* s_tab
     return kInsFull;                      // the probe sequence leaves the chunk
 }
 
-// Sharded tables also register their BOUNDARY starts here (the k-mers a local walk starts from: backward ext 'F', or
-// a predecessor that another GPU owns).  That is a pure function of the slot value, so it is decided in one dense
-// sweep over the finished chunk -- every lane busy -- instead of per insert; ids are handed out with shared-memory
-// counters and ONE global atomic per chunk.  Requires a clean table (every occupied slot of the chunk is new).
-struct BoundaryReg {
-    u32* seg_of_slot;       // slot position -> boundary id
-    void* boundary_list;    // boundary id -> slot value
-    u32 bcap;
-    int rank, world, mo;
-};
-
-template <int W, bool SHARD>
+template <int W>
 __global__ void __launch_bounds__(kBuildThreads)
 build_chunks_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u32* __restrict__ chunk_cursor, u32 chunk_cap,
-                    typename Slot<W>::value_t* table, u64 nbuckets, int k, int m, int load_existing,
-                    typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap, Counters* ctr, const BoundaryReg br) {
+                    typename Slot<W>::value_t* table, u64 nbuckets, int load_existing,
+                    typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap, Counters* ctr) {
     typedef Slot<W> S;
     typedef typename S::value_t V;
     extern __shared__ __align__(16) unsigned char s_raw[];
     V* s_tab = reinterpret_cast<V*>(s_raw);                            // kChunkBuckets * 32 bytes
-    __shared__ u32 s_inserted, s_dups, s_nbound, s_bbase;
+    __shared__ u32 s_inserted, s_dups;
     const u64 b0 = (u64)blockIdx.x << kChunkShift;
     const u32 nb = (u32)min((u64)kChunkBuckets, nbuckets - b0);
     const u32 nvec = nb * 2;                                           // 16-byte vectors in this chunk
@@ -536,7 +524,7 @@ build_chunks_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u3
         const u32 i = threadIdx.x + r * kBuildThreads;
         v[r] = i < cnt ? recs[i] : S::zero();
     }
-    if (threadIdx.x == 0) { s_inserted = 0; s_dups = 0; s_nbound = 0; }
+    if (threadIdx.x == 0) { s_inserted = 0; s_dups = 0; }
     if (load_existing) for (u32 i = threadIdx.x; i < nvec; i += blockDim.x) s4[i] = g4[i];
     else for (u32 i = threadIdx.x; i < nvec; i += blockDim.x) s4[i] = make_uint4(0, 0, 0, 0);
     __syncthreads();
@@ -551,7 +539,7 @@ build_chunks_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u3
 #pragma unroll
         for (int r = 0; r < kBuildBatch; ++r) {
             if (S::empty(v[r])) continue;
-            const u32 b = (u32)(place_bucket<W>(v[r], k, m, nbuckets) - b0);      // local bucket, < nb by construction
+            const u32 b = (u32)(place_bucket<W>(v[r], nbuckets) - b0);      // local bucket, < nb by construction
             const int rc = build_insert_one<W>(s_tab, nb, b, v[r]);
             inserted += (rc == kInsInserted);
             dups += (rc == kInsDuplicate);
@@ -576,56 +564,18 @@ build_chunks_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u3
         if (s_inserted) atomicAdd(&ctr->n_inserted, (u64)s_inserted);
         if (s_dups) atomicAdd(&ctr->n_duplicates, (u64)s_dups);
     }
-    if (SHARD) {
-        constexpr int kSweep = (int)(kChunkBuckets * S::kPerBucket) / kBuildThreads;      // slots per thread
-        const u32 nslots = nb * S::kPerBucket;
-        u32 is_bnd = 0;                        // bit r: slot threadIdx.x + r * kBuildThreads is a boundary start
-        unsigned short lid[kSweep];            // its id within this chunk
-#pragma unroll
-        for (int r = 0; r < kSweep; ++r) {
-            const u32 i = threadIdx.x + r * kBuildThreads;
-            bool bnd = false;
-            if (i < nslots) {
-                const V v = s_tab[i];
-                if (!S::empty(v)) {
-                    bnd = S::back(v) == kExtF;
-                    if (!bnd && br.world > 1) bnd = owner_of<W>(S::prev_key(v, k), br.world, k, br.mo) != (u32)br.rank;
-                }
-            }
-            const u32 bal = __ballot_sync(kFullMask, bnd);
-            u32 first = 0;
-            if (lane_id() == 0 && bal) first = atomicAdd(&s_nbound, (u32)__popc(bal));
-            first = __shfl_sync(kFullMask, first, 0);
-            lid[r] = (unsigned short)(first + __popc(bal & ((1u << lane_id()) - 1u)));
-            is_bnd |= (bnd ? 1u : 0u) << r;
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) s_bbase = s_nbound ? atomicAdd(&ctr->n_boundary, s_nbound) : 0u;
-        __syncthreads();
-        V* __restrict__ blist = static_cast<V*>(br.boundary_list);
-        u32 err = 0;
-#pragma unroll
-        for (int r = 0; r < kSweep; ++r) {
-            if (!((is_bnd >> r) & 1u)) continue;
-            const u32 i = threadIdx.x + r * kBuildThreads;
-            const u32 id = s_bbase + lid[r];
-            if (id < br.bcap) { blist[id] = s_tab[i]; br.seg_of_slot[b0 * S::kPerBucket + i] = id; }
-            else err = kErrInternal;
-        }
-        if (err) atomicOr(&ctr->errors, err);
-    }
 }
 
 // the few records the chunk build could not place: ordinary global insert, after every chunk is final
 template <int W>
 __global__ void __launch_bounds__(256)
-insert_overflow_kernel(const typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap, int k, int m,
+insert_overflow_kernel(const typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap,
                        typename Slot<W>::value_t* table, u64 nbuckets, Counters* ctr) {
     typedef Slot<W> S;
     const u32 n = min(ctr->n_outbox, overflow_cap);
     for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const typename S::value_t v = overflow[i];
-        const u64 b = place_bucket<W>(v, k, m, nbuckets);
+        const u64 b = place_bucket<W>(v, nbuckets);
         u64 q[4];
         load256_cg(table + b * S::kPerBucket, q);
         const int rc = insert_one<W>(table, nbuckets, b, v, q);
@@ -642,16 +592,15 @@ warm_kernel(const char* __restrict__ base, u64 nlines) {
         asm volatile("prefetch.global.L2 [%0];" ::"l"(base + (l << 7)));
 }
 
-#ifndef KH_INS_SLOTS_MIN_BLOCKS
-#define KH_INS_SLOTS_MIN_BLOCKS 6          // latency-bound kernel: trade registers for resident warps
-#endif
-// pass 3: insert pre-converted slot values (grouped by partition, so the table traffic is L2-resident).
-// MODE 0: read the bucket, then CAS the first empty slot.  MODE 1: CAS slot 0 of the home bucket blind
-// (4 independent atomics in flight per thread) and fall back to read + CAS only when it is taken.
-template <int W, int MODE>
-__global__ void __launch_bounds__(kInsThreads, KH_INS_SLOTS_MIN_BLOCKS)
+constexpr int kInsSlotsMinBlocks = 6;      // latency-bound kernel: trade registers for resident warps
+constexpr u32 kWarmAhead = 1;              // table regions (partitions) prefetched ahead of the inserts
+// pass 3: insert pre-converted slot values (grouped by partition, so the table traffic is L2-resident).  CAS slot 0
+// of the home bucket blind (4 independent atomics in flight per thread) and fall back to read + CAS only when it is
+// taken.
+template <int W>
+__global__ void __launch_bounds__(kInsThreads, kInsSlotsMinBlocks)
 insert_slots_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const u32* __restrict__ cursor,
-                    u64 part_cap, u32 blocks_per_part, u32 nparts, u32 part_shift, u32 warm_ahead, int k, int m,
+                    u64 part_cap, u32 blocks_per_part, u32 nparts, u32 part_shift,
                     typename Slot<W>::value_t* table, u64 nbuckets, Counters* ctr) {
     typedef Slot<W> S;
     typedef typename S::value_t V;
@@ -662,12 +611,12 @@ insert_slots_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const
     const u64 n = min((u64)cursor[part], part_cap);         // records grouped into this partition
     const V* __restrict__ slots = grouped + (u64)part * part_cap;
     const u64 base = (u64)jblk * kInsTile;
-    // Warm the table region `warm_ahead` partitions ahead of this block's own with sequential L2
+    // Warm the table region kWarmAhead partitions ahead of this block's own with sequential L2
     // prefetches: a first touch by a random CAS costs a DRAM row activation each (the 41 G/s ceiling),
     // a sequential sweep of the same region costs streaming bandwidth.  Non-destructive, so no ordering
-    // between blocks is needed.  Each block of partition p warms its share of region p + warm_ahead.
-    if (warm_ahead && part + warm_ahead < nparts) {
-        const u32 tp = part + warm_ahead;
+    // between blocks is needed.  Each block of partition p warms its share of region p + kWarmAhead.
+    if (part + kWarmAhead < nparts) {
+        const u32 tp = part + kWarmAhead;
         const u64 b0 = (u64)tp << part_shift, b1 = min(nbuckets, ((u64)tp + 1) << part_shift);
         const u64 nlines = ((b1 - b0) * 32 + 127) >> 7;
         const u64 per = (nlines + blocks_per_part - 1) / blocks_per_part;
@@ -677,51 +626,31 @@ insert_slots_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const
             asm volatile("prefetch.global.L2 [%0];" ::"l"(region + (l << 7)));
     }
     if (base >= n) return;
-    V v[kInsPerThread];
-    u64 b[kInsPerThread];
+    V v[kInsPerThread], old[kInsPerThread];
     bool live[kInsPerThread];
     u32 inserted = 0, dups = 0, err = 0;
-    if (MODE == 0) {
-        u64 q[kInsPerThread][4];
 #pragma unroll
-        for (int r = 0; r < kInsPerThread; ++r) {
-            const u64 i = base + (u64)r * kInsThreads + threadIdx.x;
-            live[r] = i < n;
-            v[r] = live[r] ? slots[i] : S::zero();
-            b[r] = live[r] ? place_bucket<W>(v[r], k, m, nbuckets) : 0;
-            if (live[r]) load256_cg(table + b[r] * S::kPerBucket, q[r]);
-        }
+    for (int r = 0; r < kInsPerThread; ++r) {
+        const u64 i = base + (u64)r * kInsThreads + threadIdx.x;
+        live[r] = i < n;
+        v[r] = live[r] ? slots[i] : S::zero();
+        old[r] = S::zero();
+        if (live[r]) old[r] = S::cas(table + place_bucket<W>(v[r], nbuckets) * S::kPerBucket, S::zero(), v[r]);
+    }
 #pragma unroll
-        for (int r = 0; r < kInsPerThread; ++r) {
-            if (!live[r]) continue;
-            const int rc = insert_one<W>(table, nbuckets, b[r], v[r], q[r]);
-            inserted += (rc == kInsInserted);
-            dups += (rc == kInsDuplicate);
-            if (rc == kInsFull) err |= kErrTableFull;
-        }
-    } else {
-        V old[kInsPerThread];
-#pragma unroll
-        for (int r = 0; r < kInsPerThread; ++r) {
-            const u64 i = base + (u64)r * kInsThreads + threadIdx.x;
-            live[r] = i < n;
-            v[r] = live[r] ? slots[i] : S::zero();
-            b[r] = live[r] ? place_bucket<W>(v[r], k, m, nbuckets) : 0;
-            old[r] = S::zero();
-            if (live[r]) old[r] = S::cas(table + b[r] * S::kPerBucket, S::zero(), v[r]);
-        }
-#pragma unroll
-        for (int r = 0; r < kInsPerThread; ++r) {
-            if (!live[r]) continue;
-            if (S::empty(old[r])) { ++inserted; continue; }
-            if (S::same_key(old[r], v[r])) { ++dups; continue; }
-            u64 q[4];
-            load256_cg(table + b[r] * S::kPerBucket, q);     // slot 0 is occupied by another key: general path
-            const int rc = insert_one<W>(table, nbuckets, b[r], v[r], q);
-            inserted += (rc == kInsInserted);
-            dups += (rc == kInsDuplicate);
-            if (rc == kInsFull) err |= kErrTableFull;
-        }
+    for (int r = 0; r < kInsPerThread; ++r) {
+        if (!live[r]) continue;
+        if (S::empty(old[r])) { ++inserted; continue; }
+        if (S::same_key(old[r], v[r])) { ++dups; continue; }
+        // slot 0 is occupied by another key: general path.  The home bucket is hashed again rather than kept from the
+        // first loop: four live bucket numbers do not fit the 40 registers of 6 blocks per SM and were spilled.
+        const u64 b = place_bucket<W>(v[r], nbuckets);
+        u64 q[4];
+        load256_cg(table + b * S::kPerBucket, q);
+        const int rc = insert_one<W>(table, nbuckets, b, v[r], q);
+        inserted += (rc == kInsInserted);
+        dups += (rc == kInsDuplicate);
+        if (rc == kInsFull) err |= kErrTableFull;
     }
     inserted = __reduce_add_sync(kFullMask, inserted);
     dups = __reduce_add_sync(kFullMask, dups);
@@ -838,11 +767,11 @@ scatter_starts_kernel(const unsigned char* __restrict__ recs, u64 n, int k,
 // K4  lookup
 // =========================================================================================
 template <int W>
-__device__ __forceinline__ bool lookup(const typename Slot<W>::value_t* __restrict__ table, u64 nbuckets, int k, int m,
+__device__ __forceinline__ bool lookup(const typename Slot<W>::value_t* __restrict__ table, u64 nbuckets,
                                        typename Slot<W>::value_t keybits, typename Slot<W>::value_t& found,
                                        u64& bucket, int& slot) {
     typedef Slot<W> S;
-    u64 b = place_bucket<W>(keybits, k, m, nbuckets);
+    u64 b = place_bucket<W>(keybits, nbuckets);
     for (u64 tries = 0; tries < nbuckets; ++tries) {
         u64 q[4];
         load256_nc(table + b * S::kPerBucket, q);
@@ -868,7 +797,7 @@ __device__ __forceinline__ bool lookup(const typename Slot<W>::value_t* __restri
 
 template <int W>
 __global__ void __launch_bounds__(256)
-find_kernel(const typename Slot<W>::value_t* __restrict__ table, u64 nbuckets, int k, int m,
+find_kernel(const typename Slot<W>::value_t* __restrict__ table, u64 nbuckets, int k,
             const unsigned char* __restrict__ pkmers, u64 n,
             unsigned char* __restrict__ pairs_out, unsigned char* __restrict__ found_out) {
     typedef Slot<W> S;
@@ -879,7 +808,7 @@ find_kernel(const typename Slot<W>::value_t* __restrict__ table, u64 nbuckets, i
     for (int j = 0; j < pl; ++j) key[j] = pkmers[i * pl + j];
     typename S::value_t hit;
     u64 b; int s;
-    const bool ok = lookup<W>(table, nbuckets, k, m, S::from_packed(key, k, pl), hit, b, s);
+    const bool ok = lookup<W>(table, nbuckets, S::from_packed(key, k, pl), hit, b, s);
     unsigned char rec[18];
     for (int j = 0; j < pb; ++j) rec[j] = 0;
     if (ok) S::to_record(hit, k, pl, rec);
@@ -913,7 +842,6 @@ struct WalkParams {
     u32 seg_chars;        // multiple of 8
     u32 seg_cap;          // capacity of link/seglen/tmp in segments
     int k;
-    int m;                // minimizer length of the placement (0 = plain key hash)
 };
 
 constexpr u32 kWalkBatch = 128;     // walker ids a warp takes per global atomic
@@ -1022,7 +950,7 @@ walk_kernel(const WalkParams p) {
                     acc = 0;
                 }
                 V nxt; u64 b; int s;
-                if (!lookup<W>(table, p.nbuckets, p.k, p.m, S::next_key(cur, p.k), nxt, b, s)) {
+                if (!lookup<W>(table, p.nbuckets, S::next_key(cur, p.k), nxt, b, s)) {
                     // kmer_hash.cpp:47-49 throws only for chains it walks: mark the segment, rank_kernel raises the
                     // error if a START-rooted contig ends here (a walker started at a splitter may sit on a chain no
                     // start node reaches, which the reference never visits)

@@ -140,7 +140,6 @@ template <> struct Slot<1> {
     static __host__ __device__ __forceinline__ bool equal(value_t a, value_t b) { return a == b; }
     static __host__ __device__ __forceinline__ value_t key_only(value_t v) { return v & ~63ull; }
     static __host__ __device__ __forceinline__ u64 hash(value_t v) { return fmix64(v >> 6); }
-    static __host__ __device__ __forceinline__ u64 owner_hash(value_t v) { return fmix64((v >> 6) ^ 0x9E3779B97F4A7C15ull); }
     static __device__ __forceinline__ value_t from_bucket(const u64 (&q)[4], int i) { return q[i]; }
 
     // kmer_pair bytes -> slot.  pl = (k+3)/4.
@@ -213,9 +212,6 @@ template <> struct Slot<2> {
     static __host__ __device__ __forceinline__ value_t key_only(value_t v) { return u128{v.lo & ~63ull, v.hi}; }
     static __host__ __device__ __forceinline__ u64 hash(value_t v) {
         return fmix64((v.lo >> 6) ^ fmix64(v.hi + 0x9E3779B97F4A7C15ull));
-    }
-    static __host__ __device__ __forceinline__ u64 owner_hash(value_t v) {
-        return fmix64((v.lo >> 6) + 0xD6E8FEB86659FD93ull + fmix64(v.hi ^ 0xA0761D6478BD642Full));
     }
     static __device__ __forceinline__ value_t from_bucket(const u64 (&q)[4], int i) { return u128{q[2 * i], q[2 * i + 1]}; }
 
@@ -309,53 +305,7 @@ template <> struct Slot<2> {
 };
 
 
-// ---- placement: where a k-mer lives -------------------------------------------------------------
-// With a plain key hash, the successor of a k-mer (its last K-1 bases + one new base) lands in an
-// unrelated bucket, so every step of a contig walk is a random DRAM access (and, sharded, usually a
-// remote one).  Hashing the k-mer's MINIMIZER instead -- the m-mer with the smallest order value
-// among its K-m+1 m-mers, leftmost on ties -- gives consecutive k-mers of a contig the same home for
-// as long as they share the minimizer (a "supermer": (K-m+2)/2 k-mers on average on random
-// sequence), so they fill adjacent slots of one bucket run on one GPU.  Nothing else about the table
-// changes: the home is still a pure function of the key, probing is linear from the home bucket.
-// m = 0 selects the plain key hash.
-__host__ __device__ __forceinline__ int minimizer_len(int k) {
-    return k <= 14 ? k : (k <= 18 ? 11 : (k <= 29 ? 13 : (k <= 40 ? 21 : 31)));
-}
-__host__ __device__ __forceinline__ u32 mmer_order(u64 x) {      // order value of an m-mer (<= 42 bits)
-    return (u32)((x * 0x9E3779B97F4A7C15ull) >> 32);
-}
-template <int W> __host__ __device__ __forceinline__ u64 minimizer_value(typename Slot<W>::value_t v, int k, int m);
-template <> __host__ __device__ __forceinline__ u64 minimizer_value<1>(u64 v, int k, int m) {
-    const u64 key = v >> 6, mask = (m >= 32) ? ~0ull : ((1ull << (2 * m)) - 1ull);
-    u32 best = 0xFFFFFFFFu;
-    u64 bx = 0;
-    for (int s = 2 * (k - m); s >= 0; s -= 2) {                  // leftmost m-mer first
-        const u64 x = (key >> s) & mask;
-        const u32 g = mmer_order(x);
-        if (g < best) { best = g; bx = x; }
-    }
-    return bx;
-}
-template <> __host__ __device__ __forceinline__ u64 minimizer_value<2>(u128 v, int k, int m) {
-    const u64 lo = (v.lo >> 6) | (v.hi << 58), hi = v.hi >> 6, mask = (m >= 32) ? ~0ull : ((1ull << (2 * m)) - 1ull);
-    u32 best = 0xFFFFFFFFu;
-    u64 bx = 0;
-    for (int s = 2 * (k - m); s >= 0; s -= 2) {
-        const u64 x = (s >= 64 ? (hi >> (s - 64)) : (s == 0 ? lo : ((lo >> s) | (hi << (64 - s))))) & mask;
-        const u32 g = mmer_order(x);
-        if (g < best) { best = g; bx = x; }
-    }
-    return bx;
-}
-// The owner function may use a shorter minimizer than the placement: it only has to balance a handful of
-// GPUs, and a shorter m-mer means a longer window, i.e. longer runs of k-mers that stay on one GPU.
-__host__ __device__ __forceinline__ int owner_minimizer_len(int k) { return k <= 14 ? k : 7; }
-
-// hash that selects the owning GPU, and hash that selects the home bucket (independent of each other)
-template <int W> __host__ __device__ __forceinline__ u64 owner_hash_of(typename Slot<W>::value_t v, int k, int m) {
-    return m ? fmix64(minimizer_value<W>(v, k, m) + 0x632BE59BD9B4E019ull) : Slot<W>::owner_hash(v);
-}
-
+// ---- placement of the plain table: where a k-mer lives --------------------------------------------
 // hash -> bucket without requiring a power-of-two table (load-factor sweeps need exact sizes)
 __host__ __device__ __forceinline__ u64 bucket_of(u64 h, u64 nbuckets) {
 #ifdef __CUDA_ARCH__
@@ -365,28 +315,10 @@ __host__ __device__ __forceinline__ u64 bucket_of(u64 h, u64 nbuckets) {
 #endif
 }
 
-// rank (GPU) that stores a k-mer: hash_map.hpp:28-30's get_target_rank with a supermer-preserving hash
+// Home bucket of a k-mer: a hash of the key; probing is linear from there.
 template <int W>
-__host__ __device__ __forceinline__ u32 owner_of(typename Slot<W>::value_t v, int world, int k, int m) {
-    return (u32)bucket_of(owner_hash_of<W>(v, k, m), (u64)world);
-}
-
-// Home bucket of a k-mer.  With locality (m != 0) the REGION -- kRegionBuckets consecutive buckets: one
-// 128-byte line of 16 slots for 64-bit slots, four lines of 32 slots for 128-bit slots -- is chosen by
-// the minimizer, and the bucket inside the region by the key itself: the members of a supermer spread
-// over the region instead of queueing behind one home bucket (probe chains stay ~1 bucket), yet they
-// share cache lines and DRAM rows.  Regions that overflow spill into the following buckets as usual.
-template <int W> struct RegionOf { static constexpr u64 kBuckets = (W == 1) ? 4 : 16; };
-template <int W>
-__host__ __device__ __forceinline__ u64 place_bucket_from(u64 minimizer_hash, typename Slot<W>::value_t v, u64 nbuckets) {
-    constexpr u64 G = RegionOf<W>::kBuckets;
-    const u64 region = bucket_of(fmix64(minimizer_hash ^ 0x9E3779B97F4A7C15ull), nbuckets / G);   // nbuckets % G == 0
-    return region * G + (Slot<W>::hash(v) & (G - 1));
-}
-template <int W>
-__host__ __device__ __forceinline__ u64 place_bucket(typename Slot<W>::value_t v, int k, int m, u64 nbuckets) {
-    if (m == 0) return bucket_of(Slot<W>::hash(v), nbuckets);
-    return place_bucket_from<W>(fmix64(minimizer_value<W>(v, k, m) + 0x632BE59BD9B4E019ull), v, nbuckets);
+__host__ __device__ __forceinline__ u64 place_bucket(typename Slot<W>::value_t v, u64 nbuckets) {
+    return bucket_of(Slot<W>::hash(v), nbuckets);
 }
 
 // =============================================================================================
@@ -553,8 +485,7 @@ struct Counters {
     u64 scan_total;       // result of the last device scan (start nodes of the last insert call)
     u64 n_nodes;
     u64 contig_bytes;
-    u32 n_boundary;       // sharded: nodes of this shard whose predecessor lives on another GPU (walker starts)
-    u32 n_outbox;         // sharded: pending links produced by the local walk
+    u32 n_outbox;         // plain table, chunked build: records the chunks could not place (the overflow list)
     u32 flags[40];
     u32 rank_done;        // ctable: no rank moved a link in the last pointer-jumping round (agreed on by all ranks)
     u32 err_where;        // ctable: which capacity / wait raised kErrInternal (CtSite bits), for the error message

@@ -29,7 +29,7 @@ __device__ __forceinline__ bool device_find_w(const kh_device_view& v, const uns
     typename S::value_t hit;
     u64 b;
     int s;
-    if (!lookup<W>(static_cast<const typename S::value_t*>(v.table), v.n_buckets, v.k, v.placement_m, key, hit, b, s)) return false;
+    if (!lookup<W>(static_cast<const typename S::value_t*>(v.table), v.n_buckets, key, hit, b, s)) return false;
     if (pair_out) S::to_record(hit, v.k, pl, pair_out);
     return true;
 }
@@ -42,7 +42,7 @@ __device__ __forceinline__ int device_insert_w(const kh_device_view& v, const un
     const V val = S::from_record(pair, v.k, pl, ok);
     if (!ok) return kDevBadInput;
     V* table = static_cast<V*>(v.table);
-    const u64 b = place_bucket<W>(val, v.k, v.placement_m, v.n_buckets);
+    const u64 b = place_bucket<W>(val, v.n_buckets);
     u64 q[4];
     load256_cg(table + b * S::kPerBucket, q);
     const int rc = insert_one<W>(table, v.n_buckets, b, val, q);

@@ -147,7 +147,7 @@ typedef struct kh_device_view {
     uint64_t n_buckets;
     int32_t k;
     int32_t slot_bytes;        /* 8 or 16                                                      */
-    int32_t placement_m;       /* internal: minimizer length of the bucket placement (0 = none) */
+    int32_t placement_m;       /* reserved, always 0                                           */
     int32_t device;            /* CUDA ordinal that owns the table                             */
 } kh_device_view;
 int kh_get_device_view(kh_table* t, kh_device_view* out);

@@ -20,7 +20,7 @@ import cs267_hw3_b200 as kh  # noqa: E402
 from tools import kmergen, readgen  # noqa: E402
 
 
-def run(k=51, n=4_000_000, coverage=8, read_len=150, reps=5, seed=267, sweep=False):
+def run(k=51, n=4_000_000, coverage=8, read_len=150, reps=5, seed=267):
     c = max(1, round(n * 860329 / 89710742))
     d = kmergen.Dataset(k, n, c, seed=seed)
     t0 = time.time()
@@ -49,19 +49,6 @@ def run(k=51, n=4_000_000, coverage=8, read_len=150, reps=5, seed=267, sweep=Fal
         ts = tab.stats()
         lines = sorted(buf.tobytes().split(b"\n")[:-1])
         verified = nodes == n and b"\n".join(lines) + b"\n" == d.solution()
-        variants = {}
-        if sweep:                                          # the kernel's two switches, same reads, same table size
-            for pf in (0, 1):
-                for mb in ((8,) if k <= 31 else (6, 8)):
-                    os.environ["KH_COUNT_PREFETCH"], os.environ["KH_COUNT_BLOCKS"] = str(pf), str(mb)
-                    with kh.KmerCounter(k, n, 0.5, device=0) as kv:
-                        t = []
-                        for _ in range(4):
-                            kv.clear()
-                            kv.count_reads_device(p.value, reads.size)
-                            t.append(kv.stats()["ms_count"])
-                        variants[f"prefetch{pf}_blocks{mb}"] = round(float(np.median(t[1:])), 4)
-            os.environ.pop("KH_COUNT_PREFETCH"); os.environ.pop("KH_COUNT_BLOCKS")
         pin = kh.PinnedBuffer(reads.size)
         pin.array[:] = reads
         ms_host = []
@@ -91,7 +78,6 @@ def run(k=51, n=4_000_000, coverage=8, read_len=150, reps=5, seed=267, sweep=Fal
         "ms_extract": float(np.median(ms_ext[1:])), "ms_count_host_buffers": float(np.median(ms_host[1:])),
         "host_gbs": reads.size / float(np.median(ms_host[1:])) / 1e6,
         "then_insert_ms_first_call": ts["ms_insert"], "then_assemble_ms_first_call": ts["ms_assemble"], "verified": bool(verified),
-        "variants_ms": variants or None,
     })
     # a bounded piece of the same reads for bench.py's CPU leg (whole lines, about 8 MB); not part of the JSON record
     cut = int(np.flatnonzero(reads[: 8 << 20] == 10)[-1]) + 1
@@ -100,7 +86,6 @@ def run(k=51, n=4_000_000, coverage=8, read_len=150, reps=5, seed=267, sweep=Fal
 
 
 if __name__ == "__main__":
-    a = [int(x) for x in sys.argv[1:] if x != "--sweep"]
-    rec = run(*a, sweep="--sweep" in sys.argv)
+    rec = run(*[int(x) for x in sys.argv[1:]])
     rec.pop("_sample", None)
     print(json.dumps(rec))

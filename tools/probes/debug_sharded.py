@@ -56,7 +56,7 @@ for rep in range(reps):
             lk = buf(s, "link", np.uint64, max(next_seg, hcap))
             links.append(lk)
             print(f"rank {r}: hcap {hcap} next_seg {next_seg} n_starts {s.tab.stats()['n_starts']} inbox_cnt {buf(s, 'inbox_cnt', np.uint32, 8)} "
-                  f"out_cursor {buf(s, 'out_cursor', np.uint32, 8)} epoch {caps[6]} flags(moved) {ctr[14:14 + 12]}")
+                  f"out_cursor {buf(s, 'out_cursor', np.uint32, 8)} epoch {caps[6]} flags(moved) {ctr[15:15 + 12]}")
         names = {0xFFFFFFFF: "TAIL", 0xFFFFFFFE: "UNUSED", 0xFFFFFFFD: "CLAIMED", 0xFFFFFFFC: "PENDING", 0xFFFFFFFB: "MISSING", 0xFFFFFFFA: "CONVERGE"}
         shown = 0
         for r, s in enumerate(shards):
