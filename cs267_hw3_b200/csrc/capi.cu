@@ -46,11 +46,9 @@ struct kh_table {
     DevBuf mask, tile_counts, tile_offs, scan_blocks;
     DevBuf part_cursor, grouped;
     DevBuf fine, chunk_cursor, overflow;          // chunked (shared-memory) build
-    int build_mode = 1;               // KH_BUILD: 1 = shared-memory chunk build for large batches, 0 = atomic insert_slots
     bool table_dirty = false;         // something was inserted since create/clear
     bool chunk_attr_set = false;
     int debug_cap_pct = 100;          // KH_DEBUG_CAP_PCT: scale the grouping buffers' capacities (tests force the overflow paths)
-    int partition_mode = -1;          // -1 auto, 0 never, 1 always (KH_PARTITION)
     bool part_attr_set = false;
     Counters* d_ctr = nullptr;
     Counters* h_ctr = nullptr;
@@ -185,6 +183,13 @@ static size_t partition_smem(int W, u32 nparts, int pb) {
     return ((12 * (size_t)nparts + 2 * kPartTile + 15) & ~(size_t)15) + un;
 }
 
+// Capacity of a grouping buffer for the records whose home lies in `span` buckets of the table: their expected share
+// of n plus 24 binomial sigmas and `slack`, scaled by KH_DEBUG_CAP_PCT.  The hash is uniform, so no histogram pass.
+static u64 group_cap(const kh_table* t, u64 n, u64 span, double slack) {
+    const double share = (double)n * (double)std::min<u64>(t->nbuckets, span) / (double)t->nbuckets;
+    return (u64)(share + 24.0 * std::sqrt(share + 1.0) + slack) * t->debug_cap_pct / 100;
+}
+
 template <int W>
 int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool record_start) {
     typedef typename Slot<W>::value_t V;
@@ -195,19 +200,21 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
     KH_TRY(ensure(t, t->tile_counts, (ntiles + 1) * sizeof(u32)));
     KH_TRY(ensure(t, t->tile_offs, (ntiles + 1) * sizeof(u64)));
     // Tables larger than L2 get their records grouped by table region first (see kernels.cuh K2p).
-    const bool part = t->partition_mode == 1 || (t->partition_mode < 0 && t->table_bytes > (64ull << 20) && n >= (1u << 16));
-    u32 part_shift = 0, nparts = 1, bpp = 1;
+    const bool part = t->table_bytes > (64ull << 20) && n >= (1u << 16);
+    // Large batches (>= 1/8 of the table's slots) are built chunk by chunk in shared memory: no global atomics.
+    // Measured against insert_slots: faster with 64-bit slots (2.85 vs 3.03 ms), slower with 128-bit slots (4.6 vs
+    // 4.1 ms: twice the bytes through the two grouping passes), so the chunked build is the 64-bit path only.
+    const bool chunked = W == 1 && part && n * 8 >= t->nbuckets * (u64)t->per_bucket;
+    u32 part_shift = 0, nparts = 1;
     u64 part_cap = 0;
     if (part) {
-        while ((32ull << part_shift) < kPartBytes) ++part_shift;
+        if (chunked) part_shift = kChunkShift + 7;                     // 128 chunks (8 MB of table) per partition
+        else while ((32ull << part_shift) < kPartBytes) ++part_shift;
         while (((t->nbuckets - 1) >> part_shift) + 1 > (u64)kMaxParts) ++part_shift;
+        if (chunked && part_shift - kChunkShift > 10) return fail(t, KH_ERR_ARG, "table too large for the chunked build");
         nparts = (u32)(((t->nbuckets - 1) >> part_shift) + 1);
-        // a partition's expected share of n plus slack (24 binomial sigmas), rounded to whole insert tiles; overflow
-        // falls back to a direct insert
-        const double share = (double)n * (double)std::min<u64>(t->nbuckets, 1ull << part_shift) / (double)t->nbuckets;
-        part_cap = (u64)(share + 24.0 * std::sqrt(share + 1.0) + 64.0) * t->debug_cap_pct / 100;
-        part_cap = (part_cap + kInsTile - 1) / kInsTile * kInsTile;
-        bpp = (u32)(part_cap / kInsTile);
+        // rounded to whole insert tiles; overflow falls back to a direct insert (or the chunked build's fix-up list)
+        part_cap = (group_cap(t, n, 1ull << part_shift, 64.0) + kInsTile - 1) / kInsTile * kInsTile;
         KH_TRY(ensure(t, t->part_cursor, kMaxParts * sizeof(u32)));
         KH_TRY(ensure(t, t->grouped, (u64)nparts * part_cap * sizeof(V)));
         if (!t->part_attr_set) {
@@ -216,33 +223,17 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
             t->part_attr_set = true;
         }
     }
-    // Large batches (>= 1/8 of the table's slots) are built chunk by chunk in shared memory: no global atomics.
-    const bool chunked = part && t->build_mode != 0 && n * 8 >= t->nbuckets * (u64)t->per_bucket;
-    u32 chunk_cap = 0, overflow_cap = 0, bpp2 = 1;
+    u32 chunk_cap = 0, overflow_cap = 0;
     u64 nchunks = 0;
-    size_t sub_smem = 0;
     if (chunked) {
-        part_shift = kChunkShift + 7;                                   // 128 chunks (8 MB of table) per partition
-        while (((t->nbuckets - 1) >> part_shift) + 1 > (u64)kMaxParts) ++part_shift;
-        if (part_shift - kChunkShift > 10) return fail(t, KH_ERR_ARG, "table too large for the chunked build");
-        nparts = (u32)(((t->nbuckets - 1) >> part_shift) + 1);
-        const double share = (double)n * (double)std::min<u64>(t->nbuckets, 1ull << part_shift) / (double)t->nbuckets;
-        part_cap = (u64)(share + 24.0 * std::sqrt(share + 1.0) + 64.0) * t->debug_cap_pct / 100;
-        part_cap = (part_cap + kInsTile - 1) / kInsTile * kInsTile;
         nchunks = (t->nbuckets + kChunkBuckets - 1) >> kChunkShift;
-        const double share2 = (double)n * (double)std::min<u64>(t->nbuckets, kChunkBuckets) / (double)t->nbuckets;
-        chunk_cap = (u32)((u64)(share2 + 24.0 * std::sqrt(share2 + 1.0) + 32.0) * t->debug_cap_pct / 100);
-        chunk_cap = std::max(4u, (chunk_cap + 3u) & ~3u);
+        chunk_cap = std::max(4u, ((u32)group_cap(t, n, kChunkBuckets, 32.0) + 3u) & ~3u);
         overflow_cap = (u32)std::min<u64>(0x7FFFFFFFull, t->debug_cap_pct < 100 ? n + 65536 : n / 32 + 65536);
-        bpp2 = (u32)((part_cap + kSubTile - 1) / kSubTile);
-        const u32 nsub = 1u << (part_shift - kChunkShift);
-        sub_smem = 8 * (size_t)nsub + 16;
-        KH_TRY(ensure(t, t->grouped, (u64)nparts * part_cap * sizeof(V)));
         KH_TRY(ensure(t, t->fine, nchunks * (u64)chunk_cap * sizeof(V)));
         KH_TRY(ensure(t, t->chunk_cursor, nchunks * sizeof(u32)));
         KH_TRY(ensure(t, t->overflow, (u64)overflow_cap * sizeof(V)));
         if (!t->chunk_attr_set) {
-            KH_CUDA(t, cudaFuncSetAttribute(build_chunks_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kChunkBuckets * 32)));
+            KH_CUDA(t, cudaFuncSetAttribute(build_chunks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kChunkBuckets * 32)));
             t->chunk_attr_set = true;
         }
     }
@@ -252,23 +243,26 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
             recs, n, t->k, static_cast<V*>(t->table), t->nbuckets, static_cast<u32*>(t->mask.p),
             static_cast<u32*>(t->tile_counts.p), t->d_ctr);
     } else if (chunked) {
-        KH_CUDA(t, cudaMemsetAsync(t->part_cursor.p, 0, kMaxParts * sizeof(u32), t->stream));
-        KH_CUDA(t, cudaMemsetAsync(t->chunk_cursor.p, 0, nchunks * sizeof(u32), t->stream));
-        KH_CUDA(t, cudaMemsetAsync(&t->d_ctr->n_outbox, 0, sizeof(u32), t->stream));
-        const u64 pblocks = (n + kPartTile - 1) / kPartTile;
-        partition_kernel<W><<<(unsigned)pblocks, kPartThreads, partition_smem(W, nparts, t->pb), t->stream>>>(
-            recs, n, t->k, t->nbuckets, part_shift, nparts, part_cap, static_cast<u32*>(t->part_cursor.p),
-            static_cast<V*>(t->grouped.p), static_cast<V*>(t->table), static_cast<u32*>(t->mask.p),
-            static_cast<u32*>(t->tile_counts.p), static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
-        subpartition_kernel<W><<<nparts * bpp2, kSubThreads, sub_smem, t->stream>>>(
-            static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), part_cap, bpp2, kChunkShift,
-            1u << (part_shift - kChunkShift), t->nbuckets, chunk_cap, static_cast<u32*>(t->chunk_cursor.p), static_cast<V*>(t->fine.p),
-            static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
-        build_chunks_kernel<W><<<(unsigned)nchunks, kBuildThreads, kChunkBuckets * 32, t->stream>>>(
-            static_cast<const V*>(t->fine.p), static_cast<const u32*>(t->chunk_cursor.p), chunk_cap, static_cast<V*>(t->table),
-            t->nbuckets, t->table_dirty ? 1 : 0, static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
-        insert_overflow_kernel<W><<<64, 256, 0, t->stream>>>(static_cast<const V*>(t->overflow.p), overflow_cap,
-                                                            static_cast<V*>(t->table), t->nbuckets, t->d_ctr);
+        if constexpr (W == 1) {
+            KH_CUDA(t, cudaMemsetAsync(t->part_cursor.p, 0, kMaxParts * sizeof(u32), t->stream));
+            KH_CUDA(t, cudaMemsetAsync(t->chunk_cursor.p, 0, nchunks * sizeof(u32), t->stream));
+            KH_CUDA(t, cudaMemsetAsync(&t->d_ctr->n_outbox, 0, sizeof(u32), t->stream));
+            const u64 pblocks = (n + kPartTile - 1) / kPartTile;
+            partition_kernel<W><<<(unsigned)pblocks, kPartThreads, partition_smem(W, nparts, t->pb), t->stream>>>(
+                recs, n, t->k, t->nbuckets, part_shift, nparts, part_cap, static_cast<u32*>(t->part_cursor.p),
+                static_cast<V*>(t->grouped.p), static_cast<V*>(t->table), static_cast<u32*>(t->mask.p),
+                static_cast<u32*>(t->tile_counts.p), static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
+            const u32 bpp = (u32)((part_cap + kSubTile - 1) / kSubTile), nsub = 1u << (part_shift - kChunkShift);
+            subpartition_kernel<<<nparts * bpp, kSubThreads, 8 * (size_t)nsub + 16, t->stream>>>(
+                static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), part_cap, bpp, kChunkShift,
+                nsub, t->nbuckets, chunk_cap, static_cast<u32*>(t->chunk_cursor.p), static_cast<V*>(t->fine.p),
+                static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
+            build_chunks_kernel<<<(unsigned)nchunks, kBuildThreads, kChunkBuckets * 32, t->stream>>>(
+                static_cast<const V*>(t->fine.p), static_cast<const u32*>(t->chunk_cursor.p), chunk_cap, static_cast<V*>(t->table),
+                t->nbuckets, t->table_dirty ? 1 : 0, static_cast<V*>(t->overflow.p), overflow_cap, t->d_ctr);
+            insert_overflow_kernel<<<64, 256, 0, t->stream>>>(static_cast<const V*>(t->overflow.p), overflow_cap,
+                                                             static_cast<V*>(t->table), t->nbuckets, t->d_ctr);
+        }
     } else {
         KH_CUDA(t, cudaMemsetAsync(t->part_cursor.p, 0, kMaxParts * sizeof(u32), t->stream));
         const u64 warm_buckets = std::min<u64>(t->nbuckets, (u64)kWarmAhead << part_shift);
@@ -279,6 +273,7 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
             recs, n, t->k, t->nbuckets, part_shift, nparts, part_cap, static_cast<u32*>(t->part_cursor.p),
             static_cast<V*>(t->grouped.p), static_cast<V*>(t->table), static_cast<u32*>(t->mask.p),
             static_cast<u32*>(t->tile_counts.p), static_cast<V*>(nullptr), 0u, t->d_ctr);
+        const u32 bpp = (u32)(part_cap / kInsTile);
         const unsigned iblocks = nparts * bpp;
         insert_slots_kernel<W><<<iblocks, kInsThreads, 0, t->stream>>>(
             static_cast<const V*>(t->grouped.p), static_cast<const u32*>(t->part_cursor.p), part_cap, bpp, nparts,
@@ -1037,10 +1032,6 @@ int kh_create(int k, uint64_t n_expected, double load_factor, int device, kh_tab
     memset(t->h_ctr, 0, sizeof(Counters));
     int v = env_int("KH_SPLIT_BUCKETS", 0);
     if (v > 0 && set_option(t, "split_buckets", v) != KH_OK) fprintf(stderr, "libkh_b200: ignoring KH_SPLIT_BUCKETS=%d\n", v);
-    t->partition_mode = env_int("KH_PARTITION", -1);
-    // measured: the shared-memory build wins for 64-bit slots (2.85 vs 3.03 ms) and loses for 128-bit slots
-    // (4.6 vs 4.1 ms: twice the bytes through the two grouping passes), so it is the default only for K <= 29
-    t->build_mode = env_int("KH_BUILD", t->W == 1 ? 1 : 0);
     t->debug_cap_pct = std::max(1, env_int("KH_DEBUG_CAP_PCT", 100));
     v = env_int("KH_SEG_CHARS", 0);
     if (v > 0 && set_option(t, "seg_chars", v) != KH_OK) fprintf(stderr, "libkh_b200: ignoring KH_SEG_CHARS=%d\n", v);

@@ -42,20 +42,6 @@ __device__ __forceinline__ void stage_in(unsigned char* s_dst, const unsigned ch
         for (u32 i = threadIdx.x; i < bytes; i += blockDim.x) s_dst[i] = g_src[i];
     }
 }
-// same with the block size known at compile time (a run-time stride costs a division per loop for the trip count)
-template <int THREADS>
-__device__ __forceinline__ void stage_in_fixed(unsigned char* s_dst, const unsigned char* g_src, u32 bytes) {
-    if ((reinterpret_cast<uintptr_t>(g_src) & 15u) == 0) {
-        const u32 nv = bytes >> 4;
-        const uint4* s4 = reinterpret_cast<const uint4*>(g_src);
-        uint4* d4 = reinterpret_cast<uint4*>(s_dst);
-#pragma unroll 4
-        for (u32 i = threadIdx.x; i < nv; i += THREADS) d4[i] = load128_stream(s4 + i);
-        for (u32 i = (nv << 4) + threadIdx.x; i < bytes; i += THREADS) s_dst[i] = g_src[i];
-    } else {
-        for (u32 i = threadIdx.x; i < bytes; i += THREADS) s_dst[i] = g_src[i];
-    }
-}
 __device__ __forceinline__ void stage_out(unsigned char* g_dst, const unsigned char* s_src, u32 bytes) {
     if ((reinterpret_cast<uintptr_t>(g_dst) & 15u) == 0) {
         const u32 nv = bytes >> 4;
@@ -393,8 +379,10 @@ partition_kernel(const unsigned char* __restrict__ recs, u64 n, int k, u64 nbuck
 }
 
 // =========================================================================================
-// K2c  chunked build: no global atomics at all
+// K2c  chunked build (64-bit slots): no global atomics at all
 // =========================================================================================
+// The path for large batches into tables of 64-bit slots.  With 128-bit slots twice the bytes go through the two
+// grouping passes and insert_slots_kernel is faster (capi.cu), so these kernels exist for Slot<1> only.
 // The grouped records of one partition (partition_kernel) are split once more by 64 KB table chunk
 // (subpartition_kernel); then one block per chunk builds the chunk in SHARED memory with ATOMS.CAS and
 // writes it to HBM in one coalesced sweep (build_chunks_kernel).  DRAM sees only streaming traffic
@@ -412,14 +400,13 @@ constexpr int kSubTile = kSubThreads * kSubPerThread;  // 2048 slot values per b
 // the sector writes); staging a sorted copy in shared memory first was measured slower (2.71 vs 2.52 ms insert).
 // The kernel splits input partition `part` (values whose home lies in units [part*nsub, (part+1)*nsub), a unit being
 // 2^unit_shift buckets) into one buffer per unit.  Level 2 of the chunked build uses it with unit = chunk.
-template <int W>
 __global__ void __launch_bounds__(kSubThreads, 4)
-subpartition_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const u32* __restrict__ part_cursor,
+subpartition_kernel(const u64* __restrict__ grouped, const u32* __restrict__ part_cursor,
                     u64 part_cap, u32 blocks_per_part, u32 unit_shift, u32 nsub, u64 nbuckets,
-                    u32 chunk_cap, u32* __restrict__ chunk_cursor, typename Slot<W>::value_t* __restrict__ fine,
-                    typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap, Counters* ctr) {
-    typedef Slot<W> S;
-    typedef typename S::value_t V;
+                    u32 chunk_cap, u32* __restrict__ chunk_cursor, u64* __restrict__ fine,
+                    u64* __restrict__ overflow, u32 overflow_cap, Counters* ctr) {
+    typedef Slot<1> S;
+    typedef u64 V;
     extern __shared__ __align__(16) unsigned char s_raw[];
     u32* s_hist = reinterpret_cast<u32*>(s_raw);                       // nsub <= 1024 units per input partition
     u32* s_gbase = s_hist + nsub;
@@ -442,7 +429,7 @@ subpartition_kernel(const typename Slot<W>::value_t* __restrict__ grouped, const
     for (int r = 0; r < kSubPerThread; ++r) {
         sid[r] = 0xFFFFFFFFu;
         if (!S::empty(v[r])) {
-            const u64 chunk = place_bucket<W>(v[r], nbuckets) >> unit_shift;
+            const u64 chunk = place_bucket<1>(v[r], nbuckets) >> unit_shift;
             sid[r] = min((u32)(chunk - first_chunk), nsub - 1u);
             rk[r] = atomicAdd(&s_hist[sid[r]], 1u);
         }
@@ -474,10 +461,9 @@ constexpr int kBuildBatch = 4;          // records a thread fetches before it st
 // without branches, then ONE ATOMS.CAS claims it; only a lost race (another thread took that slot meanwhile) or a full
 // bucket loops.  Probing slot by slot instead ran with ~7 of 32 lanes active and was 60 % of this kernel's issued
 // instructions.  Slots of a bucket fill in order and are never emptied, so every occupied slot precedes every empty one.
-template <int W>
-__device__ __forceinline__ int build_insert_one(typename Slot<W>::value_t* s_tab, u32 nb, u32 b, typename Slot<W>::value_t v) {
-    typedef Slot<W> S;
-    typedef typename S::value_t V;
+__device__ __forceinline__ int build_insert_one(u64* s_tab, u32 nb, u32 b, u64 v) {
+    typedef Slot<1> S;
+    typedef u64 V;
     const unsigned s_base = (unsigned)__cvta_generic_to_shared(s_tab);
     while (b < nb) {
         u64 q[4];
@@ -500,13 +486,12 @@ __device__ __forceinline__ int build_insert_one(typename Slot<W>::value_t* s_tab
     return kInsFull;                      // the probe sequence leaves the chunk
 }
 
-template <int W>
 __global__ void __launch_bounds__(kBuildThreads)
-build_chunks_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u32* __restrict__ chunk_cursor, u32 chunk_cap,
-                    typename Slot<W>::value_t* table, u64 nbuckets, int load_existing,
-                    typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap, Counters* ctr) {
-    typedef Slot<W> S;
-    typedef typename S::value_t V;
+build_chunks_kernel(const u64* __restrict__ fine, const u32* __restrict__ chunk_cursor, u32 chunk_cap,
+                    u64* table, u64 nbuckets, int load_existing,
+                    u64* __restrict__ overflow, u32 overflow_cap, Counters* ctr) {
+    typedef Slot<1> S;
+    typedef u64 V;
     extern __shared__ __align__(16) unsigned char s_raw[];
     V* s_tab = reinterpret_cast<V*>(s_raw);                            // kChunkBuckets * 32 bytes
     __shared__ u32 s_inserted, s_dups;
@@ -539,8 +524,8 @@ build_chunks_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u3
 #pragma unroll
         for (int r = 0; r < kBuildBatch; ++r) {
             if (S::empty(v[r])) continue;
-            const u32 b = (u32)(place_bucket<W>(v[r], nbuckets) - b0);      // local bucket, < nb by construction
-            const int rc = build_insert_one<W>(s_tab, nb, b, v[r]);
+            const u32 b = (u32)(place_bucket<1>(v[r], nbuckets) - b0);      // local bucket, < nb by construction
+            const int rc = build_insert_one(s_tab, nb, b, v[r]);
             inserted += (rc == kInsInserted);
             dups += (rc == kInsDuplicate);
             if (rc == kInsFull) {
@@ -567,18 +552,16 @@ build_chunks_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u3
 }
 
 // the few records the chunk build could not place: ordinary global insert, after every chunk is final
-template <int W>
 __global__ void __launch_bounds__(256)
-insert_overflow_kernel(const typename Slot<W>::value_t* __restrict__ overflow, u32 overflow_cap,
-                       typename Slot<W>::value_t* table, u64 nbuckets, Counters* ctr) {
-    typedef Slot<W> S;
+insert_overflow_kernel(const u64* __restrict__ overflow, u32 overflow_cap, u64* table, u64 nbuckets, Counters* ctr) {
+    typedef Slot<1> S;
     const u32 n = min(ctr->n_outbox, overflow_cap);
     for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const typename S::value_t v = overflow[i];
-        const u64 b = place_bucket<W>(v, nbuckets);
+        const u64 v = overflow[i];
+        const u64 b = place_bucket<1>(v, nbuckets);
         u64 q[4];
         load256_cg(table + b * S::kPerBucket, q);
-        const int rc = insert_one<W>(table, nbuckets, b, v, q);
+        const int rc = insert_one<1>(table, nbuckets, b, v, q);
         if (rc == kInsInserted) atomicAdd(&ctr->n_inserted, 1ull);
         else if (rc == kInsDuplicate) atomicAdd(&ctr->n_duplicates, 1ull);
         else atomicOr(&ctr->errors, kErrTableFull);

@@ -93,10 +93,6 @@ __device__ __forceinline__ void load256_nc(const void* p, u64 (&q)[4]) {   // re
     asm volatile("ld.global.nc.L1::no_allocate.v4.u64 {%0,%1,%2,%3}, [%4];"
                  : "=l"(q[0]), "=l"(q[1]), "=l"(q[2]), "=l"(q[3]) : "l"(p));
 }
-__device__ __forceinline__ void load256_ro(const void* p, u64 (&q)[4]) {   // read-only table, keep the line in L1/L2
-    asm volatile("ld.global.nc.v4.u64 {%0,%1,%2,%3}, [%4];"
-                 : "=l"(q[0]), "=l"(q[1]), "=l"(q[2]), "=l"(q[3]) : "l"(p));
-}
 __device__ __forceinline__ void load256_cg(const void* p, u64 (&q)[4]) {   // coherent at L2 (table being built)
     asm volatile("ld.global.cg.v4.u64 {%0,%1,%2,%3}, [%4];"
                  : "=l"(q[0]), "=l"(q[1]), "=l"(q[2]), "=l"(q[3]) : "l"(p) : "memory");
@@ -130,14 +126,12 @@ template <int W> struct Slot;
 template <> struct Slot<1> {
     typedef u64 value_t;
     static constexpr int kPerBucket = 4;
-    static constexpr int kBits = 64;
 
     static __host__ __device__ __forceinline__ value_t zero() { return 0ull; }
     static __host__ __device__ __forceinline__ bool empty(value_t v) { return v == 0ull; }
     static __host__ __device__ __forceinline__ u32 fwd(value_t v) { return (u32)(v & 7u) - 1u; }
     static __host__ __device__ __forceinline__ u32 back(value_t v) { return (u32)(v >> 3) & 7u; }
     static __host__ __device__ __forceinline__ bool same_key(value_t a, value_t b) { return ((a ^ b) >> 6) == 0ull; }
-    static __host__ __device__ __forceinline__ bool equal(value_t a, value_t b) { return a == b; }
     static __host__ __device__ __forceinline__ value_t key_only(value_t v) { return v & ~63ull; }
     static __host__ __device__ __forceinline__ u64 hash(value_t v) { return fmix64(v >> 6); }
     static __device__ __forceinline__ value_t from_bucket(const u64 (&q)[4], int i) { return q[i]; }
@@ -193,13 +187,11 @@ template <> struct Slot<1> {
     static __device__ __forceinline__ value_t cas_shared(value_t* addr, value_t expect, value_t val) {
         return atomicCAS(addr, expect, val);        // ATOMS.CAS.64
     }
-    static __device__ __forceinline__ value_t load_shared(const value_t* addr) { return *reinterpret_cast<const volatile value_t*>(addr); }
 };
 
 template <> struct Slot<2> {
     typedef u128 value_t;
     static constexpr int kPerBucket = 2;
-    static constexpr int kBits = 128;
 
     static __host__ __device__ __forceinline__ value_t zero() { return u128{0ull, 0ull}; }
     static __host__ __device__ __forceinline__ bool empty(value_t v) { return (v.lo | v.hi) == 0ull; }
@@ -208,7 +200,6 @@ template <> struct Slot<2> {
     static __host__ __device__ __forceinline__ bool same_key(value_t a, value_t b) {
         return (((a.lo ^ b.lo) >> 6) | (a.hi ^ b.hi)) == 0ull;
     }
-    static __host__ __device__ __forceinline__ bool equal(value_t a, value_t b) { return a.lo == b.lo && a.hi == b.hi; }
     static __host__ __device__ __forceinline__ value_t key_only(value_t v) { return u128{v.lo & ~63ull, v.hi}; }
     static __host__ __device__ __forceinline__ u64 hash(value_t v) {
         return fmix64((v.lo >> 6) ^ fmix64(v.hi + 0x9E3779B97F4A7C15ull));
@@ -297,10 +288,6 @@ template <> struct Slot<2> {
                      : "=l"(old.lo), "=l"(old.hi)
                      : "l"(expect.lo), "l"(expect.hi), "l"(val.lo), "l"(val.hi), "r"(saddr) : "memory");
         return old;
-    }
-    static __device__ __forceinline__ value_t load_shared(const value_t* addr) {
-        const volatile u64* p = reinterpret_cast<const volatile u64*>(addr);
-        return u128{p[0], p[1]};
     }
 };
 
@@ -470,7 +457,6 @@ constexpr u32 kLinkTail = 0xFFFFFFFFu;      // segment ends a contig (forward ex
 constexpr u32 kLinkUnused = 0xFFFFFFFEu;    // id never walked
 constexpr u32 kLinkClaimed = 0xFFFFFFFDu;   // tail claimed by a contig; low word = contig id
 constexpr u32 kLinkPending = 0xFFFFFFFCu;   // sharded walk: successor lives on another GPU, link not resolved yet
-constexpr u32 kLinkFirstMarker = kLinkPending;
 
 // where a kErrInternal came from (Counters::err_where)
 enum : u32 { kSiteBarrier = 1u, kSiteStarts = 2u, kSiteSegCap = 4u, kSiteInbox = 8u, kSiteStubOpen = 16u, kSiteOutCap = 32u };

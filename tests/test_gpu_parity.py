@@ -140,45 +140,99 @@ def test_insert_in_chunks_keeps_start_order(kh):
     assert out == d.expected()[0]
 
 
-@pytest.mark.parametrize("k,lf,chunks", [(19, 0.5, 1), (19, 0.5, 3), (19, 0.9, 1), (19, 0.97, 2), (51, 0.5, 1), (51, 0.8, 3), (31, 0.6, 2)])
-def test_chunked_shared_memory_build(kh, monkeypatch, k, lf, chunks):
-    """Large batches are built chunk by chunk in shared memory (no global atomics); batches after the first
-    load the existing chunk back in.  KH_PARTITION=1 forces the partitioned paths on a small table; KH_BUILD=0 is
-    the atomic insert_slots path -- all must give the reference's bytes."""
-    d = kmergen.Dataset(k, 300000, 900, seed=int(lf * 100) + k)
-    want = d.expected()[0]
-    monkeypatch.setenv("KH_PARTITION", "1")
-    for build in ("1", "0"):
-        monkeypatch.setenv("KH_BUILD", build)
-        out, _, nodes, st = _assemble_text(kh, d.text(), k, load_factor=lf, chunks=chunks)
-        assert out == want and nodes == d.n
-        assert st["n_inserted"] == d.n and st["n_duplicates"] == 0
+@pytest.fixture(scope="module")
+def large_set():
+    """(records, expected output) of a kmergen set, made once per (k, n) for the large plain-table cases below: seed 267
+    and the contig density of the test.txt shape (4 514 197 k-mers in 5 736 contigs)."""
+    made = {}
+
+    def get(k, n):
+        if (k, n) not in made:
+            d = kmergen.Dataset(k, n, round(n / 787), seed=267)
+            made[k, n] = d.pairs(), d.expected()[0]
+            d.close()
+        return made[k, n]
+    return get
 
 
-@pytest.mark.parametrize("build", ["1", "0"])
-@pytest.mark.parametrize("pct", ["70", "20"])
-def test_grouping_buffer_overflow_paths(kh, monkeypatch, build, pct):
-    """The grouping buffers are sized for the expected share plus slack; the rare record that does not fit is
-    inserted directly (atomic path) or through the fix-up list (chunked build).  KH_DEBUG_CAP_PCT shrinks the
-    buffers so a large part of the input takes those paths -- the result must not change."""
-    monkeypatch.setenv("KH_PARTITION", "1")
-    monkeypatch.setenv("KH_BUILD", build)
-    monkeypatch.setenv("KH_DEBUG_CAP_PCT", pct)
-    for k in (19, 51):
-        d = kmergen.Dataset(k, 250000, 700, seed=int(pct) + k)
-        out, _, nodes, st = _assemble_text(kh, d.text(), k, chunks=2)
-        assert out == d.expected()[0] and nodes == d.n and st["n_inserted"] == d.n
+# Kernels a plain-table insert call launches on each path.  The call adds 3 for the start-list scan, and 1 more when it
+# brings new start nodes.
+_PATH_OF_LAUNCHES = {1: "direct", 3: "insert_slots", 4: "chunked"}
 
 
-def test_chunked_build_counts_duplicates(kh, monkeypatch):
-    monkeypatch.setenv("KH_PARTITION", "1")
-    d = kmergen.Dataset(19, 200000, 300, seed=44)
-    pairs = d.pairs()
-    with kh.KmerHashTable(19, 400000) as tab:
-        tab.insert_pairs(pairs)
-        tab.insert_pairs(pairs[:150000])               # a second large batch: every record is already there
+def _insert_paths(tab, pairs, batches):
+    """Insert `pairs` from the host in `batches` calls, each within one 64 MB staging piece; the path each call took."""
+    paths, step = [], -(-len(pairs) // batches)
+    for lo in range(0, len(pairs), step):
+        before = tab.stats()
+        tab.insert_pairs(pairs[lo:lo + step])
+        after = tab.stats()
+        launches = after["n_launches"] - before["n_launches"] - 3 - int(after["n_starts"] > before["n_starts"])
+        paths.append(_PATH_OF_LAUNCHES.get(launches, launches))
+    return paths
+
+
+def _large_plain(kh, monkeypatch, large_set, k, n, lf, batches):
+    """Build a plain table (KH_CT=0) of n k-mers in `batches` calls and check its output; the paths the calls took."""
+    monkeypatch.setenv("KH_CT", "0")
+    pairs, want = large_set(k, n)
+    with kh.KmerHashTable(k, n, lf) as tab:
+        paths = _insert_paths(tab, pairs, batches)
+        buf, _, nodes = tab.assemble()
         st = tab.stats()
-        assert st["n_inserted"] == 200000 and st["n_duplicates"] == 150000
+    assert buf.tobytes() == want and nodes == n
+    assert st["n_inserted"] == n and st["n_duplicates"] == 0
+    return paths
+
+
+# (k, load factor, batches) -> (k-mers, path of every batch).  Every table is over 64 MiB (n / lf above 8.39 M for
+# 64-bit slots, 4.19 M for 128-bit slots), so each call of >= 65 536 records is grouped by table region.
+_LARGE_PLAIN = {
+    (19, 0.5, 1): (4514197, "chunked"),
+    (19, 0.5, 3): (4514197, "chunked"),            # batches after the first load the existing chunks back in
+    (19, 0.5, 5): (4514197, "insert_slots"),       # each batch under 1/8 of the table's slots
+    (19, 0.9, 1): (8_000_000, "chunked"),
+    (19, 0.97, 2): (8_200_000, "chunked"),
+    (19, 0.97, 8): (8_200_000, "insert_slots"),
+    (51, 0.5, 1): (2_200_000, "insert_slots"),     # 128-bit slots always take insert_slots
+    (51, 0.8, 3): (3_500_000, "insert_slots"),
+    (31, 0.6, 2): (2_600_000, "insert_slots"),
+}
+
+
+@pytest.mark.parametrize("k,lf,chunks", list(_LARGE_PLAIN))
+def test_chunked_shared_memory_build(kh, monkeypatch, large_set, k, lf, chunks):
+    """Into a table larger than L2, a batch of at least 1/8 of its 64-bit slots is built chunk by chunk in shared memory
+    (no global atomics); smaller batches and 128-bit slots go through the atomic insert_slots path.  Each case reaches
+    its path through table and batch size, and all must give the reference's bytes."""
+    n, path = _LARGE_PLAIN[k, lf, chunks]
+    assert _large_plain(kh, monkeypatch, large_set, k, n, lf, chunks) == [path] * chunks
+
+
+@pytest.mark.parametrize("chunked", [1, 0])
+@pytest.mark.parametrize("pct", ["70", "20"])
+def test_grouping_buffer_overflow_paths(kh, monkeypatch, large_set, chunked, pct):
+    """The grouping buffers are sized for the expected share plus slack; the rare record that does not fit goes through
+    the fix-up list (chunked build) or is inserted directly by partition_kernel (insert_slots path).  KH_DEBUG_CAP_PCT
+    shrinks the buffers so a large part of the input takes those paths -- the result must not change."""
+    monkeypatch.setenv("KH_DEBUG_CAP_PCT", pct)
+    cases = [(19, 4514197, 2, "chunked")] if chunked else [(19, 4514197, 5, "insert_slots"), (51, 2_200_000, 2, "insert_slots")]
+    for k, n, batches, path in cases:
+        assert _large_plain(kh, monkeypatch, large_set, k, n, 0.5, batches) == [path] * batches
+
+
+def test_chunked_build_counts_duplicates(kh, large_set):
+    """Records already in the table are counted as duplicates by the chunked build and by insert_slots."""
+    n = 4514197
+    pairs, _ = large_set(19, n)
+    with kh.KmerHashTable(19, n) as tab:
+        assert _insert_paths(tab, pairs, 1) == ["chunked"]
+        assert _insert_paths(tab, pairs[:3_000_000], 1) == ["chunked"]          # a second large batch, all present
+        st = tab.stats()
+        assert st["n_inserted"] == n and st["n_duplicates"] == 3_000_000
+        assert _insert_paths(tab, pairs[:900_000], 1) == ["insert_slots"]
+        st = tab.stats()
+        assert st["n_inserted"] == n and st["n_duplicates"] == 3_900_000
 
 
 def test_insert_lines_path(kh):
