@@ -38,6 +38,7 @@ ABI_SYMBOLS = [
     "kh_count_create", "kh_count_destroy", "kh_count_clear", "kh_count_reads", "kh_count_reads_device",
     "kh_count_extract", "kh_count_extract_device", "kh_count_extract_lines", "kh_count_lookup", "kh_count_get_stats", "kh_count_last_error",
     "kh_count_record_bytes", "kh_count_partition", "kh_count_merge_device", "kh_count_histogram", "kh_count_auto_min_count",
+    "kh_count_contig_depth", "kh_count_contig_depth_device",
 ]
 
 
@@ -140,6 +141,8 @@ def lib() -> C.CDLL:
     L.kh_count_histogram.argtypes = [vp, pu64]
     L.kh_count_auto_min_count.argtypes = [pu64]
     L.kh_count_auto_min_count.restype = u32
+    L.kh_count_contig_depth.argtypes = [vp, vp, vp, u64, u32, u32, vp]
+    L.kh_count_contig_depth_device.argtypes = [vp, vp, vp, u64, u32, u32, vp]
     _lib = L
     return L
 
@@ -394,6 +397,24 @@ class KmerCounter:
         self._check(lib().kh_count_histogram(self._h, h.ctypes.data_as(C.POINTER(C.c_uint64))))
         return h
 
+    def contig_depth(self, text, offsets, world: int = 1, rank: int = 0) -> np.ndarray:
+        """Per contig [offsets[i], offsets[i+1]) of `text`: its windows and the sum / min / max of their k-mers'
+        occurrence counts (kh_count_contig_depth), as a DEPTH_DTYPE array; depth = sum / n_kmers.  world > 1: only the
+        k-mers owner `rank` owns (combine the owners' partials with combine_depth)."""
+        t = np.frombuffer(text, dtype=np.uint8) if not isinstance(text, np.ndarray) else np.ascontiguousarray(text)
+        offs = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = max(offs.size - 1, 0)
+        if n and int(offs[-1]) > t.size:
+            raise ValueError("offsets reach past the end of the text")
+        out = np.zeros(n, dtype=DEPTH_DTYPE)
+        self._check(lib().kh_count_contig_depth(self._h, t.ctypes.data, offs.ctypes.data, n, world, rank, out.ctypes.data))
+        return out
+
+    def contig_depth_device(self, contigs_ptr: int, offsets_ptr: int, n: int, out_ptr: int, world: int = 1, rank: int = 0) -> None:
+        """kh_count_contig_depth_device: contig text, n + 1 offsets and n 24-byte records, all in the counter's device
+        memory (e.g. KmerHashTable.assemble_device's output).  Host-synchronous."""
+        self._check(lib().kh_count_contig_depth_device(self._h, contigs_ptr, offsets_ptr, n, world, rank, out_ptr))
+
     def stats(self) -> dict:
         s = CountStats()
         self._check(lib().kh_count_get_stats(self._h, C.byref(s)))
@@ -419,6 +440,22 @@ class KmerCounter:
 
 
 HIST_BINS = 256
+
+# kh_contig_depth: one record per contig (24 bytes)
+DEPTH_DTYPE = np.dtype([("n_kmers", np.uint64), ("sum", np.uint64), ("min", np.uint32), ("max", np.uint32)])
+assert DEPTH_DTYPE.itemsize == 24
+
+
+def combine_depth(parts) -> np.ndarray:
+    """Contig depth partials of disjoint window sets (one per owner) -> the records over all of them: +, +, min, max."""
+    parts = list(parts)
+    out = parts[0].copy()
+    for p in parts[1:]:
+        out["n_kmers"] += p["n_kmers"]
+        out["sum"] += p["sum"]
+        out["min"] = np.minimum(out["min"], p["min"])
+        out["max"] = np.maximum(out["max"], p["max"])
+    return out
 
 
 def auto_min_count(hist) -> int:

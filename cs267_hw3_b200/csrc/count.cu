@@ -9,6 +9,7 @@
 //   kc_extract_kernel  table scan -> kmer_pair records of the k-mers with enough occurrences (block-wise compaction)
 //   kc_lookup_kernel   counters of given k-mers
 //   kc_histogram_kernel  table scan -> the k-mer spectrum (distinct k-mers per occurrence count)
+//   kc_depth_kernel    contig text -> per contig: windows, sum / min / max of their k-mers' occurrences (read-only)
 //
 // HBM-bound integer work like the rest of the library: what an occurrence costs is one random 32-byte sector (the slot)
 // read and written back.  Algorithmic bytes per occurrence = 1 (the character) + 64.
@@ -239,6 +240,85 @@ kc_histogram_kernel(const u64* __restrict__ table, u64 n_slots, u64* __restrict_
         if (s_bin[b]) atomicAdd(&hist[b], (u64)s_bin[b]);
 }
 
+// Contig depth (kh_count_contig_depth*): one block per 2048-byte tile of the contig text [offsets[0], offsets[n]), seen
+// through `seg` = the text at offsets[0], so nothing outside that range is read.  The tile is packed and its windows
+// listed as in kc_count_kernel (positions past the range read as separators).  A block first finds the contigs its
+// tile touches (two binary searches over offsets), then every listed position searches only that range; windows that
+// run past their contig's end, or whose k-mer another rank owns, are dropped.  The lookup is read-only (kc_find).  The
+// loop bound is warp-uniform: lanes without a window carry kKcNoContig, the lanes of one contig are grouped with
+// __match_any_sync and reduced with __reduce_*_sync, and the group's first lane adds the group into the record with
+// integer atomics -- the records do not depend on the schedule.  Tiles cost the same whatever the contig lengths: a
+// 10^6-k-mer contig is spread over ~500 blocks, and a tile of hundreds of short contigs costs one more search level.
+template <int W>
+__global__ void __launch_bounds__(kKcThreads, 8)
+kc_depth_kernel(const unsigned char* __restrict__ seg, u64 span, u64 p_begin, const u64* __restrict__ offsets, u64 n_contigs,
+                const u64* __restrict__ table, u64 n_slots, int k, u32 world, u32 rank, KcDepth* __restrict__ out) {
+    __shared__ u32 s_code[kKcWords], s_inv[kKcWords];
+    __shared__ unsigned short s_list[kKcTile];
+    __shared__ u32 s_n;
+    __shared__ u64 s_lo, s_hi;
+    const u64 t0 = (u64)blockIdx.x * kKcTile;
+    if (threadIdx.x == 0) {
+        s_n = 0;
+        s_lo = kc_contig_of(offsets, 0, n_contigs, p_begin + t0);
+    } else if (threadIdx.x == 32) {
+        const u64 last = p_begin + (t0 + kKcTile < span ? t0 + kKcTile : span) - 1;
+        s_hi = kc_contig_of(offsets, 0, n_contigs, last) + 1;
+    }
+    for (u32 i = threadIdx.x; i < kKcWords; i += kKcThreads)
+        kc_pack_word(seg, span, (long long)t0 - 16 + 16ll * (long long)i, s_code[i], s_inv[i]);
+    __syncthreads();
+    const u32 lane = threadIdx.x & 31u;
+#pragma unroll
+    for (int r = 0; r < kKcPer; ++r) {
+        const u32 local = threadIdx.x + (u32)r * kKcThreads;
+        const bool ok = t0 + local < span && kc_kmer_valid(s_inv, local, k);
+        const u32 bal = __ballot_sync(kFull, ok);
+        u32 base = 0;
+        if (lane == 0 && bal) base = atomicAdd(&s_n, (u32)__popc(bal));
+        base = __shfl_sync(kFull, base, 0);
+        if (ok) s_list[base + (u32)__popc(bal & ((1u << lane) - 1u))] = (unsigned short)local;
+    }
+    __syncthreads();
+    // offsets that decrease somewhere could give hi <= lo: the range stays non-empty and inside [0, n_contigs)
+    const u64 lo = s_lo, hi = s_hi > lo ? s_hi : lo + 1;
+    const u32 cnt = s_n;
+#pragma unroll 1
+    for (u32 i0 = threadIdx.x & ~31u; i0 < cnt; i0 += kKcThreads) {
+        const u32 i = i0 + lane;
+        u64 c = kKcNoContig;
+        u32 v = 0;
+        if (i < cnt) {
+            const u32 local = s_list[i];
+            const u64 p = p_begin + t0 + local;
+            const u64 cc = kc_contig_of(offsets, lo, hi, p);
+            if (kc_window_in_contig(offsets, cc, p, k)) {
+                const KcOcc o = kc_position(s_code, s_inv, local, k);
+                if (world == 1 || kc_owner(o.key_hi, o.key_lo, world) == rank) {
+                    c = cc;
+                    v = kc_depth_value<W>(table, n_slots, o.key_hi, o.key_lo);
+                }
+            }
+        }
+        const u32 peers = __match_any_sync(kFull, c);
+        if (c != kKcNoContig) {
+            const u32 sum = __reduce_add_sync(peers, v), mn = __reduce_min_sync(peers, v), mx = __reduce_max_sync(peers, v);
+            if (lane == (u32)__ffs(peers) - 1u) {
+                KcDepth* rec = out + c;
+                atomicAdd(&rec->n_kmers, (u64)__popc(peers));
+                atomicAdd(&rec->sum, (u64)sum);
+                atomicMin(&rec->min, mn);
+                atomicMax(&rec->max, mx);
+            }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) kc_depth_init_kernel(KcDepth* __restrict__ out, u64 n) {
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x)
+        out[i] = KcDepth{0ull, 0ull, kKcDepthNoMin, 0u};
+}
+
 template <int W>
 __global__ void __launch_bounds__(256)
 kc_lookup_kernel(const u64* __restrict__ table, u64 n_slots, int k, const unsigned char* __restrict__ pkmers, u64 n, u32* __restrict__ counts_out) {
@@ -292,6 +372,8 @@ struct kh_counter {
     size_t cursor_cap = 0;
     void* hist = nullptr;             // kh_count_histogram: 256 x u64 bins
     size_t hist_cap = 0;
+    void* depth = nullptr;            // kh_count_contig_depth: records | offsets | contig text
+    size_t depth_cap = 0;
     u64 peers_enabled = 0;            // bit d: this counter's device reads device d's memory directly
     u64 n_bytes = 0;
     u32 n_launches = 0;
@@ -397,6 +479,33 @@ int kc_launch_count(kh_counter* c, const unsigned char* buf, u64 n, u64 p_begin,
     return KH_OK;
 }
 
+static_assert(sizeof(KcDepth) == sizeof(kh_contig_depth) && sizeof(KcDepth) == 24, "kh_contig_depth layout");
+
+int kc_depth_check(kh_counter* c, bool null_arg, u64 n, uint32_t world, uint32_t rank, const char* what) {
+    if (!c) return KH_ERR_ARG;
+    if (n && null_arg) return kc_fail(c, KH_ERR_ARG, std::string(what) + ": null pointer");
+    if (world < 1 || world > kKcMaxWorld || rank >= world) return kc_fail(c, KH_ERR_ARG, std::string(what) + ": 1 <= world <= 64 and rank < world");
+    return KH_OK;
+}
+
+// records initialised, then the tiles of [p_begin, p_begin + span) (seg = the text at p_begin); host waits for both
+int kc_launch_depth(kh_counter* c, const unsigned char* seg, u64 span, u64 p_begin, const u64* offsets, u64 n, u32 world, u32 rank, KcDepth* out) {
+    const u64 blocks = (span + kKcTile - 1) / kKcTile;
+    if (blocks > 0x7FFFFFFFull) return kc_fail(c, KH_ERR_ARG, "kh_count_contig_depth: at most 2^42 bytes of contig text per call");
+    kc_depth_init_kernel<<<(unsigned)std::min<u64>((n + 255) / 256, 4096), 256, 0, c->stream>>>(out, n);
+    KC_CUDA(c, cudaGetLastError());
+    ++c->n_launches;
+    if (blocks) {
+        const unsigned g = (unsigned)blocks;
+        if (c->W == 1) kc_depth_kernel<1><<<g, kKcThreads, 0, c->stream>>>(seg, span, p_begin, offsets, n, c->table, c->n_slots, c->k, world, rank, out);
+        else kc_depth_kernel<2><<<g, kKcThreads, 0, c->stream>>>(seg, span, p_begin, offsets, n, c->table, c->n_slots, c->k, world, rank, out);
+        KC_CUDA(c, cudaGetLastError());
+        ++c->n_launches;
+    }
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    return KH_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -450,7 +559,7 @@ int kh_count_destroy(kh_counter* c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     cudaFree(c->table); cudaFree(c->d_ctr); cudaFree(c->stage[0]); cudaFree(c->stage[1]); cudaFree(c->out); cudaFree(c->scratch);
-    cudaFree(c->outbox); cudaFree(c->inbox); cudaFree(c->cursor); cudaFree(c->hist);
+    cudaFree(c->outbox); cudaFree(c->inbox); cudaFree(c->cursor); cudaFree(c->hist); cudaFree(c->depth);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     if (c->ev2) cudaEventDestroy(c->ev2);
@@ -714,6 +823,46 @@ int kh_count_histogram(kh_counter* c, uint64_t* hist_host_out) {
 }
 
 uint32_t kh_count_auto_min_count(const uint64_t* hist) { return kc_auto_min_count(reinterpret_cast<const u64*>(hist)); }
+
+// Host contigs: the records, the offsets and the text [offsets[0], offsets[n]) share one counter-owned buffer.
+int kh_count_contig_depth(kh_counter* c, const char* contigs_host, const uint64_t* offsets_host, uint64_t n_contigs, uint32_t world,
+                          uint32_t rank, kh_contig_depth* out_host) {
+    KC_TRY(kc_depth_check(c, !contigs_host || !offsets_host || !out_host, n_contigs, world, rank, "kh_count_contig_depth"));
+    if (n_contigs == 0) return KH_OK;
+    for (u64 i = 0; i < n_contigs; ++i)
+        if (offsets_host[i + 1] < offsets_host[i]) return kc_fail(c, KH_ERR_ARG, "kh_count_contig_depth: offsets must be non-decreasing");
+    KC_CUDA(c, cudaSetDevice(c->device));
+    KC_TRY(kc_settle(c));                                   // a table that overflowed while counting is reported here
+    const u64 p_begin = offsets_host[0], span = offsets_host[n_contigs] - p_begin;
+    const size_t rec_bytes = ((size_t)n_contigs * sizeof(KcDepth) + 15) & ~(size_t)15;
+    const size_t off_bytes = ((size_t)(n_contigs + 1) * sizeof(u64) + 15) & ~(size_t)15;
+    KC_TRY(kc_grow(c, &c->depth, &c->depth_cap, rec_bytes + off_bytes + (size_t)span));
+    unsigned char* base = static_cast<unsigned char*>(c->depth);
+    KcDepth* d_out = reinterpret_cast<KcDepth*>(base);
+    u64* d_off = reinterpret_cast<u64*>(base + rec_bytes);
+    unsigned char* d_text = base + rec_bytes + off_bytes;
+    KC_CUDA(c, cudaMemcpyAsync(d_off, offsets_host, (size_t)(n_contigs + 1) * sizeof(u64), cudaMemcpyHostToDevice, c->stream));
+    if (span) KC_CUDA(c, cudaMemcpyAsync(d_text, contigs_host + p_begin, (size_t)span, cudaMemcpyHostToDevice, c->stream));
+    KC_TRY(kc_launch_depth(c, d_text, span, p_begin, d_off, n_contigs, world, rank, d_out));
+    KC_CUDA(c, cudaMemcpyAsync(out_host, d_out, (size_t)n_contigs * sizeof(KcDepth), cudaMemcpyDeviceToHost, c->stream));
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    return KH_OK;
+}
+
+int kh_count_contig_depth_device(kh_counter* c, const char* contigs_dev, const uint64_t* offsets_dev, uint64_t n_contigs, uint32_t world,
+                                 uint32_t rank, kh_contig_depth* out_dev) {
+    KC_TRY(kc_depth_check(c, !contigs_dev || !offsets_dev || !out_dev, n_contigs, world, rank, "kh_count_contig_depth_device"));
+    if (n_contigs == 0) return KH_OK;
+    KC_CUDA(c, cudaSetDevice(c->device));
+    KC_TRY(kc_settle(c));
+    u64 ends[2];                                            // offsets[0] and offsets[n]: the text range and the grid
+    KC_CUDA(c, cudaMemcpyAsync(&ends[0], offsets_dev, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+    KC_CUDA(c, cudaMemcpyAsync(&ends[1], offsets_dev + n_contigs, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    const u64 span = ends[1] > ends[0] ? ends[1] - ends[0] : 0ull;
+    return kc_launch_depth(c, reinterpret_cast<const unsigned char*>(contigs_dev) + ends[0], span, ends[0], reinterpret_cast<const u64*>(offsets_dev),
+                           n_contigs, world, rank, reinterpret_cast<KcDepth*>(out_dev));
+}
 
 int kh_count_lookup(kh_counter* c, const void* pkmers_host, uint64_t n, uint32_t* counts_host_out) {
     if (!c || (n && (!pkmers_host || !counts_host_out))) return KH_ERR_ARG;

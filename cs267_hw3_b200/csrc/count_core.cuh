@@ -450,6 +450,38 @@ inline u32 kc_auto_min_count(const u64* hist) {
     }
     return kKcDefaultMinCount;
 }
+// ---- contig depth (kh_count_contig_depth*) ---------------------------------------------------------------------
+// Contig c is the text [offsets[c], offsets[c+1]); a window is a position p with p + K <= offsets[c+1] whose K bytes are
+// bases; its value is the k-mer's occurrence count (kc_total, 0 when never seen).  Per contig: windows, sum, min, max --
+// the layout of kh_contig_depth.  Partials of disjoint window sets (the owners' of a sharded counter) combine field by
+// field: +, +, min, max.
+struct KcDepth {
+    u64 n_kmers, sum;
+    u32 min, max;
+};
+constexpr u32 kKcDepthNoMin = 0xFFFFFFFFu;
+constexpr u64 kKcNoContig = ~0ull;                          // the sentinel contig of a lane without a window
+
+// The contig holding byte p: the largest c in [lo, hi) with offsets[c] <= p (empty contigs share their offset with the
+// next one, so the largest is the one the byte belongs to).  Needs offsets[lo] <= p; returns lo when no c qualifies.
+__host__ __device__ __forceinline__ u64 kc_contig_of(const u64* offsets, u64 lo, u64 hi, u64 p) {
+    while (hi - lo > 1) {
+        const u64 mid = lo + (hi - lo) / 2;
+        if (offsets[mid] <= p) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+// the window at byte p (all K bytes are bases) belongs to contig c when it starts inside it and ends by its end
+__host__ __device__ __forceinline__ bool kc_window_in_contig(const u64* offsets, u64 c, u64 p, int k) {
+    return offsets[c] <= p && p + (u64)k <= offsets[c + 1];
+}
+// the value of one window: its k-mer's occurrences, read-only
+template <int W>
+__host__ __device__ __forceinline__ u32 kc_depth_value(const u64* table, u64 n_slots, u64 key_hi, u64 key_lo) {
+    return kc_total(kc_find<W>(table, n_slots, key_hi, key_lo));
+}
+
 template <int W>
 __host__ __device__ __forceinline__ void kc_slot_record(const u64* table, u64 i, int k, u32 min_ext, unsigned char* rec) {
     const u64* p = table + i * (u64)KcSlot<W>::kWords;

@@ -155,6 +155,13 @@ class ShardedCounter:
         k-mer has one owner and the owned counters equal one counter's, so the sum of the owners' spectra is exact."""
         return np.sum([c.histogram() for c in self.owned], axis=0, dtype=np.uint64)
 
+    def contig_depth(self, text, offsets) -> np.ndarray:
+        """After reduce(): KmerCounter.contig_depth against everything reduced so far.  Owner o looks up the windows
+        whose k-mer it owns; every k-mer has one owner, so the combined partials are exactly one counter's records."""
+        import cs267_hw3_b200 as kh
+
+        return kh.combine_depth(self._each(lambda o: self.owned[o].contig_depth(text, offsets, self.world, o)))
+
     def lookup(self, rank: int, pkmers) -> np.ndarray:
         return self.owned[rank].lookup(pkmers)
 

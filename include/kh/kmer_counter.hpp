@@ -17,6 +17,14 @@
 
 namespace kh {
 
+// Contig depth partials of disjoint window sets (one per owner of a sharded counter) -> the record over all of them
+inline void combine_depth(kh_contig_depth& into, const kh_contig_depth& part) {
+    into.n_kmers += part.n_kmers;
+    into.sum += part.sum;
+    into.min = part.min < into.min ? part.min : into.min;
+    into.max = part.max > into.max ? part.max : into.max;
+}
+
 class KmerCounter {
     kh_counter* c_ = nullptr;
     int k_;
@@ -72,6 +80,12 @@ class KmerCounter {
         std::array<uint64_t, 256> h{};
         check(kh_count_histogram(c_, h.data()), "histogram");
         return h;
+    }
+    // per contig [offsets[i], offsets[i+1]) of text: its k-mers' occurrence counts, kh_count_contig_depth (world 1)
+    std::vector<kh_contig_depth> contig_depth(const char* text, const uint64_t* offsets, uint64_t n) {
+        std::vector<kh_contig_depth> out(n);
+        check(kh_count_contig_depth(c_, text, offsets, n, 1, 0, out.data()), "contig_depth");
+        return out;
     }
     kh_count_stats stats() {
         kh_count_stats s{};

@@ -25,6 +25,7 @@
 #include <vector>
 
 #include "../kh_capi.h"
+#include "kmer_counter.hpp"
 
 namespace kh_sharded {
 
@@ -164,6 +165,21 @@ class CountCluster {
             for (size_t c = 0; c < h.size(); ++c) sum[c] += h[c];
         }
         return sum;
+    }
+
+    // After reduce(): the depth of contigs [offsets[i], offsets[i+1]) of host text against everything reduced so far.
+    // Every owner looks up the windows whose k-mer it owns (kh_count_contig_depth with world, rank = owner); every
+    // k-mer has exactly one owner, so the partials combine into exactly one counter's records.
+    std::vector<kh_contig_depth> contig_depth(const char* text, const uint64_t* offsets, uint64_t n) {
+        std::vector<std::vector<kh_contig_depth>> part(world_, std::vector<kh_contig_depth>(n));
+        each_rank([&](int o) {
+            count_must(kh_count_contig_depth(owned_[o], text, offsets, n, (uint32_t)world_, (uint32_t)o, part[o].data()), owned_[o],
+                       "contig_depth");
+        });
+        std::vector<kh_contig_depth> out(n, kh_contig_depth{0, 0, UINT32_MAX, 0});
+        for (int o = 0; o < world_; ++o)
+            for (uint64_t i = 0; i < n; ++i) kh::combine_depth(out[i], part[o][i]);
+        return out;
     }
 
     // totals over all ranks: occurrences and read bytes counted (reduced or not), distinct k-mers reduced so far

@@ -299,6 +299,31 @@ int kh_count_merge_device(kh_counter* c, const void* records_dev, uint64_t n);
  * the result like any other min_count. */
 int kh_count_histogram(kh_counter* c, uint64_t* hist_host_out);
 uint32_t kh_count_auto_min_count(const uint64_t* hist);
+/* Contig depth: the mean occurrence count of a contig's k-mers in the reads (the `cov` assemblers report), straight from
+ * the counter.  Contig i is the text [offsets[i], offsets[i+1]) -- '\n'-separated or not, e.g. kh_assemble* output.
+ *   A window is a position p with p + K <= offsets[i+1] whose K bytes are all ACGT: windows never cross a contig
+ *   boundary or a non-base byte (a trailing '\n' is simply not a base).
+ *   Its value is the counter's occurrence count of that k-mer -- saturated at 255, the count kh_count_histogram bins --
+ *   and 0 for a k-mer the counter never saw.  Depth above 255x is therefore reported as 255x: the occurrence counter
+ *   is 8 bits wide.
+ * Per contig: n_kmers windows looked up, the sum / min / max of their values; depth = sum / n_kmers.
+ * world > 1: only windows whose k-mer belongs to owner `rank` (the owner kh_count_partition groups by) are looked up --
+ * the partial of a sharded counter's owned counter `rank`.  Every k-mer has exactly one owner, so the partials of ranks
+ * 0..world-1 combine field by field (+, +, min, max) into exactly the world = 1 record.  1 <= world <= 64, rank < world.
+ * kh_count_contig_depth: host text, offsets (n_contigs + 1, non-decreasing) and records; they travel through
+ * counter-owned device buffers.  kh_count_contig_depth_device: all three in memory of the counter's device (e.g.
+ * kh_assemble_device's output read in place); only records 0..n_contigs-1 are written and only text inside
+ * [offsets[0], offsets[n_contigs]) is read.  Both are host-synchronous, return KH_ERR_TABLE_FULL after a count that
+ * overflowed the table, and with n_contigs = 0 return KH_OK without launching anything. */
+typedef struct kh_contig_depth {
+    uint64_t n_kmers;          /* windows looked up (world > 1: only those `rank` owns)           */
+    uint64_t sum;              /* sum of their values                                             */
+    uint32_t min, max;         /* UINT32_MAX / 0 when n_kmers == 0                                */
+} kh_contig_depth;             /* 24 bytes */
+int kh_count_contig_depth(kh_counter* c, const char* contigs_host, const uint64_t* offsets_host, uint64_t n_contigs,
+                          uint32_t world, uint32_t rank, kh_contig_depth* out_host);
+int kh_count_contig_depth_device(kh_counter* c, const char* contigs_dev, const uint64_t* offsets_dev, uint64_t n_contigs,
+                                 uint32_t world, uint32_t rank, kh_contig_depth* out_dev);
 
 /* Introspection for tests and debugging: device pointer and capacity of an internal buffer of a chunk table
  * ("link", "meta", "chunk_base", "seg_base", "chunk_cursor", "counters", ...; "caps" returns HOST numbers). */

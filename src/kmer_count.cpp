@@ -1,7 +1,7 @@
 // kmer_count -- reads -> the reference's k-mer file, or straight to contigs, on the B200 library.
 //
 //   kmer_count K reads_file [--histo HISTO_FILE] kmer_file_out   [min_count [min_ext]]
-//   kmer_count K reads_file [--histo HISTO_FILE] --contigs PREFIX [min_count [min_ext]]
+//   kmer_count K reads_file [--histo HISTO_FILE] [--depth] --contigs PREFIX [min_count [min_ext]]
 //   kmer_count K reads_file --histo HISTO_FILE
 //
 // The first form writes what the reference's read_kmers parses (read_kmers.hpp:64-76: K bases, a blank, backward and
@@ -17,6 +17,10 @@
 // GenomeScope reads: "c n" per line for every count c in 1..255 with n > 0 distinct k-mers, ascending; 255 stands for
 // 255 or more.  With --histo alone nothing else is written.  min_count may be the word `auto`: the valley of the
 // spectrum (kh_count_auto_min_count).  Whenever the spectrum is computed, one more stdout line reports it.
+//
+// --depth (with --contigs only) writes PREFIX_r.depth next to every PREFIX_r.dat: line j describes line j of the .dat as
+// "n_kmers mean min max" -- the contig's k-mers, the mean (%.2f), least and largest of their occurrence counts in the
+// reads (kh_count_contig_depth; counts saturate at 255) -- and one more stdout line reports the overall mean.
 // Environment: KH_DEVICE, KH_LOAD_FACTOR (0.5), KH_COUNT_DISTINCT = distinct k-mers to size the table for, erroneous
 // ones included (default: half the input bytes).
 //
@@ -49,8 +53,8 @@ void must(int status, kh_table* t, const char* what) {
 }
 
 int usage() {
-    fprintf(stderr, "Usage: kmer_count K reads_file [--histo HISTO_FILE] [kmer_file_out | --contigs PREFIX] [min_count|auto [min_ext]]\n"
-                    "       (the output may be left out only with --histo)\n");
+    fprintf(stderr, "Usage: kmer_count K reads_file [--histo HISTO_FILE] [--depth] [kmer_file_out | --contigs PREFIX] [min_count|auto [min_ext]]\n"
+                    "       (the output may be left out only with --histo; --depth needs --contigs)\n");
     return 1;
 }
 
@@ -70,6 +74,25 @@ void spectrum(const std::array<uint64_t, 256>& hist, int k, const std::string& h
     if (auto_min_count) min_count = valley;
     printf("Spectrum of %llu distinct %d-mers%s%s: min_count %u, auto min_count %u\n", (unsigned long long)distinct, k,
            histo.empty() ? "" : " written to ", histo.c_str(), min_count, valley);
+}
+
+// PREFIX_r.depth: line j = "n_kmers mean min max" of contig j (line j of PREFIX_r.dat); adds to the totals
+void write_depth(const std::string& name, const std::vector<kh_contig_depth>& d, uint64_t& n_kmers, uint64_t& sum) {
+    FILE* o = fopen(name.c_str(), "wb");
+    if (o == nullptr) throw std::runtime_error("kmer_count: could not open " + name);
+    for (const kh_contig_depth& r : d) {
+        const double mean = r.n_kmers ? (double)r.sum / (double)r.n_kmers : 0.0;
+        if (fprintf(o, "%llu %.2f %u %u\n", (unsigned long long)r.n_kmers, mean, r.min, r.max) < 0)
+            throw std::runtime_error("kmer_count: short write to " + name);
+        n_kmers += r.n_kmers;
+        sum += r.sum;
+    }
+    if (fclose(o) != 0) throw std::runtime_error("kmer_count: short write to " + name);
+}
+
+void report_depth(uint64_t n_contigs, uint64_t n_kmers, uint64_t sum, const std::string& prefix, int ranks) {
+    printf("Depth of %llu contigs (%llu k-mers): mean %.2f; wrote %s_0.depth .. %s_%d.depth\n", (unsigned long long)n_contigs,
+           (unsigned long long)n_kmers, n_kmers ? (double)sum / (double)n_kmers : 0.0, prefix.c_str(), prefix.c_str(), ranks - 1);
 }
 
 // The file goes through in pieces of about `buffer` bytes that end on a line boundary (FASTA: before a header); each
@@ -100,7 +123,7 @@ template <class Sink> void read_pieces(FILE* f, size_t buffer, Sink sink) {
 }
 
 int count_sharded(FILE* f, int k, int ranks, uint64_t distinct, double lf, bool contigs, const std::string& out_name,
-                  const std::string& histo, bool auto_min_count, uint32_t min_count, uint32_t min_ext) {
+                  const std::string& histo, bool auto_min_count, uint32_t min_count, uint32_t min_ext, bool depth) {
     using clock = std::chrono::high_resolution_clock;
     const uint64_t batch = getenv("KH_COUNT_BATCH_BYTES") ? strtoull(getenv("KH_COUNT_BATCH_BYTES"), nullptr, 10) : 0;
     const size_t buffer = batch ? (size_t)std::min<uint64_t>(128u << 20, std::max<uint64_t>(batch, 4096)) : (128u << 20) + (1u << 20);
@@ -161,6 +184,17 @@ int count_sharded(FILE* f, int k, int ranks, uint64_t distinct, double lf, bool 
     printf("Assembled %llu k-mers into %llu contigs with %llu nodes in %lf s; wrote %s_0.dat .. %s_%d.dat\n",
            (unsigned long long)n_total, (unsigned long long)nc, (unsigned long long)nodes,
            std::chrono::duration<double>(t3 - t2).count(), out_name.c_str(), out_name.c_str(), ranks - 1);
+    if (depth) {
+        uint64_t dk = 0, ds = 0;
+        for (int r = 0; r < ranks; ++r) {
+            const std::vector<char>& text = outs[r].text;                // one '\n'-terminated line per contig
+            std::vector<uint64_t> offs(1, 0);
+            for (size_t i = 0; i < text.size(); ++i)
+                if (text[i] == '\n') offs.push_back(i + 1);
+            write_depth(out_name + "_" + std::to_string(r) + ".depth", cluster.contig_depth(text.data(), offs.data(), offs.size() - 1), dk, ds);
+        }
+        report_depth(nc, dk, ds, out_name, ranks);
+    }
     return 0;
 }
 
@@ -172,13 +206,23 @@ int main(int argc, char** argv) {
     const std::string reads_file = argv[2];
     int a = 3;
     std::string histo;
-    if (std::string(argv[a]) == "--histo") {
-        if (++a >= argc) return usage();
-        histo = argv[a++];
+    bool depth = false;
+    while (a < argc) {                                                    // --histo and --depth, in either order
+        const std::string flag = argv[a];
+        if (flag == "--histo" && histo.empty()) {
+            if (++a >= argc) return usage();
+            histo = argv[a++];
+        } else if (flag == "--depth" && !depth) {
+            depth = true;
+            ++a;
+        } else {
+            break;
+        }
     }
     if (histo.empty() && a >= argc) return usage();
     const bool contigs = a < argc && std::string(argv[a]) == "--contigs";
     if (contigs && ++a >= argc) return usage();
+    if (depth && !contigs) return usage();
     const std::string out_name = a < argc ? argv[a++] : "";              // empty: --histo alone
     const bool auto_min_count = a < argc && std::string(argv[a]) == "auto";
     uint32_t min_count = a < argc ? (auto_min_count ? 0u : (uint32_t)atoi(argv[a])) : 2u;
@@ -198,7 +242,7 @@ int main(int argc, char** argv) {
     const int ranks = getenv("KH_RANKS") ? atoi(getenv("KH_RANKS")) : 1;
     if (ranks < 1 || ranks > 8) { fprintf(stderr, "kmer_count: KH_RANKS must be 1..8\n"); return 1; }
     if (ranks > 1 && contigs && (k < 17 || k > 54)) { fprintf(stderr, "kmer_count: --contigs with KH_RANKS > 1 needs 17 <= K <= 54\n"); return 1; }
-    if (ranks > 1) return count_sharded(f, k, ranks, distinct, lf, contigs, out_name, histo, auto_min_count, min_count, min_ext);
+    if (ranks > 1) return count_sharded(f, k, ranks, distinct, lf, contigs, out_name, histo, auto_min_count, min_count, min_ext, depth);
     const auto t0 = std::chrono::high_resolution_clock::now();
     kh::KmerCounter counter(k, distinct, lf, device);
 
@@ -240,6 +284,11 @@ int main(int argc, char** argv) {
     fclose(o);
     printf("Assembled %llu k-mers into %llu contigs with %llu nodes in %lf s; wrote %s\n", (unsigned long long)n,
            (unsigned long long)nc, (unsigned long long)nodes, std::chrono::duration<double>(t3 - t2).count(), dat.c_str());
+    if (depth) {
+        uint64_t dk = 0, ds = 0;
+        write_depth(out_name + "_0.depth", counter.contig_depth(text, offs, nc), dk, ds);
+        report_depth(nc, dk, ds, out_name, 1);
+    }
     kh_destroy(t);
     return 0;
 }
