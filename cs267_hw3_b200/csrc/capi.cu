@@ -76,7 +76,6 @@ struct kh_table {
         CtPeers pe = {};
         u32 epoch = 0;                    // barriers passed (all ranks call them in lockstep)
         u64 n_local_max = 0, n_total = 0, n_starts_max = 0, out_cap = 0;
-        u64 n_starts_host = 0;            // non-sharded handles learn it at every insert (they sync anyway)
         DevBuf xin_vals, xin_chunk, xin_cnt, xin_done, xout_cursor, extra_vals, extra_chunk, extra_cnt, fine, chunk_cursor,
                chunk_base, pool_off, seg_base, ext_key, meta, pool, inbox, inbox_cnt, out_cursor, flags,
                answers, req_seg, g_link, g_meta, g_pool, g_hdr;
@@ -190,6 +189,51 @@ static u64 group_cap(const kh_table* t, u64 n, u64 span, double slack) {
     return (u64)(share + 24.0 * std::sqrt(share + 1.0) + slack) * t->debug_cap_pct / 100;
 }
 
+// Tail of every insert call, both tables: scan the per-tile start counts the insert or staging kernel left, append the
+// call's start nodes to the start list in input order behind n_starts_dev, and raise that count.  A handle that may
+// block (every non-sharded one) reads the counters after the scan, reports input errors there and grows the list to
+// exactly the new count, which is then also the host's copy (t->n_starts); knowing it, the host stores it into
+// n_starts_dev behind the scatter.  A sharded handle must not block inside a step (see ct_setup): it writes into the
+// list kh_shard_init sized, bounded by hcap, ct_bump_starts_kernel adds the count on the device, and the host learns
+// it at ct_finish.
+template <int W>
+int register_starts(kh_table* t, const unsigned char* recs, u64 n, u64 ntiles) {
+    typedef typename Slot<W>::value_t V;
+    KH_TRY(device_scan(t, static_cast<u32*>(t->tile_counts.p), ntiles, static_cast<u64*>(t->tile_offs.p),
+                       &t->d_ctr->scan_total));
+    u64 hcap = t->ct.caps.hcap;
+    if (!t->ct.sharded) {
+        KH_TRY(read_counters(t));
+        const u32 e = t->h_ctr->errors;
+        if (e) {
+            clear_error_bits(t);
+            return status_from_errors(t, e);
+        }
+        if (t->h_ctr->scan_total == 0) return KH_OK;
+        hcap = t->n_starts + t->h_ctr->scan_total;
+        if (hcap > 0xFFFFFF00ull) return fail(t, KH_ERR_ARG, "more than 2^32-256 start nodes in one table");
+        KH_TRY(ensure(t, t->starts, hcap * sizeof(V), /*keep=*/true));
+        t->n_starts = hcap;
+    }
+    ct_scatter_starts_kernel<W><<<(unsigned)((ntiles * 32 + 255) / 256), 256, 0, t->stream>>>(
+        recs, n, t->k, static_cast<u32*>(t->mask.p), static_cast<u64*>(t->tile_offs.p), ntiles, static_cast<V*>(t->starts.p),
+        t->d_ctr, (u32)hcap);
+    KH_CUDA(t, cudaGetLastError());
+    ++t->n_launches;
+    if (!t->ct.sharded) {
+        // from the pinned mirror, which the copy reads when it runs: the next read_counters lands behind it on the stream,
+        // and kh_clear, the one host writer, enqueues its reset of the device counters behind it before it writes
+        t->h_ctr->n_starts_dev = hcap;
+        KH_CUDA(t, cudaMemcpyAsync(&t->d_ctr->n_starts_dev, &t->h_ctr->n_starts_dev, sizeof(u64), cudaMemcpyHostToDevice,
+                                   t->stream));
+    } else {
+        ct_bump_starts_kernel<<<1, 1, 0, t->stream>>>(t->d_ctr, (u32)hcap);
+        KH_CUDA(t, cudaGetLastError());
+        ++t->n_launches;
+    }
+    return KH_OK;
+}
+
 template <int W>
 int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool record_start) {
     typedef typename Slot<W>::value_t V;
@@ -282,25 +326,7 @@ int insert_device_impl(kh_table* t, const unsigned char* recs, u64 n, bool recor
     t->table_dirty = true;
     t->n_launches += !part ? 1 : (chunked ? 4 : 3);
     KH_CUDA(t, cudaGetLastError());
-    KH_TRY(device_scan(t, static_cast<u32*>(t->tile_counts.p), ntiles, static_cast<u64*>(t->tile_offs.p),
-                       &t->d_ctr->scan_total));
-    KH_TRY(read_counters(t));     // number of new start nodes (sizes the start list) + error bits
-    const u32 e = t->h_ctr->errors;
-    if (e) {
-        clear_error_bits(t);
-        return status_from_errors(t, e);
-    }
-    const u64 fresh = t->h_ctr->scan_total;
-    if (fresh) {
-        KH_TRY(ensure(t, t->starts, (t->n_starts + fresh) * sizeof(V), /*keep=*/true));
-        const u64 threads = ntiles * 32;
-        scatter_starts_kernel<W><<<(unsigned)((threads + 255) / 256), 256, 0, t->stream>>>(
-            recs, n, t->k, static_cast<u32*>(t->mask.p), static_cast<u64*>(t->tile_offs.p), ntiles,
-            static_cast<V*>(t->starts.p), t->n_starts);
-        KH_CUDA(t, cudaGetLastError());
-        t->n_starts += fresh;
-        ++t->n_launches;
-    }
+    KH_TRY(register_starts<W>(t, recs, n, ntiles));
     KH_CUDA(t, cudaEventRecord(t->ev[EV_INS1], t->stream));
     t->have_ins = true;
     return KH_OK;
@@ -389,8 +415,7 @@ int assemble_impl(kh_table* t) {
         wp.link, wp.seglen, wp.tmp, t->seg_chars, (u32)seg_cap, t->d_ctr, rp.contig_pre,
         static_cast<u64*>(t->contig_off.p), t->k, out_cap, static_cast<char*>(t->out.p));
     if (n_starts) {
-        const u64 head_threads = n_starts * (u64)(t->k + 1);
-        emit_heads_kernel<W><<<(unsigned)((head_threads + 255) / 256), 256, 0, t->stream>>>(
+        ct_emit_heads_kernel<W><<<(unsigned)t->sm_count * 8, 256, 0, t->stream>>>(
             static_cast<const V*>(t->starts.p), (u32)n_starts, t->k, rp.contig_len,
             static_cast<u64*>(t->contig_off.p), t->d_ctr, out_cap, static_cast<char*>(t->out.p));
     }
@@ -623,10 +648,6 @@ int ct_stage(kh_table* t, const unsigned char* recs, u64 n) {
         KH_TRY(ensure(t, t->mask, (ntiles + 1) * (kInsTile / 32) * sizeof(u32)));
         KH_TRY(ensure(t, t->tile_counts, (ntiles + 1) * sizeof(u32)));
         KH_TRY(ensure(t, t->tile_offs, (ntiles + 1) * sizeof(u64)));
-        KH_TRY(ensure(t, t->scan_blocks, ((ntiles + kScanTile - 1) / kScanTile + 2) * sizeof(u64)));
-        // the start list may have to hold every record of this call
-        KH_TRY(ensure(t, t->starts, (c.n_starts_host + n + 1) * sizeof(V), /*keep=*/true));
-        c.caps.hcap = (u32)std::min<u64>(0xFFFFFF00ull, c.n_starts_host + n + 1);        // bound for this call's start scatter only
     } else if (n > c.n_local_max) {
         return fail(t, KH_ERR_ARG, "more records than kh_shard_init reserved (n_local_max)");
     }
@@ -634,17 +655,12 @@ int ct_stage(kh_table* t, const unsigned char* recs, u64 n) {
         recs, n, c.g, c.pe, c.caps, static_cast<u32*>(c.chunk_cursor.p), static_cast<V*>(c.fine.p), static_cast<u32*>(c.xout_cursor.p),
         static_cast<u32*>(t->mask.p), static_cast<u32*>(t->tile_counts.p), t->d_ctr);
     KH_CUDA(t, cudaGetLastError());
-    KH_TRY(device_scan(t, static_cast<u32*>(t->tile_counts.p), ntiles, static_cast<u64*>(t->tile_offs.p), &t->d_ctr->scan_total));
-    ct_scatter_starts_kernel<W><<<(unsigned)((ntiles * 32 + 255) / 256), 256, 0, t->stream>>>(
-        recs, n, t->k, static_cast<u32*>(t->mask.p), static_cast<u64*>(t->tile_offs.p), ntiles, static_cast<V*>(t->starts.p),
-        t->d_ctr, c.caps.hcap);
-    ct_bump_starts_kernel<<<1, 1, 0, t->stream>>>(t->d_ctr, c.caps.hcap);
-    KH_CUDA(t, cudaGetLastError());
-    t->n_launches += 3;
-    KH_CUDA(t, cudaEventRecord(t->ev[EV_STAGE1], t->stream));
-    t->have_stage = true;
+    ++t->n_launches;
     c.sealed = false; c.assembled = false;
     t->table_dirty = true;
+    KH_TRY(register_starts<W>(t, recs, n, ntiles));
+    KH_CUDA(t, cudaEventRecord(t->ev[EV_STAGE1], t->stream));
+    t->have_stage = true;
     return KH_OK;
 }
 
@@ -681,7 +697,7 @@ int ct_seal_build(kh_table* t) {
     auto& c = t->ct;
     const u32 C = c.g.chunks_per_rank;
     if (!c.sharded) {                 // plain handle: the host knows the start count (every insert call synchronises)
-        const u64 hcap = c.n_starts_host + 1;
+        const u64 hcap = t->n_starts + 1;
         const u64 seg_cap = hcap + std::max<u64>(t->n_expected, 1) + 64;
         if (seg_cap >= 0xFFFFFF00ull) return fail(t, KH_ERR_ARG, "too many segments for 32-bit ids");
         c.caps.hcap = (u32)hcap; c.caps.seg_cap = (u32)seg_cap;
@@ -758,11 +774,11 @@ int ct_assemble_part(kh_table* t, int part) {
     case 1: {
         if (!c.sealed) { KH_TRY(ct_seal_build<W>(t)); KH_CUDA(t, cudaEventRecord(t->ev[EV_INS1], t->stream)); t->have_ins = true; }
         if (!c.sharded) {
-            const u64 hc = c.n_starts_host;
+            const u64 hc = t->n_starts;
             KH_TRY(ensure(t, t->contig_len, (hc + 3) * sizeof(u32)));
             KH_TRY(ensure(t, t->contig_pre, (hc + 3) * sizeof(u32)));
             KH_TRY(ensure(t, t->contig_off, (hc + 3) * sizeof(u64)));
-            c.out_cap = t->h_ctr->n_inserted + c.n_starts_host * (u64)(t->k + 1) + 64;       // n_inserted: refreshed by the seal's sync below
+            c.out_cap = t->h_ctr->n_inserted + hc * (u64)(t->k + 1) + 64;       // n_inserted: refreshed by the seal's sync below
             ct_set_self(t);
         }
         if (c.pe.world > 1) {             // meta words and characters are final: send them while the links are being resolved
@@ -851,7 +867,7 @@ int ct_assemble_part(kh_table* t, int part) {
         if (!c.slow) return KH_OK;
         ct_emit_kernel<<<gb, 256, 0, t->stream>>>(c.pe, link, static_cast<const u64*>(c.meta.p), static_cast<const unsigned char*>(c.pool.p),
                                                   c.caps, t->d_ctr, t->k);
-        ct_emit_heads_kernel<W><<<gb, 256, 0, t->stream>>>(static_cast<const V*>(t->starts.p), c.caps, t->k, static_cast<const u32*>(t->contig_len.p),
+        ct_emit_heads_kernel<W><<<gb, 256, 0, t->stream>>>(static_cast<const V*>(t->starts.p), c.caps.hcap, t->k, static_cast<const u32*>(t->contig_len.p),
                                                           static_cast<const u64*>(t->contig_off.p), t->d_ctr, c.out_cap, static_cast<char*>(t->out.p));
         KH_CUDA(t, cudaGetLastError());
         t->n_launches += 2;
@@ -905,16 +921,10 @@ int ct_finish(kh_table* t, u32* bits_out) {
 // plain-handle wrappers -----------------------------------------------------------------------------------------
 template <int W>
 int ct_insert_plain(kh_table* t, const unsigned char* recs, u64 n, bool record_start) {
-    auto& c = t->ct;
     if (record_start) KH_CUDA(t, cudaEventRecord(t->ev[EV_INS0], t->stream));
     KH_TRY(ct_stage<W>(t, recs, n));
-    KH_TRY(read_counters(t));                 // start count (sizes the start list of the next call) + input errors
-    c.n_starts_host = std::min<u64>(t->h_ctr->n_starts_dev, 0xFFFFFF00ull);
-    t->n_starts = c.n_starts_host;
     KH_CUDA(t, cudaEventRecord(t->ev[EV_INS1], t->stream));
     t->have_ins = true;
-    const u32 e = t->h_ctr->errors;
-    if (e) { clear_error_bits(t); return status_from_errors(t, e); }
     return KH_OK;
 }
 
@@ -936,7 +946,7 @@ int ct_assemble_plain(kh_table* t) {
     auto& c = t->ct;
     if (c.assembled) { c.sealed = false; c.assembled = false; }
     KH_TRY(ct_seal_plain<W>(t));              // also refreshes n_inserted on the host (sizes the output)
-    KH_TRY(ensure(t, t->out, t->h_ctr->n_inserted + c.n_starts_host * (u64)(t->k + 1) + 64));
+    KH_TRY(ensure(t, t->out, t->h_ctr->n_inserted + t->n_starts * (u64)(t->k + 1) + 64));
     for (int part = 0; part < kCtParts; ++part) KH_TRY(ct_assemble_part<W>(t, part));
     u32 bits = 0;
     KH_TRY(ct_finish(t, &bits));
@@ -1085,7 +1095,6 @@ int kh_clear(kh_table* t) {
     if (t->ct.on) {              // a chunk table is rewritten chunk by chunk at the next seal: only the staging cursors go back to zero
         KH_TRY(ct_reset_staging(t));
         t->ct.sealed = false; t->ct.assembled = false;
-        t->ct.n_starts_host = 0;
     } else {
         KH_CUDA(t, cudaMemsetAsync(t->table, 0, t->table_bytes, t->stream));
     }
@@ -1307,7 +1316,6 @@ int kh_get_stats(kh_table* t, kh_stats* out) {
     s.n_duplicates = t->h_ctr->n_duplicates;
     s.n_starts = t->n_starts;
     s.slot_bits = t->W == 1 ? 64 : 128;
-    if (t->ct.on) s.n_starts = std::min<u64>(t->h_ctr->n_starts_dev, 0xFFFFFFFFull);
     if (t->have_ins) s.ms_insert = elapsed(t->ev[EV_INS0], t->ev[EV_INS1]);
     if (t->have_as) {
         s.ms_assemble = elapsed(t->ev[EV_AS0], t->ev[EV_AS1]);
@@ -1619,7 +1627,7 @@ int kh_debug_buffer(kh_table* t, const char* name, void** ptr_out, uint64_t* byt
     if (n == "link") b = &t->link; else if (n == "meta") b = &c.meta; else if (n == "ext_key") b = &c.ext_key;
     else if (n == "chunk_base") b = &c.chunk_base; else if (n == "seg_base") b = &c.seg_base; else if (n == "chunk_cursor") b = &c.chunk_cursor;
     else if (n == "inbox_cnt") b = &c.inbox_cnt; else if (n == "out_cursor") b = &c.out_cursor; else if (n == "xin_cnt") b = &c.xin_cnt;
-    else if (n == "contig_len") b = &t->contig_len; else if (n == "pool") b = &c.pool;
+    else if (n == "contig_len") b = &t->contig_len; else if (n == "pool") b = &c.pool; else if (n == "starts") b = &t->starts;
     else if (n == "counters") { *ptr_out = t->d_ctr; *bytes_out = sizeof(Counters); return KH_OK; }
     else if (n == "caps") {          // host-side numbers: hcap, seg_cap, inbox_cap, cap_rs, chunks_per_rank, regions_per_rank
         static thread_local uint64_t v[8];

@@ -347,7 +347,8 @@ __global__ void ct_publish_xin_kernel(const CtPeers pe, const CtCaps caps, const
     if (d < pe.world && d != pe.rank) pe.xin_cnt[d][pe.rank] = min(xout_cursor[d], caps.xin_cap);
 }
 
-// start nodes seen so far live on the device (no host round trip per insert call in the sharded path)
+// start nodes seen so far live on the device (no host round trip per insert call in the sharded path); follows
+// ct_scatter_starts_kernel in a sharded insert (a non-sharded handle has read the count and stores it from the host)
 __global__ void ct_bump_starts_kernel(Counters* ctr, u32 hcap) {
     const u64 total = ctr->n_starts_dev + ctr->scan_total;
     if (total > hcap) { ct_internal(ctr, kSiteStarts); ctr->n_starts_dev = hcap; }
@@ -1265,15 +1266,16 @@ ct_emit_kernel(const CtPeers pe, const u64* __restrict__ link, const u64* __rest
     }
 }
 
-// first k-mer of each contig + '\n' (read_kmers.hpp:84, kmer_hash.cpp:66); n_starts read on the device
+// first k-mer of each contig + '\n' (read_kmers.hpp:84, kmer_hash.cpp:66); n_starts read on the device.
+// Both tables: the plain traverse writes its heads with it too.
 template <int W>
 __global__ void __launch_bounds__(256)
-ct_emit_heads_kernel(const typename Slot<W>::value_t* __restrict__ starts, const CtCaps caps, int k,
+ct_emit_heads_kernel(const typename Slot<W>::value_t* __restrict__ starts, u32 hcap, int k,
                      const u32* __restrict__ contig_len, const u64* __restrict__ contig_off,
                      const Counters* __restrict__ ctr, u64 out_cap, char* __restrict__ out) {
     typedef Slot<W> S;
     if (ctr->errors & (kErrConverge | kErrCycle | kErrInternal | kErrNotFound)) return;
-    const u32 n_starts = (u32)min(ctr->n_starts_dev, (u64)caps.hcap);
+    const u32 n_starts = (u32)min(ctr->n_starts_dev, (u64)hcap);
     const u64 total = (u64)n_starts * (u32)(k + 1);
     for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (u64)gridDim.x * blockDim.x) {
         const u64 c = t / (u32)(k + 1);
@@ -1287,7 +1289,9 @@ ct_emit_heads_kernel(const typename Slot<W>::value_t* __restrict__ starts, const
     }
 }
 
-// start list with the write position read from the device (ct path: no host round trip per insert call)
+// Start list in input order, one warp per insert tile (kInsTile records = 32 mask words), appended behind the
+// n_starts_dev already registered and bounded by hcap: the write position comes from the device, so a sharded step
+// needs no host round trip.  Both tables register their start nodes with it (register_starts in capi.cu).
 template <int W>
 __global__ void __launch_bounds__(256)
 ct_scatter_starts_kernel(const unsigned char* __restrict__ recs, u64 n, int k, const u32* __restrict__ start_mask,

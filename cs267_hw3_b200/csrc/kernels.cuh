@@ -5,11 +5,13 @@
 //                                                                         (hash_map.hpp:55-72, kmer_hash.cpp:27-31)
 //   K2p partition_kernel      records grouped by ~16 MB table region (+ start bitmask)
 //       insert_slots_kernel   grouped slot values -> table, CAS-first, region warm-up      (tables larger than L2)
-//   K3 scan_* / scatter_starts_kernel   start bitmask -> start list in file order           (kmer_hash.cpp:27-31)
+//   K3 scan_*                 per-tile start counts -> offsets; the start list itself is written by
+//                             ct_scatter_starts_kernel (ctable.cuh), shared with the chunk table  (kmer_hash.cpp:27-31)
 //   K4 find_kernel            batch lookup                                (hash_map.hpp:83-92)
 //   K5 walk_kernel            one lane per walk segment                   (kmer_hash.cpp:38-55, kmer_t.hpp:51-53)
 //      rank_kernel            pointer jumping over the segment list (cooperative launch)
-//   K6 emit_segments_kernel / emit_heads_kernel   contig text             (read_kmers.hpp:81-92)
+//   K6 emit_segments_kernel   contig text; the heads are written by ct_emit_heads_kernel (ctable.cuh)
+//                                                                         (read_kmers.hpp:81-92)
 //
 // All of it is HBM-bound integer work: no tensor cores, no floating point.  The multi-GPU path uses the chunk
 // table (ctable.cuh).
@@ -256,7 +258,7 @@ constexpr int kPartTile = kPartThreads * kPartPerThread;     // 2048 records per
 // capacity (no histogram pass: a partition's expected share is known from the uniform hash; space is
 // reserved with one atomicAdd per (block, partition); a record that does not fit -- never in practice
 // -- is inserted directly).  Also produces the start bitmask / per-tile start counts that
-// scatter_starts_kernel consumes (tiles of kInsTile records, identical to insert_kernel's).
+// ct_scatter_starts_kernel consumes (tiles of kInsTile records, identical to insert_kernel's).
 #ifndef KH_PART_MIN_BLOCKS
 #define KH_PART_MIN_BLOCKS 4
 #endif
@@ -710,43 +712,6 @@ scan_apply_kernel(const u32* __restrict__ in, u64 n, const u64* __restrict__ blo
 }
 
 // =========================================================================================
-// K3  start nodes: bitmask + per-tile offsets -> slot values in input order
-// =========================================================================================
-// One warp per insert tile (kInsTile records = 32 mask words).
-template <int W>
-__global__ void __launch_bounds__(256)
-scatter_starts_kernel(const unsigned char* __restrict__ recs, u64 n, int k,
-                      const u32* __restrict__ start_mask, const u64* __restrict__ tile_offsets, u64 ntiles,
-                      typename Slot<W>::value_t* __restrict__ starts_out, u64 out_base) {
-    typedef Slot<W> S;
-    const u64 tile = ((u64)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (tile >= ntiles) return;
-    const int pl = (k + 3) >> 2, pb = pl + 2;
-    const u64 word = tile * (kInsTile / 32) + lane_id();
-    const u64 nwords = (n + 31) >> 5;
-    u32 m = word < nwords ? start_mask[word] : 0u;
-    // exclusive prefix of popcounts across the warp
-    u32 inc = __popc(m);
-    const u32 mine = inc;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const u32 y = __shfl_up_sync(kFullMask, inc, d);
-        if (lane_id() >= (u32)d) inc += y;
-    }
-    u64 dst = out_base + tile_offsets[tile] + (inc - mine);
-    while (m) {
-        const int bit = __ffs(m) - 1;
-        m &= m - 1;
-        const u64 rec = (word << 5) + bit;
-        bool ok;
-        unsigned char tmp[18];
-        const unsigned char* src = recs + rec * pb;
-        for (int i = 0; i < pb; ++i) tmp[i] = src[i];
-        starts_out[dst++] = S::from_record(tmp, k, pl, ok);
-    }
-}
-
-// =========================================================================================
 // K4  lookup
 // =========================================================================================
 template <int W>
@@ -1093,24 +1058,6 @@ emit_segments_kernel(const u64* __restrict__ link, const unsigned char* __restri
         const unsigned char* src = tmp + (seg0 + src_lane) * (u64)seg_chars;
         for (u32 j = lane_id(); j < n; j += 32) out[d + j] = (char)src[j];
     }
-}
-
-// first k-mer of each contig + trailing newline (read_kmers.hpp:84, kmer_hash.cpp:66)
-template <int W>
-__global__ void __launch_bounds__(256)
-emit_heads_kernel(const typename Slot<W>::value_t* __restrict__ starts, u32 n_starts, int k,
-                  const u32* __restrict__ contig_len, const u64* __restrict__ contig_off,
-                  const Counters* __restrict__ ctr, u64 out_cap, char* __restrict__ out) {
-    typedef Slot<W> S;
-    if (ctr->contig_bytes > out_cap || (ctr->errors & (kErrConverge | kErrCycle | kErrInternal))) return;
-    const u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    const u64 c = t / (u32)(k + 1);
-    const u32 j = (u32)(t - c * (u32)(k + 1));
-    if (c >= n_starts) return;
-    const u32 len = contig_len[c];
-    if (len == 0) return;
-    if (j < (u32)k) out[contig_off[c] + j] = (char)ext_char(S::base_at(starts[c], k, (int)j));
-    else out[contig_off[c] + len - 1] = '\n';
 }
 
 // =========================================================================================

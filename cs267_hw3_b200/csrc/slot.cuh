@@ -475,7 +475,7 @@ struct Counters {
     u32 flags[40];
     u32 rank_done;        // ctable: no rank moved a link in the last pointer-jumping round (agreed on by all ranks)
     u32 err_where;        // ctable: which capacity / wait raised kErrInternal (CtSite bits), for the error message
-    u64 n_starts_dev;     // ctable: start nodes registered so far (kept on the device: no host round trip per insert)
+    u64 n_starts_dev;     // both tables: start nodes registered so far (kept on the device: no host round trip per insert)
     u32 need_jump;        // ctable: a contig of this rank is too long for the bounded walk
     u32 use_jump;         // ctable: some rank said so (agreed on at a barrier): rank by pointer jumping instead
 };

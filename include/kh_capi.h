@@ -326,7 +326,8 @@ int kh_count_contig_depth_device(kh_counter* c, const char* contigs_dev, const u
                                  uint32_t world, uint32_t rank, kh_contig_depth* out_dev);
 
 /* Introspection for tests and debugging: device pointer and capacity of an internal buffer of a chunk table
- * ("link", "meta", "chunk_base", "seg_base", "chunk_cursor", "counters", ...; "caps" returns HOST numbers). */
+ * ("link", "meta", "chunk_base", "seg_base", "chunk_cursor", "counters", ...; "caps" returns HOST numbers), or of
+ * either table's start list ("starts"). */
 int kh_debug_buffer(kh_table* t, const char* name, void** ptr_out, uint64_t* bytes_out);
 
 /* small device-memory helpers for hosts without their own CUDA binding */
