@@ -18,13 +18,13 @@ CLIS := $(addprefix kmer_hash_,$(KS))
 
 all: $(LIB) $(CLIS) kmer_count tools/gen_kmers tools/libkmergen.so
 
-$(LIB): $(CSRC) include/kh_capi.h
+$(LIB): $(CSRC) include/kh_capi.h include/kh/record_line.hpp
 	$(NVCC) $(NVCCFLAGS) -Xcompiler -fPIC -shared $(PKG)/csrc/capi.cu $(PKG)/csrc/count.cu -o $@
 
 kmer_hash_%: src/kmer_hash.cpp $(HDRS) $(LIB)
 	$(CXX) $(CXXFLAGS) -DKMER_LEN=$* -Iinclude $< -L$(PKG) -lkh_b200 -Wl,-rpath,$(abspath $(PKG)) -o $@
 
-kmer_count: src/kmer_count.cpp include/kh_capi.h include/kh/kmer_counter.hpp include/kh/sharded_counter.hpp include/kh/sharded_host.hpp $(LIB)
+kmer_count: src/kmer_count.cpp include/kh_capi.h include/kh/kmer_counter.hpp include/kh/sharded_counter.hpp include/kh/sharded_host.hpp include/kh/record_line.hpp $(LIB)
 	$(CXX) $(CXXFLAGS) -Iinclude $< -L$(PKG) -lkh_b200 -Wl,-rpath,$(abspath $(PKG)) -o $@
 
 tools/gen_kmers: tools/kmer_gen.cpp

@@ -38,7 +38,7 @@ ABI_SYMBOLS = [
     "kh_count_create", "kh_count_destroy", "kh_count_clear", "kh_count_reads", "kh_count_reads_device",
     "kh_count_extract", "kh_count_extract_device", "kh_count_extract_lines", "kh_count_lookup", "kh_count_get_stats", "kh_count_last_error",
     "kh_count_record_bytes", "kh_count_partition", "kh_count_merge_device", "kh_count_histogram", "kh_count_auto_min_count",
-    "kh_count_contig_depth", "kh_count_contig_depth_device",
+    "kh_count_contig_depth", "kh_count_contig_depth_device", "kh_count_link_check", "kh_count_link_check_device",
 ]
 
 
@@ -143,6 +143,8 @@ def lib() -> C.CDLL:
     L.kh_count_auto_min_count.restype = u32
     L.kh_count_contig_depth.argtypes = [vp, vp, vp, u64, u32, u32, vp]
     L.kh_count_contig_depth_device.argtypes = [vp, vp, vp, u64, u32, u32, vp]
+    L.kh_count_link_check.argtypes = [vp, vp, u64, u32, u32, u32, u32, pu64]
+    L.kh_count_link_check_device.argtypes = [vp, vp, vp, u64, u32, u32, u32, u32, pu64]
     _lib = L
     return L
 
@@ -414,6 +416,23 @@ class KmerCounter:
         """kh_count_contig_depth_device: contig text, n + 1 offsets and n 24-byte records, all in the counter's device
         memory (e.g. KmerHashTable.assemble_device's output).  Host-synchronous."""
         self._check(lib().kh_count_contig_depth_device(self._h, contigs_ptr, offsets_ptr, n, world, rank, out_ptr))
+
+    def link_check(self, pairs, min_count: int = 2, min_ext: int = 2, world: int = 1, rank: int = 0) -> tuple[np.ndarray, int]:
+        """Unitig extensions (kh_count_link_check): a copy of the kmer_pair records with every extension whose neighbour
+        is not reported at (min_count, min_ext) or does not name the k-mer back turned to 'F', and the number of sides
+        cut.  world > 1: only the sides whose neighbour owner `rank` owns."""
+        p = np.array(pairs, dtype=np.uint8, order="C").reshape(-1, pair_bytes(self.k))
+        n_cut = C.c_uint64()
+        self._check(lib().kh_count_link_check(self._h, p.ctypes.data, p.shape[0], min_count, min_ext, world, rank, C.byref(n_cut)))
+        return p, n_cut.value
+
+    def link_check_device(self, in_ptr: int, out_ptr: int, n: int, min_count: int = 2, min_ext: int = 2, world: int = 1,
+                          rank: int = 0) -> int:
+        """kh_count_link_check_device: n records from in_ptr, checked, to out_ptr (may equal in_ptr; either on any device,
+        e.g. extract_device's buffer).  Host-synchronous; returns the sides cut."""
+        n_cut = C.c_uint64()
+        self._check(lib().kh_count_link_check_device(self._h, in_ptr, out_ptr, n, min_count, min_ext, world, rank, C.byref(n_cut)))
+        return n_cut.value
 
     def stats(self) -> dict:
         s = CountStats()

@@ -33,7 +33,8 @@ def _stale(target: str, sources: list[str]) -> bool:
 
 
 def lib_sources() -> list[str]:
-    return [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(ROOT, "include", "kh_capi.h")]
+    return [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(ROOT, "include", "kh_capi.h"),
+                                                                      os.path.join(ROOT, "include", "kh", "record_line.hpp")]
 
 
 def build_lib(force: bool = False) -> str:
@@ -64,7 +65,7 @@ def build_count_cli(force: bool = False) -> str:
     build_lib()
     src = os.path.join(ROOT, "src", "kmer_count.cpp")
     hdrs = [os.path.join(ROOT, "include", "kh_capi.h")] + [os.path.join(ROOT, "include", "kh", f) for f in
-                                                            ("kmer_counter.hpp", "sharded_counter.hpp", "sharded_host.hpp")]
+                                                            ("kmer_counter.hpp", "sharded_counter.hpp", "sharded_host.hpp", "record_line.hpp")]
     out = os.path.join(ROOT, "kmer_count")
     if force or _stale(out, [src, LIB, *hdrs]):
         _run(["g++", "-O2", "-std=c++17", "-pthread", "-I" + os.path.join(ROOT, "include"), src,

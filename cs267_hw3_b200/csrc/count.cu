@@ -10,6 +10,8 @@
 //   kc_lookup_kernel   counters of given k-mers
 //   kc_histogram_kernel  table scan -> the k-mer spectrum (distinct k-mers per occurrence count)
 //   kc_depth_kernel    contig text -> per contig: windows, sum / min / max of their k-mers' occurrences (read-only)
+//   kc_link_kernel     kmer_pair records -> the same records with every extension whose neighbour does not name the k-mer
+//                      back turned to 'F' (unitig extensions; read-only on the table)
 //
 // HBM-bound integer work like the rest of the library: what an occurrence costs is one random 32-byte sector (the slot)
 // read and written back.  Algorithmic bytes per occurrence = 1 (the character) + 64.
@@ -319,6 +321,56 @@ __global__ void __launch_bounds__(256) kc_depth_init_kernel(KcDepth* __restrict_
         out[i] = KcDepth{0ull, 0ull, kKcDepthNoMin, 0u};
 }
 
+// Unitig extensions (kh_count_link_check*): one block per kKcLinkRecs records.  Records are K/4 + 2 = 3..18 bytes at
+// any alignment, so the block stages its byte range through shared memory -- aligned 32-bit loads in, one byte per
+// thread out, both coalesced -- and every thread checks kKcLinkPer records there (kc_link_plan, kc_find_pair with the
+// successor and predecessor lookups in flight together, kc_link_apply).  The table is only read.  `out` may be `in`: a
+// block reads its whole range before it writes any of it, and ranges of blocks are disjoint.  Cuts and malformed
+// records are summed per warp, one atomic each.
+struct KcLink {
+    u64 n_cut;
+    u32 bad, pad;
+};
+constexpr int kKcLinkThreads = 256;
+constexpr int kKcLinkPer = 4;
+constexpr u32 kKcLinkRecs = kKcLinkThreads * kKcLinkPer;
+constexpr u32 kKcLinkWords = (kKcLinkRecs * 18 + 3 + 3) / 4;          // the longest record (K = 61) + the first word's head
+
+template <int W>
+__global__ void __launch_bounds__(kKcLinkThreads)
+kc_link_kernel(const unsigned char* in, unsigned char* out, u64 n, const u64* __restrict__ table, u64 n_slots, int k, u32 min_count,
+               u32 min_ext, u32 world, u32 rank, KcLink* __restrict__ acc) {
+    __shared__ u32 s_w[kKcLinkWords];
+    const u64 pb = (u64)((k + 3) >> 2) + 2, first = (u64)blockIdx.x * kKcLinkRecs;
+    const u32 cnt = n - first < kKcLinkRecs ? (u32)(n - first) : kKcLinkRecs;
+    const u32 bytes = cnt * (u32)pb;
+    const unsigned char* src = in + first * pb;
+    const u32 head = (u32)(reinterpret_cast<uintptr_t>(src) & 3u);
+    const u32* words = reinterpret_cast<const u32*>(src - head);     // aligned words that hold a byte of the range
+    for (u32 i = threadIdx.x; i < (head + bytes + 3u) / 4u; i += kKcLinkThreads) s_w[i] = words[i];
+    __syncthreads();
+    unsigned char* s_b = reinterpret_cast<unsigned char*>(s_w) + head;
+    u32 cut = 0, bad = 0;
+#pragma unroll 1
+    for (u32 i = threadIdx.x; i < cnt; i += kKcLinkThreads) {
+        unsigned char* rec = s_b + i * (u32)pb;
+        const KcLinkPlan p = kc_link_plan(rec, k, world, rank);
+        u64 c[2];
+        kc_find_pair<W>(table, n_slots, p, c);
+        bad |= p.bad ? 1u : 0u;
+        cut += kc_link_apply(p, c, k, min_count, min_ext, rec);
+    }
+    __syncthreads();
+    unsigned char* dst = out + first * pb;
+    for (u32 j = threadIdx.x; j < bytes; j += kKcLinkThreads) dst[j] = s_b[j];
+    cut = __reduce_add_sync(kFull, cut);
+    bad = __reduce_or_sync(kFull, bad);
+    if ((threadIdx.x & 31u) == 0u) {
+        if (cut) atomicAdd(&acc->n_cut, (u64)cut);
+        if (bad) atomicOr(&acc->bad, 1u);
+    }
+}
+
 template <int W>
 __global__ void __launch_bounds__(256)
 kc_lookup_kernel(const u64* __restrict__ table, u64 n_slots, int k, const unsigned char* __restrict__ pkmers, u64 n, u32* __restrict__ counts_out) {
@@ -366,7 +418,7 @@ struct kh_counter {
     size_t scratch_cap = 0;
     void* outbox = nullptr;           // kh_count_partition: the slots grouped by owner
     size_t outbox_cap = 0;
-    void* inbox = nullptr;            // kh_count_merge_device: records copied over from another device
+    void* inbox = nullptr;            // kh_count_merge_device / kh_count_link_check*: records copied over from another device or the host
     size_t inbox_cap = 0;
     void* cursor = nullptr;           // kh_count_partition: per-owner counts / write cursors
     size_t cursor_cap = 0;
@@ -374,6 +426,8 @@ struct kh_counter {
     size_t hist_cap = 0;
     void* depth = nullptr;            // kh_count_contig_depth: records | offsets | contig text
     size_t depth_cap = 0;
+    void* link = nullptr;             // kh_count_link_check*: the KcLink sums
+    size_t link_cap = 0;
     u64 peers_enabled = 0;            // bit d: this counter's device reads device d's memory directly
     u64 n_bytes = 0;
     u32 n_launches = 0;
@@ -506,6 +560,74 @@ int kc_launch_depth(kh_counter* c, const unsigned char* seg, u64 span, u64 p_beg
     return KH_OK;
 }
 
+// Memory of any device of this process handed to a counter call: KH_ERR_ARG unless it is device (or managed) memory.
+// *foreign: it lives on another device; this counter's device then reads that device's memory peer to peer where the
+// two allow it (the copies below go through the host otherwise).
+int kc_device_memory(kh_counter* c, const void* p, const char* what, bool* foreign) {
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)) {
+        cudaGetLastError();
+        return kc_fail(c, KH_ERR_ARG, std::string(what) + " is not device memory");
+    }
+    *foreign = a.type == cudaMemoryTypeDevice && a.device != c->device;
+    if (*foreign && a.device >= 0 && a.device < 64 && !((c->peers_enabled >> a.device) & 1ull)) {
+        int can = 0;
+        if (cudaDeviceCanAccessPeer(&can, c->device, a.device) == cudaSuccess && can) {
+            const cudaError_t e = cudaDeviceEnablePeerAccess(a.device, 0);
+            if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) KC_CUDA(c, e);
+            cudaGetLastError();
+        }
+        c->peers_enabled |= 1ull << a.device;
+    }
+    return KH_OK;
+}
+
+// `bytes` at p, readable by this counter's kernels: p itself, or -- another GPU's memory -- one copy into the counter's
+// inbox, in stream order
+int kc_stage_in(kh_counter* c, const void* p, size_t bytes, const char* what, const void** local) {
+    bool foreign = false;
+    KC_TRY(kc_device_memory(c, p, what, &foreign));
+    *local = p;
+    if (!foreign) return KH_OK;
+    KC_TRY(kc_grow(c, &c->inbox, &c->inbox_cap, bytes));
+    KC_CUDA(c, cudaMemcpyAsync(c->inbox, p, bytes, cudaMemcpyDefault, c->stream));
+    *local = c->inbox;
+    return KH_OK;
+}
+
+int kc_link_check_args(kh_counter* c, bool null_arg, u64 n, u32 min_count, u32 min_ext, u32 world, u32 rank, uint64_t* n_cut_out,
+                       const char* what) {
+    if (!c || !n_cut_out) return KH_ERR_ARG;
+    *n_cut_out = 0;
+    if (min_count < 1 || min_count > kKcCountCap || min_ext < 1 || min_ext > kKcExtCap)
+        return kc_fail(c, KH_ERR_ARG, std::string(what) + ": 1 <= min_count <= 255 and 1 <= min_ext <= 127");
+    return kc_depth_check(c, null_arg, n, world, rank, what);
+}
+
+// kc_link_kernel over n records at `in` (this device) into `out` (this device; may be `in`); host waits, *n_cut = its sum
+int kc_launch_link(kh_counter* c, const void* in, void* out, u64 n, u32 min_count, u32 min_ext, u32 world, u32 rank, uint64_t* n_cut,
+                   const char* what) {
+    const u64 blocks = (n + kKcLinkRecs - 1) / kKcLinkRecs;
+    if (blocks > 0x7FFFFFFFull) return kc_fail(c, KH_ERR_ARG, std::string(what) + ": at most 2^41 records per call");
+    KC_TRY(kc_grow(c, &c->link, &c->link_cap, sizeof(KcLink)));
+    KcLink* acc = static_cast<KcLink*>(c->link);
+    KC_CUDA(c, cudaMemsetAsync(acc, 0, sizeof(KcLink), c->stream));
+    const unsigned char* i = static_cast<const unsigned char*>(in);
+    unsigned char* o = static_cast<unsigned char*>(out);
+    if (c->W == 1)
+        kc_link_kernel<1><<<(unsigned)blocks, kKcLinkThreads, 0, c->stream>>>(i, o, n, c->table, c->n_slots, c->k, min_count, min_ext, world, rank, acc);
+    else
+        kc_link_kernel<2><<<(unsigned)blocks, kKcLinkThreads, 0, c->stream>>>(i, o, n, c->table, c->n_slots, c->k, min_count, min_ext, world, rank, acc);
+    KC_CUDA(c, cudaGetLastError());
+    ++c->n_launches;
+    KcLink h{};
+    KC_CUDA(c, cudaMemcpyAsync(&h, acc, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (h.bad) return kc_fail(c, KH_ERR_BAD_INPUT, std::string(what) + ": an extension byte is not one of A C G T F");
+    *n_cut = h.n_cut;
+    return KH_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -559,7 +681,7 @@ int kh_count_destroy(kh_counter* c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     cudaFree(c->table); cudaFree(c->d_ctr); cudaFree(c->stage[0]); cudaFree(c->stage[1]); cudaFree(c->out); cudaFree(c->scratch);
-    cudaFree(c->outbox); cudaFree(c->inbox); cudaFree(c->cursor); cudaFree(c->hist); cudaFree(c->depth);
+    cudaFree(c->outbox); cudaFree(c->inbox); cudaFree(c->cursor); cudaFree(c->hist); cudaFree(c->depth); cudaFree(c->link);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     if (c->ev2) cudaEventDestroy(c->ev2);
@@ -760,28 +882,10 @@ int kh_count_merge_device(kh_counter* c, const void* records_dev, uint64_t n) {
     if (!c || (n && !records_dev)) return KH_ERR_ARG;
     if (n == 0) return KH_OK;
     KC_CUDA(c, cudaSetDevice(c->device));
-    cudaPointerAttributes a{};
-    if (cudaPointerGetAttributes(&a, records_dev) != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)) {
-        cudaGetLastError();
-        return kc_fail(c, KH_ERR_ARG, "kh_count_merge_device: records_dev is not device memory");
-    }
     const u64 rb = c->W == 1 ? 16 : 32;
-    const u64* src = static_cast<const u64*>(records_dev);
-    if (a.type == cudaMemoryTypeDevice && a.device != c->device) {
-        // another GPU's records: one copy into this counter's inbox, peer to peer where the devices allow it
-        if (a.device >= 0 && a.device < 64 && !((c->peers_enabled >> a.device) & 1ull)) {
-            int can = 0;
-            if (cudaDeviceCanAccessPeer(&can, c->device, a.device) == cudaSuccess && can) {
-                const cudaError_t e = cudaDeviceEnablePeerAccess(a.device, 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) KC_CUDA(c, e);
-                cudaGetLastError();
-            }
-            c->peers_enabled |= 1ull << a.device;
-        }
-        KC_TRY(kc_grow(c, &c->inbox, &c->inbox_cap, (size_t)(n * rb)));
-        KC_CUDA(c, cudaMemcpyAsync(c->inbox, records_dev, (size_t)(n * rb), cudaMemcpyDefault, c->stream));
-        src = static_cast<const u64*>(c->inbox);
-    }
+    const void* staged = nullptr;
+    KC_TRY(kc_stage_in(c, records_dev, (size_t)(n * rb), "kh_count_merge_device: records_dev", &staged));
+    const u64* src = static_cast<const u64*>(staged);
     for (u64 done = 0; done < n;) {                        // like kh_count_reads: every record may be a new k-mer
         u64 take = 0;
         KC_TRY(kc_reserve(c, n - done, &take));
@@ -862,6 +966,46 @@ int kh_count_contig_depth_device(kh_counter* c, const char* contigs_dev, const u
     const u64 span = ends[1] > ends[0] ? ends[1] - ends[0] : 0ull;
     return kc_launch_depth(c, reinterpret_cast<const unsigned char*>(contigs_dev) + ends[0], span, ends[0], reinterpret_cast<const u64*>(offsets_dev),
                            n_contigs, world, rank, reinterpret_cast<KcDepth*>(out_dev));
+}
+
+// Unitig extensions.  Host records: one copy to the counter's inbox, checked there in place, one copy back.
+int kh_count_link_check(kh_counter* c, void* pairs_host, uint64_t n, uint32_t min_count, uint32_t min_ext, uint32_t world, uint32_t rank,
+                        uint64_t* n_cut_out) {
+    KC_TRY(kc_link_check_args(c, !pairs_host, n, min_count, min_ext, world, rank, n_cut_out, "kh_count_link_check"));
+    if (n == 0) return KH_OK;
+    KC_CUDA(c, cudaSetDevice(c->device));
+    KC_TRY(kc_settle(c));                                   // a table that overflowed while counting is reported here
+    const size_t bytes = (size_t)n * (size_t)c->pb;
+    KC_TRY(kc_grow(c, &c->inbox, &c->inbox_cap, bytes));
+    KC_CUDA(c, cudaMemcpyAsync(c->inbox, pairs_host, bytes, cudaMemcpyHostToDevice, c->stream));
+    KC_TRY(kc_launch_link(c, c->inbox, c->inbox, n, min_count, min_ext, world, rank, n_cut_out, "kh_count_link_check"));
+    KC_CUDA(c, cudaMemcpyAsync(pairs_host, c->inbox, bytes, cudaMemcpyDeviceToHost, c->stream));
+    KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    return KH_OK;
+}
+
+// Device records on any device of the process: another device's input is staged into the inbox (kc_stage_in); output
+// for another device is written to the inbox and copied over.
+int kh_count_link_check_device(kh_counter* c, const void* pairs_in_dev, void* pairs_out_dev, uint64_t n, uint32_t min_count, uint32_t min_ext,
+                               uint32_t world, uint32_t rank, uint64_t* n_cut_out) {
+    static const char* what = "kh_count_link_check_device";
+    KC_TRY(kc_link_check_args(c, !pairs_in_dev || !pairs_out_dev, n, min_count, min_ext, world, rank, n_cut_out, what));
+    if (n == 0) return KH_OK;
+    KC_CUDA(c, cudaSetDevice(c->device));
+    KC_TRY(kc_settle(c));
+    const size_t bytes = (size_t)n * (size_t)c->pb;
+    bool out_foreign = false;
+    KC_TRY(kc_device_memory(c, pairs_out_dev, "kh_count_link_check_device: pairs_out", &out_foreign));
+    if (out_foreign) KC_TRY(kc_grow(c, &c->inbox, &c->inbox_cap, bytes));
+    const void* src = nullptr;
+    KC_TRY(kc_stage_in(c, pairs_in_dev, bytes, "kh_count_link_check_device: pairs_in", &src));
+    void* dst = out_foreign ? c->inbox : pairs_out_dev;
+    KC_TRY(kc_launch_link(c, src, dst, n, min_count, min_ext, world, rank, n_cut_out, what));
+    if (out_foreign) {
+        KC_CUDA(c, cudaMemcpyAsync(pairs_out_dev, dst, bytes, cudaMemcpyDefault, c->stream));
+        KC_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    return KH_OK;
 }
 
 int kh_count_lookup(kh_counter* c, const void* pkmers_host, uint64_t n, uint32_t* counts_host_out) {

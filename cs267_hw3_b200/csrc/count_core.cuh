@@ -493,15 +493,90 @@ __host__ __device__ __forceinline__ void kc_slot_record(const u64* table, u64 i,
     rec[pl + 1] = kc_pick(c, 36u, min_ext);
 }
 
-// a kmer_pair record as a line of the reference's k-mer file (read_kmers.hpp:64-76 parses exactly this): K bases, a
-// blank, the backward and the forward extension letter, '\n' -- K + 4 bytes
-__host__ __device__ __forceinline__ void kc_record_to_line(const unsigned char* rec, int k, unsigned char* line) {
+// ---- unitig extensions (kh_count_link_check*) --------------------------------------------------------------------
+// S = the k-mers the counter reports at (min_count, min_ext), each with its raw extensions (kc_pick at min_ext).  For a
+// record x = (s, b, f): f is kept iff f != 'F', y = s[1..K-1] f is in S and y's raw backward extension is s[0]; b is kept
+// iff b != 'F', w = b s[0..K-2] is in S and w's raw forward extension is s[K-1].  Otherwise the side becomes 'F'.  The rule
+// is symmetric (x -> y kept iff y <- x kept), so on checked records every k-mer has at most one successor and one
+// predecessor, each naming it back: paths (unitigs, one start each) and isolated cycles.  world > 1: only sides whose
+// neighbour `rank` owns (kc_owner) are looked at; the others stay as they are.  A cut only ever writes 'F', so the owners'
+// partials applied one after another in any order give the world = 1 records.
+//
+// Split in three so that the kernel can keep both lookups in flight: kc_link_plan (the record -> the neighbour keys to
+// look up), kc_find_pair (both lookups, probing side by side), kc_link_apply (the counter words -> the checked sides).
+struct KcLinkPlan {
+    u64 key_hi[2], key_lo[2];        // [0] = successor y, [1] = predecessor w
+    u32 want[2];                     // the base the neighbour must name back: s[0] (for y) and s[K-1] (for w)
+    bool look[2];                    // side not 'F' and owned by `rank`: the neighbour is looked up
+    bool bad;                        // an extension byte outside ACGTF
+};
+
+// the record's K-mer (rec: packed k-mer, backward, forward) -> the plan
+__host__ __device__ __forceinline__ KcLinkPlan kc_link_plan(const unsigned char* rec, int k, u32 world, u32 rank) {
+    const int pl = (k + 3) >> 2, kb = 2 * k;
+    u64 hi, lo;
+    kc_packed_to_key(rec, k, hi, lo);
+    const u32 b = ext_code(rec[pl]), f = ext_code(rec[pl + 1]);
+    KcLinkPlan p;
+    p.bad = b > kExtF || f > kExtF;
+    p.want[0] = kb - 2 >= 64 ? (u32)(hi >> (kb - 66)) & 3u : (u32)(lo >> (kb - 2)) & 3u;             // s[0]
+    p.want[1] = (u32)lo & 3u;                                                                           // s[K-1]
+    // y = ((s << 2) | f) mod 4^K
+    u64 yh = (hi << 2) | (lo >> 62), yl = (lo << 2) | (f & 3u);
+    if (kb <= 64) { yh = 0ull; yl &= kb == 64 ? ~0ull : (1ull << kb) - 1ull; }
+    else yh &= (1ull << (kb - 64)) - 1ull;
+    // w = (s >> 2) | b 4^(K-1)
+    u64 wh = hi >> 2, wl = (lo >> 2) | (hi << 62);
+    if (kb - 2 >= 64) wh |= (u64)(b & 3u) << (kb - 66);
+    else wl |= (u64)(b & 3u) << (kb - 2);
+    p.key_hi[0] = yh; p.key_lo[0] = yl;
+    p.key_hi[1] = wh; p.key_lo[1] = wl;
+    p.look[0] = !p.bad && f < kExtF && (world == 1 || kc_owner(yh, yl, world) == rank);
+    p.look[1] = !p.bad && b < kExtF && (world == 1 || kc_owner(wh, wl, world) == rank);
+    return p;
+}
+
+// kc_find for the keys the plan looks up (0 for the others), both probe sequences advanced side by side: the two slot
+// reads of one step are independent, so a thread has both in flight
+template <int W>
+__host__ __device__ __forceinline__ void kc_find_pair(const u64* table, u64 n_slots, const KcLinkPlan& p, u64 (&c)[2]) {
+    u64 t0[2], t1[2], s[2];
+    bool live[2];
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+        kc_tag<W>(p.key_hi[j], p.key_lo[j], t0[j], t1[j]);
+        s[j] = kc_home(p.key_hi[j], p.key_lo[j], n_slots);
+        live[j] = p.look[j];
+        c[j] = 0ull;
+    }
+    for (u64 tries = 0, lim = n_slots < kKcMaxProbes ? n_slots : kKcMaxProbes; tries < lim && (live[0] || live[1]); ++tries) {
+        u64 q[2][4];
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            const u64* a = table + (live[j] ? s[j] : 0ull) * (u64)KcSlot<W>::kWords;
+            q[j][0] = a[0]; q[j][1] = a[1]; q[j][2] = W == 1 ? 0ull : a[2]; q[j][3] = 0ull;
+        }
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            if (!live[j]) continue;
+            if (kc_slot_empty<W>(q[j])) live[j] = false;
+            else if (kc_slot_is<W>(q[j], t0[j], t1[j])) { c[j] = kc_slot_counters<W>(q[j]); live[j] = false; }
+            else s[j] = (s[j] + 1 == n_slots) ? 0ull : s[j] + 1;
+        }
+    }
+}
+
+// The checked sides written into rec (sides not looked up stay); returns the number of sides turned to 'F' (0..2)
+__host__ __device__ __forceinline__ u32 kc_link_apply(const KcLinkPlan& p, const u64 (&c)[2], int k, u32 min_count, u32 min_ext,
+                                                      unsigned char* rec) {
     const int pl = (k + 3) >> 2;
-    for (int i = 0; i < k; ++i) line[i] = ext_char((u32)(rec[i >> 2] >> (6 - 2 * (i & 3))) & 3u);      // packing.hpp:94-107 (unpackKmer)
-    line[k] = ' ';
-    line[k + 1] = rec[pl];
-    line[k + 2] = rec[pl + 1];
-    line[k + 3] = '\n';
+    u32 cut = 0;
+    // y must name s[0] backward; w must name s[K-1] forward
+    if (p.look[0] && !(kc_total(c[0]) >= min_count && kc_pick(c[0], 8u, min_ext) == ext_char(p.want[0]))) { rec[pl + 1] = 'F'; ++cut; }
+    if (p.look[1] && !(kc_total(c[1]) >= min_count && kc_pick(c[1], 36u, min_ext) == ext_char(p.want[1]))) { rec[pl] = 'F'; ++cut; }
+    return cut;
 }
 
 }  // namespace kh
+
+#include "../../include/kh/record_line.hpp"

@@ -150,6 +150,16 @@ class ShardedCounter:
     def extract_lines(self, rank: int, min_count: int = 2, min_ext: int = 2) -> np.ndarray:
         return self.owned[rank].extract_lines(min_count, min_ext)
 
+    def extract_unitigs(self, rank: int, min_count: int = 2, min_ext: int = 2) -> tuple[np.ndarray, int]:
+        """After reduce(): rank's records with unitig extensions (KmerCounter.link_check) and the sides cut.  Every owner,
+        starting at `rank`, checks the sides whose neighbour it owns; the partials give exactly the one-counter records."""
+        pairs, n_cut = self.owned[rank].extract(min_count, min_ext), 0
+        for i in range(self.world):
+            o = (rank + i) % self.world
+            pairs, cut = self.owned[o].link_check(pairs, min_count, min_ext, self.world, o)
+            n_cut += cut
+        return pairs, n_cut
+
     def histogram(self) -> np.ndarray:
         """After reduce(): the k-mer spectrum of everything reduced so far, uint64[256] (KmerCounter.histogram()).  Every
         k-mer has one owner and the owned counters equal one counter's, so the sum of the owners' spectra is exact."""

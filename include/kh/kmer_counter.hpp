@@ -14,8 +14,17 @@
 #include <vector>
 
 #include "../kh_capi.h"
+#include "record_line.hpp"
 
 namespace kh {
+
+// n kmer_pair records -> the reference's k-mer file text (K + 4 bytes per record, kc_record_to_line)
+inline std::string pair_lines(const unsigned char* recs, uint64_t n, int k) {
+    const uint64_t pb = kh_pair_bytes(k), ll = (uint64_t)k + 4;
+    std::string out(n * ll, '\0');
+    for (uint64_t i = 0; i < n; ++i) kc_record_to_line(recs + i * pb, k, reinterpret_cast<unsigned char*>(&out[i * ll]));
+    return out;
+}
 
 // Contig depth partials of disjoint window sets (one per owner of a sharded counter) -> the record over all of them
 inline void combine_depth(kh_contig_depth& into, const kh_contig_depth& part) {
@@ -86,6 +95,19 @@ class KmerCounter {
         std::vector<kh_contig_depth> out(n);
         check(kh_count_contig_depth(c_, text, offsets, n, 1, 0, out.data()), "contig_depth");
         return out;
+    }
+    // unitig extensions (kh_count_link_check*): extensions whose neighbour does not name the k-mer back become 'F';
+    // returns the sides cut.  Host records in place, or device records (any device; out may be in).
+    uint64_t link_check(std::vector<unsigned char>& pairs, uint32_t min_count = 2, uint32_t min_ext = 2, uint32_t world = 1, uint32_t rank = 0) {
+        uint64_t n_cut = 0;
+        check(kh_count_link_check(c_, pairs.data(), pairs.size() / kh_pair_bytes(k_), min_count, min_ext, world, rank, &n_cut), "link_check");
+        return n_cut;
+    }
+    uint64_t link_check_device(const void* in, void* out, uint64_t n, uint32_t min_count = 2, uint32_t min_ext = 2, uint32_t world = 1,
+                               uint32_t rank = 0) {
+        uint64_t n_cut = 0;
+        check(kh_count_link_check_device(c_, in, out, n, min_count, min_ext, world, rank, &n_cut), "link_check_device");
+        return n_cut;
     }
     kh_count_stats stats() {
         kh_count_stats s{};

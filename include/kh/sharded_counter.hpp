@@ -19,6 +19,8 @@
 #include <array>
 #include <cstdint>
 #include <exception>
+#include <memory>
+#include <mutex>
 #include <stdexcept>
 #include <string>
 #include <thread>
@@ -55,6 +57,9 @@ class CountCluster {
     std::vector<kh_counter*> batch_, owned_;
     std::vector<int> dev_;
     std::vector<uint64_t> occ_, bytes_;           // per rank: what earlier batches counted (before their clear)
+    std::vector<void*> unitigs_;                   // per rank: extract_unitigs_device's records, on device(rank)
+    std::vector<uint64_t> unitigs_cap_;
+    std::unique_ptr<std::mutex[]> owner_lock_;     // extract_unitigs*: one call at a time on each owned counter
 
     template <class F> void each_rank(F fn) {
         if (in_turn_ || world_ == 1) {
@@ -78,7 +83,8 @@ class CountCluster {
     // n_distinct_expected_total: distinct k-mers of all reads (erroneous ones included); both tables grow when short.
     // A batch table is sized for all of them (one rank's reads may hold nearly every k-mer), an owned table for its share.
     CountCluster(int k, int world, uint64_t n_distinct_expected_total, double load_factor = 0.5)
-        : k_(k), world_(world), batch_(world, nullptr), owned_(world, nullptr), dev_(world, 0), occ_(world, 0), bytes_(world, 0) {
+        : k_(k), world_(world), batch_(world, nullptr), owned_(world, nullptr), dev_(world, 0), occ_(world, 0), bytes_(world, 0),
+          unitigs_(world, nullptr), unitigs_cap_(world, 0), owner_lock_(new std::mutex[world]) {
         const int ndev = kh_device_count();
         if (ndev <= 0) throw std::runtime_error("CountCluster: no CUDA device (libkh_b200 has no CPU fallback)");
         if (world < 1 || world > 64) throw std::runtime_error("CountCluster: world must be between 1 and 64");
@@ -96,7 +102,7 @@ class CountCluster {
         }
     }
     ~CountCluster() {
-        for (int r = 0; r < world_; ++r) { kh_count_destroy(batch_[r]); kh_count_destroy(owned_[r]); }
+        for (int r = 0; r < world_; ++r) { kh_count_destroy(batch_[r]); kh_count_destroy(owned_[r]); kh_device_free(unitigs_[r]); }
     }
     CountCluster(const CountCluster&) = delete;
     CountCluster& operator=(const CountCluster&) = delete;
@@ -152,6 +158,64 @@ class CountCluster {
         std::string out(n * (uint64_t)(k_ + 4), '\0');
         count_must(kh_count_extract_lines(owned_[rank], min_count, min_ext, &out[0], n, &n), owned_[rank], "extract_lines");
         return out;
+    }
+
+    // After reduce(): rank's records with unitig extensions (kh_count_link_check*) -- rank's extract, checked by every
+    // owner for the sides whose neighbour it owns; the partials apply in any order and give the one-counter records.
+    // The device form leaves them in a buffer the cluster owns on device(rank), valid until the next call for this rank;
+    // the owners start at `rank` and go round, and the records cross devices 2 (P - 1) times (in and back for every other
+    // owner).  Calls for different ranks may run concurrently (each owner checks one rank's records at a time, and rotated
+    // starts keep them apart); calls for the same rank must not overlap.  n_cut: the sides turned to 'F'.
+    const void* extract_unitigs_device(int rank, uint32_t min_count, uint32_t min_ext, uint64_t& n, uint64_t& n_cut) {
+        n_cut = 0;
+        const void* p = nullptr;
+        {
+            std::lock_guard<std::mutex> g(owner_lock_[rank]);
+            count_must(kh_count_extract_device(owned_[rank], min_count, min_ext, &p, &n), owned_[rank], "extract_unitigs");
+            const uint64_t bytes = n * kh_pair_bytes(k_);
+            if (bytes > unitigs_cap_[rank]) {
+                kh_device_free(unitigs_[rank]);
+                unitigs_[rank] = nullptr;
+                unitigs_cap_[rank] = 0;
+                count_must(kh_device_alloc_on(dev_[rank], &unitigs_[rank], bytes), nullptr, "extract_unitigs: device buffer");
+                unitigs_cap_[rank] = bytes;
+            }
+            // the owner on rank's device checks first and moves the records out of its extract buffer as it goes
+            uint64_t cut = 0;
+            count_must(kh_count_link_check_device(owned_[rank], p, unitigs_[rank], n, min_count, min_ext, (uint32_t)world_, (uint32_t)rank, &cut),
+                       owned_[rank], "extract_unitigs");
+            n_cut += cut;
+        }
+        for (int i = 1; i < world_; ++i) {
+            const int o = (rank + i) % world_;
+            std::lock_guard<std::mutex> g(owner_lock_[o]);
+            uint64_t cut = 0;
+            count_must(kh_count_link_check_device(owned_[o], unitigs_[rank], unitigs_[rank], n, min_count, min_ext, (uint32_t)world_, (uint32_t)o, &cut),
+                       owned_[o], "extract_unitigs");
+            n_cut += cut;
+        }
+        return unitigs_[rank];
+    }
+    // the same records in host memory (kh_count_link_check per owner)
+    std::vector<unsigned char> extract_unitigs(int rank, uint32_t min_count, uint32_t min_ext, uint64_t& n_cut) {
+        n_cut = 0;
+        std::vector<unsigned char> recs;
+        uint64_t n = 0;
+        {
+            std::lock_guard<std::mutex> g(owner_lock_[rank]);
+            count_must(kh_count_extract(owned_[rank], min_count, min_ext, nullptr, 0, &n), owned_[rank], "extract_unitigs");
+            recs.resize(n * kh_pair_bytes(k_));
+            count_must(kh_count_extract(owned_[rank], min_count, min_ext, recs.data(), n, &n), owned_[rank], "extract_unitigs");
+        }
+        for (int i = 0; i < world_; ++i) {
+            const int o = (rank + i) % world_;
+            std::lock_guard<std::mutex> g(owner_lock_[o]);
+            uint64_t cut = 0;
+            count_must(kh_count_link_check(owned_[o], recs.data(), n, min_count, min_ext, (uint32_t)world_, (uint32_t)o, &cut), owned_[o],
+                       "extract_unitigs");
+            n_cut += cut;
+        }
+        return recs;
     }
 
     // After reduce(): the k-mer spectrum of everything reduced so far (kh_count_histogram).  Every k-mer has exactly one

@@ -324,6 +324,37 @@ int kh_count_contig_depth(kh_counter* c, const char* contigs_host, const uint64_
                           uint32_t world, uint32_t rank, kh_contig_depth* out_host);
 int kh_count_contig_depth_device(kh_counter* c, const char* contigs_dev, const uint64_t* offsets_dev, uint64_t n_contigs,
                                  uint32_t world, uint32_t rank, kh_contig_depth* out_dev);
+/* Unitig extensions: keep an extension only when the neighbouring k-mer names the k-mer back, so that the records
+ * satisfy the reference's input contract (README.md:33-35: linear chains, each entered at its one k-mer whose backward
+ * extension is 'F') on reads with repeats and errors too.
+ *   Let S be the k-mers this counter reports at (min_count, min_ext) and, for each of them, its extensions as
+ *   kh_count_extract* gives them at those thresholds (the raw ones, never the checked ones).  For a kmer_pair record x
+ *   with K-mer s, backward extension b and forward extension f:
+ *     forward side:  f is kept iff f != 'F', y = s[1..K-1] + f is in S, and y's backward extension is s[0];
+ *     backward side: b is kept iff b != 'F', w = b + s[0..K-2] is in S, and w's forward extension is s[K-1];
+ *   a side not kept becomes 'F'.  x itself need not be in S.  No reverse complements.
+ * The rule is symmetric (x -> y is kept iff y <- x is kept): on checked records every k-mer has at most one successor
+ * and one predecessor, each naming the other back, so the k-mers split into paths -- unitigs, each with exactly one start
+ * node -- and isolated cycles.  kh_assemble* and kh_shard_assemble then never return KH_ERR_NOT_FOUND or
+ * KH_ERR_CONVERGE on them, emit no k-mer twice, and place every record on a contig except k-mers on isolated cycles
+ * (which the reference never visits either).  On linear chains whose every k-mer is reported, nothing is cut.
+ * n records (kh_pair_bytes(k) each, any alignment) are written checked to pairs_out; *n_cut_out = the sides this call
+ * turned to 'F' (a side that was 'F' already does not count).
+ * world > 1: only sides whose neighbour k-mer owner `rank` owns (kc_owner, as kh_count_partition groups) are checked;
+ * the others are copied unchanged -- the partial of a sharded counter's owned counter `rank`.  Every neighbour has one
+ * owner and a cut only writes 'F', so the owners' calls applied one after another, in any order, give exactly the
+ * world = 1 records, and their n_cut values add up to its n_cut.  1 <= world <= 64, rank < world.
+ * kh_count_link_check_device: pairs_in / pairs_out may live on any device of the process; pairs_out equals pairs_in or
+ * does not overlap it; pairs_in may be the buffer kh_count_extract_device returned.  Records on another device than the
+ * counter's are staged through a counter-owned buffer (peer to peer where possible) and the result is copied back.
+ * kh_count_link_check: host records, checked in place.
+ * Both are host-synchronous and count one launch.  KH_ERR_ARG: null pointers (n > 0), min_count outside 1..255,
+ * min_ext outside 1..127, bad world / rank.  KH_ERR_BAD_INPUT: an extension byte outside ACGTF.  KH_ERR_TABLE_FULL
+ * after a count that overflowed the table.  n = 0: KH_OK, nothing launched. */
+int kh_count_link_check_device(kh_counter* c, const void* pairs_in_dev, void* pairs_out_dev, uint64_t n, uint32_t min_count,
+                               uint32_t min_ext, uint32_t world, uint32_t rank, uint64_t* n_cut_out);
+int kh_count_link_check(kh_counter* c, void* pairs_host, uint64_t n, uint32_t min_count, uint32_t min_ext, uint32_t world,
+                        uint32_t rank, uint64_t* n_cut_out);
 
 /* Introspection for tests and debugging: device pointer and capacity of an internal buffer of a chunk table
  * ("link", "meta", "chunk_base", "seg_base", "chunk_cursor", "counters", ...; "caps" returns HOST numbers), or of

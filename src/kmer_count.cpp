@@ -1,7 +1,7 @@
 // kmer_count -- reads -> the reference's k-mer file, or straight to contigs, on the B200 library.
 //
-//   kmer_count K reads_file [--histo HISTO_FILE] kmer_file_out   [min_count [min_ext]]
-//   kmer_count K reads_file [--histo HISTO_FILE] [--depth] --contigs PREFIX [min_count [min_ext]]
+//   kmer_count K reads_file [--histo HISTO_FILE] [--unitigs] kmer_file_out   [min_count [min_ext]]
+//   kmer_count K reads_file [--histo HISTO_FILE] [--depth] [--unitigs] --contigs PREFIX [min_count [min_ext]]
 //   kmer_count K reads_file --histo HISTO_FILE
 //
 // The first form writes what the reference's read_kmers parses (read_kmers.hpp:64-76: K bases, a blank, backward and
@@ -21,6 +21,11 @@
 // --depth (with --contigs only) writes PREFIX_r.depth next to every PREFIX_r.dat: line j describes line j of the .dat as
 // "n_kmers mean min max" -- the contig's k-mers, the mean (%.2f), least and largest of their occurrence counts in the
 // reads (kh_count_contig_depth; counts saturate at 255) -- and one more stdout line reports the overall mean.
+//
+// --unitigs checks the extracted records at the same thresholds before they are written or assembled: an extension is
+// kept only when the neighbour it names is reported and names the k-mer back (kh_count_link_check*), so on reads with
+// repeats and errors the k-mers form the linear chains the reference's traversal expects (README.md:33-35) and every
+// k-mer lands on exactly one contig (k-mers on isolated cycles excepted).  One more stdout line reports the cuts.
 // Environment: KH_DEVICE, KH_LOAD_FACTOR (0.5), KH_COUNT_DISTINCT = distinct k-mers to size the table for, erroneous
 // ones included (default: half the input bytes).
 //
@@ -53,8 +58,8 @@ void must(int status, kh_table* t, const char* what) {
 }
 
 int usage() {
-    fprintf(stderr, "Usage: kmer_count K reads_file [--histo HISTO_FILE] [--depth] [kmer_file_out | --contigs PREFIX] [min_count|auto [min_ext]]\n"
-                    "       (the output may be left out only with --histo; --depth needs --contigs)\n");
+    fprintf(stderr, "Usage: kmer_count K reads_file [--histo HISTO_FILE] [--depth] [--unitigs] [kmer_file_out | --contigs PREFIX] [min_count|auto [min_ext]]\n"
+                    "       (the output may be left out only with --histo and without --unitigs; --depth needs --contigs)\n");
     return 1;
 }
 
@@ -95,6 +100,11 @@ void report_depth(uint64_t n_contigs, uint64_t n_kmers, uint64_t sum, const std:
            (unsigned long long)n_kmers, n_kmers ? (double)sum / (double)n_kmers : 0.0, prefix.c_str(), prefix.c_str(), ranks - 1);
 }
 
+void report_unitigs(uint64_t n_cut, uint64_t n) {
+    printf("Unitig extensions: %llu of %llu k-mers' extensions set to F (neighbour not reported or not naming it back)\n",
+           (unsigned long long)n_cut, (unsigned long long)n);
+}
+
 // The file goes through in pieces of about `buffer` bytes that end on a line boundary (FASTA: before a header); each
 // piece's sequence lines (kh::sequence_lines) go to sink(text, n).
 template <class Sink> void read_pieces(FILE* f, size_t buffer, Sink sink) {
@@ -123,7 +133,7 @@ template <class Sink> void read_pieces(FILE* f, size_t buffer, Sink sink) {
 }
 
 int count_sharded(FILE* f, int k, int ranks, uint64_t distinct, double lf, bool contigs, const std::string& out_name,
-                  const std::string& histo, bool auto_min_count, uint32_t min_count, uint32_t min_ext, bool depth) {
+                  const std::string& histo, bool auto_min_count, uint32_t min_count, uint32_t min_ext, bool depth, bool unitigs) {
     using clock = std::chrono::high_resolution_clock;
     const uint64_t batch = getenv("KH_COUNT_BATCH_BYTES") ? strtoull(getenv("KH_COUNT_BATCH_BYTES"), nullptr, 10) : 0;
     const size_t buffer = batch ? (size_t)std::min<uint64_t>(128u << 20, std::max<uint64_t>(batch, 4096)) : (128u << 20) + (1u << 20);
@@ -148,22 +158,37 @@ int count_sharded(FILE* f, int k, int ranks, uint64_t distinct, double lf, bool 
     if (!contigs) {
         FILE* o = fopen(out_name.c_str(), "wb");
         if (o == nullptr) throw std::runtime_error("kmer_count: could not open " + out_name);
-        uint64_t lines = 0;
+        uint64_t lines = 0, cut = 0;
         for (int r = 0; r < ranks; ++r) {
-            const std::string text = cluster.extract_lines(r, min_count, min_ext);
+            std::string text;
+            if (unitigs) {
+                uint64_t c = 0;
+                const std::vector<unsigned char> recs = cluster.extract_unitigs(r, min_count, min_ext, c);
+                text = kh::pair_lines(recs.data(), recs.size() / kh_pair_bytes(k), k);
+                cut += c;
+            } else {
+                text = cluster.extract_lines(r, min_count, min_ext);
+            }
             if (fwrite(text.data(), 1, text.size(), o) != text.size()) throw std::runtime_error("kmer_count: short write to " + out_name);
             lines += text.size() / (size_t)(k + 4);
         }
         fclose(o);
+        if (unitigs) report_unitigs(cut, lines);
         printf("Wrote %llu k-mers (count >= %u, extensions seen >= %u times) to %s\n", (unsigned long long)lines, min_count,
                min_ext, out_name.c_str());
         return 0;
     }
     std::vector<const void*> recs(ranks);
     std::vector<uint64_t> n(ranks);
-    for (int r = 0; r < ranks; ++r) recs[r] = cluster.extract_device(r, min_count, min_ext, n[r]);
+    uint64_t cut = 0;
+    for (int r = 0; r < ranks; ++r) {
+        uint64_t c = 0;
+        recs[r] = unitigs ? cluster.extract_unitigs_device(r, min_count, min_ext, n[r], c) : cluster.extract_device(r, min_count, min_ext, n[r]);
+        cut += c;
+    }
     uint64_t n_local_max = 1, n_total = 0;
     for (uint64_t x : n) { n_local_max = std::max(n_local_max, x); n_total += x; }
+    if (unitigs) report_unitigs(cut, n_total);
     const auto t2 = clock::now();
     kh_sharded::Cluster tables(k, ranks, n_local_max, std::max<uint64_t>(n_total, 1), lf);
     tables.begin();
@@ -206,14 +231,17 @@ int main(int argc, char** argv) {
     const std::string reads_file = argv[2];
     int a = 3;
     std::string histo;
-    bool depth = false;
-    while (a < argc) {                                                    // --histo and --depth, in either order
+    bool depth = false, unitigs = false;
+    while (a < argc) {                                                    // --histo, --depth and --unitigs, in any order
         const std::string flag = argv[a];
         if (flag == "--histo" && histo.empty()) {
             if (++a >= argc) return usage();
             histo = argv[a++];
         } else if (flag == "--depth" && !depth) {
             depth = true;
+            ++a;
+        } else if (flag == "--unitigs" && !unitigs) {
+            unitigs = true;
             ++a;
         } else {
             break;
@@ -224,6 +252,7 @@ int main(int argc, char** argv) {
     if (contigs && ++a >= argc) return usage();
     if (depth && !contigs) return usage();
     const std::string out_name = a < argc ? argv[a++] : "";              // empty: --histo alone
+    if (unitigs && out_name.empty()) return usage();
     const bool auto_min_count = a < argc && std::string(argv[a]) == "auto";
     uint32_t min_count = a < argc ? (auto_min_count ? 0u : (uint32_t)atoi(argv[a])) : 2u;
     if (a < argc) ++a;
@@ -242,7 +271,7 @@ int main(int argc, char** argv) {
     const int ranks = getenv("KH_RANKS") ? atoi(getenv("KH_RANKS")) : 1;
     if (ranks < 1 || ranks > 8) { fprintf(stderr, "kmer_count: KH_RANKS must be 1..8\n"); return 1; }
     if (ranks > 1 && contigs && (k < 17 || k > 54)) { fprintf(stderr, "kmer_count: --contigs with KH_RANKS > 1 needs 17 <= K <= 54\n"); return 1; }
-    if (ranks > 1) return count_sharded(f, k, ranks, distinct, lf, contigs, out_name, histo, auto_min_count, min_count, min_ext, depth);
+    if (ranks > 1) return count_sharded(f, k, ranks, distinct, lf, contigs, out_name, histo, auto_min_count, min_count, min_ext, depth, unitigs);
     const auto t0 = std::chrono::high_resolution_clock::now();
     kh::KmerCounter counter(k, distinct, lf, device);
 
@@ -257,7 +286,15 @@ int main(int argc, char** argv) {
     if (out_name.empty()) return 0;
 
     if (!contigs) {
-        const std::string lines = counter.extract_lines(min_count, min_ext);
+        std::string lines;
+        if (unitigs) {
+            std::vector<unsigned char> recs = counter.extract(min_count, min_ext);
+            const uint64_t n = recs.size() / kh_pair_bytes(k);
+            report_unitigs(counter.link_check(recs, min_count, min_ext), n);
+            lines = kh::pair_lines(recs.data(), n, k);
+        } else {
+            lines = counter.extract_lines(min_count, min_ext);
+        }
         FILE* o = fopen(out_name.c_str(), "wb");
         if (o == nullptr) throw std::runtime_error("kmer_count: could not open " + out_name);
         if (fwrite(lines.data(), 1, lines.size(), o) != lines.size()) throw std::runtime_error("kmer_count: short write to " + out_name);
@@ -268,6 +305,8 @@ int main(int argc, char** argv) {
     }
     uint64_t n = 0;
     const void* recs = counter.extract_device(min_count, min_ext, n);
+    // checked in place: the records are the counter's own extract buffer
+    if (unitigs) report_unitigs(counter.link_check_device(recs, const_cast<void*>(recs), n, min_count, min_ext), n);
     kh_table* t = nullptr;
     must(kh_create(k, n ? n : 1, lf, device, &t), nullptr, "kh_create");
     const auto t2 = std::chrono::high_resolution_clock::now();
