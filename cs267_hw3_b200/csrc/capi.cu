@@ -134,7 +134,14 @@ int ensure_pinned(kh_table* t, void*& p, size_t& cap, size_t bytes) {
 int status_from_errors(kh_table* t, u32 e) {
     if (e == 0) return KH_OK;
     if (e & kErrBadInput) return fail(t, KH_ERR_BAD_INPUT, "input contains a base outside ACGT or an extension outside ACGTF");
-    if (e & kErrTableFull) return fail(t, KH_ERR_TABLE_FULL, "hash table is full (more distinct k-mers than slots)");
+    if (e & kErrTableFull) {
+        if (!(t->h_ctr->err_where & kSiteChunkFull)) return fail(t, KH_ERR_TABLE_FULL, "hash table is full (more distinct k-mers than slots)");
+        // a chunk holds every k-mer whose minimizer hashes to it: a repeat can crowd one chunk however large the table is
+        const unsigned cap = t->W == 1 ? CtBuild<1>::kMaxSlots : CtBuild<2>::kMaxSlots;
+        return fail(t, KH_ERR_TABLE_FULL, "hash table is full: a chunk of the table was offered more than " + std::to_string(cap) +
+                    " k-mers -- either more distinct k-mers than the table was sized for (n_expected), or more than " +
+                    std::to_string(cap) + " k-mers that share one minimizer (a repeat)");
+    }
     if (e & kErrNotFound) return fail(t, KH_ERR_NOT_FOUND, "Error: k-mer not found in Distributed HashMap.");
     if (e & kErrCycle) return fail(t, KH_ERR_CYCLE, "a start-rooted chain never reaches forward extension 'F' (cycle)");
     if (e & kErrConverge) return fail(t, KH_ERR_CONVERGE, "two start nodes reach the same end node (chains are not linear)");
@@ -149,6 +156,7 @@ int read_counters(kh_table* t) {
 }
 int clear_error_bits(kh_table* t) {
     KH_CUDA(t, cudaMemsetAsync(&t->d_ctr->errors, 0, sizeof(u32), t->stream));
+    KH_CUDA(t, cudaMemsetAsync(&t->d_ctr->err_where, 0, sizeof(u32), t->stream));
     return KH_OK;
 }
 
@@ -749,7 +757,7 @@ int ct_seal_build(kh_table* t) {
 //   7+R  (slow path only) emit | barrier
 constexpr int kCtMaxRounds = 24;            // chains of up to 2^24 segments
 constexpr int kCtParts = 8 + kCtMaxRounds;
-constexpr u32 kCtWalkMaxSteps = 512;        // segments a lane follows before the step falls back to pointer jumping
+constexpr u32 kCtWalkMaxSteps = 512;        // links a lane follows: a contig of more than 513 chunk segments falls back to pointer jumping
 
 template <int W>
 int ct_assemble_part(kh_table* t, int part) {
@@ -914,7 +922,7 @@ int ct_finish(kh_table* t, u32* bits_out) {
         t->err = msg;
         fprintf(stderr, "libkh_b200: %s\n", msg);
     }
-    if (h.errors) { clear_error_bits(t); KH_CUDA(t, cudaMemsetAsync(&t->d_ctr->err_where, 0, sizeof(u32), t->stream)); }
+    if (h.errors) clear_error_bits(t);
     return KH_OK;
 }
 

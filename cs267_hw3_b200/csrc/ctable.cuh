@@ -56,6 +56,10 @@ namespace kh {
 #ifndef KH_CT_JUMPS
 #define KH_CT_JUMPS 3
 #endif
+// Rounds of phase 4 that settle a chain of n + 1 nodes: the smallest R with (KH_CT_JUMPS + 1)^R >= n.  Between two
+// barriers a thread may see every other thread's (ancestor, distance) pair as it stood at the last barrier, so a round
+// of J passes multiplies a node's reach by J + 1 (not 2^J); only its own nodes' writes it sees at once.
+constexpr int ct_jump_rounds(u32 n, u64 reach = 1) { return reach >= n ? 0 : 1 + ct_jump_rounds(n, reach * (KH_CT_JUMPS + 1)); }
 template <int W> struct CtBuild {
     // A chunk = one run of buckets that a thread block builds in shared memory.  Shared memory per block:
     //   table | succ u16[node] (later the characters) | (ancestor, distance) u32[node] | ext code + flags u8[node] | pool offset u16[node]
@@ -67,8 +71,15 @@ template <int W> struct CtBuild {
     static constexpr u32 kOffOff = kOffPd + kMaxSlots * 4u;
     static constexpr u32 kOffCode = kOffOff + kMaxSlots * 2u;
     static constexpr u32 kSmem = kOffCode + kMaxSlots;
+    // pointer-jumping rounds of phase 4: enough for one chain through every record of a full chunk
+    static constexpr int kJumpRounds = ct_jump_rounds(kMaxSlots - 1);
 };
 constexpr int kCtBuildThreads = KH_CT_THREADS;
+static_assert(CtBuild<1>::kMaxSlots <= 0x8000u && CtBuild<2>::kMaxSlots <= 0x8000u, "node ids stay below kSuccExt");
+static_assert(CtBuild<1>::kMaxSlots <= 32u * kCtBuildThreads && CtBuild<2>::kMaxSlots <= 32u * kCtBuildThreads,
+              "phase 4 keeps a thread's unsettled nodes in one 32-bit mask");
+static_assert(KH_CT_JUMPS != 3 || (CtBuild<1>::kJumpRounds == 7 && CtBuild<2>::kJumpRounds == 7),
+              "4^7 >= 6143 > 4^6: seven rounds of three passes settle a chain through a full chunk of either slot width");
 // Where record number `at` of chunk `chunk` lives in the chunk buffers: position-major, in groups of one 128-byte
 // line (8 or 16 records).  All chunks fill at about the same rate, so at any moment the appends of the staging pass
 // land in a window of a few hundred MB instead of being spread over every chunk's own multi-KB buffer (3.7 GB in
@@ -288,7 +299,7 @@ ct_stage_kernel(const unsigned char* __restrict__ recs, u64 n, const CtGeom g, c
     for (int r = 0; r < kStgPer; ++r) {
         if (dst[r] == 0xFFFFFFFFu || own[r] != 0xFFFFFFFFu) continue;
         if (at[r] < kMaxSlots) fine[ct_fine_index<W>(dst[r], at[r], g.chunks_per_rank)] = v[r];
-        else err |= kErrTableFull;                     // more k-mers share this chunk than a chunk can hold
+        else { err |= kErrTableFull; atomicOr(&ctr->err_where, kSiteChunkFull); }      // more k-mers share this chunk than it can hold
     }
     err = __reduce_or_sync(kFullMask, err);
     if (lane_id() == 0 && err) atomicOr(&s_err, err);
@@ -375,7 +386,7 @@ ct_xin_scatter_kernel(const typename Slot<W>::value_t* __restrict__ xin_vals, co
             else err |= kErrTableFull;
         }
     }
-    if (err) atomicOr(&ctr->errors, err);
+    if (err) { atomicOr(&ctr->errors, err); atomicOr(&ctr->err_where, kSiteChunkFull); }
 }
 
 template <int W>
@@ -389,7 +400,7 @@ ct_extra_kernel(const typename Slot<W>::value_t* __restrict__ extra_vals, const 
         const u32 c = extra_chunk[i];
         const u32 at = atomicAdd(&chunk_cursor[c], 1u);
         if (at < kMaxSlots) fine[ct_fine_index<W>(c, at, nchunks)] = extra_vals[i];
-        else atomicOr(&ctr->errors, kErrTableFull);
+        else { atomicOr(&ctr->errors, kErrTableFull); atomicOr(&ctr->err_where, kSiteChunkFull); }
     }
 }
 
@@ -409,6 +420,7 @@ ct_layout_kernel(const u32* __restrict__ chunk_cursor, u32 nchunks, const CtGeom
     __shared__ u64 s_warp[33];
     constexpr u32 kPer = 8;                                       // consecutive chunks per thread: 8192 chunks per block-wide scan
     u64 carry_b = 0, carry_p = 0;
+    bool over = false;                                            // a chunk was offered more records than it holds
     for (u32 c0 = 0; c0 < nchunks; c0 += blockDim.x * kPer) {
         const u32 first = c0 + threadIdx.x * kPer;
         u32 capb[kPer], chars[kPer];
@@ -418,6 +430,7 @@ ct_layout_kernel(const u32* __restrict__ chunk_cursor, u32 nchunks, const CtGeom
             const u32 c = first + q;
             capb[q] = 0; chars[q] = 0;
             if (c < nchunks) {
+                over |= chunk_cursor[c] > max_slots;
                 const u32 load = min(chunk_cursor[c], max_slots);
                 if (load) {
                     const u64 want_slots = ((u64)load * g.lf_inv_q16 + 65535u) >> 16;
@@ -443,6 +456,7 @@ ct_layout_kernel(const u32* __restrict__ chunk_cursor, u32 nchunks, const CtGeom
         pool_off[nchunks] = (u32)carry_p;
         if (carry_b > caps.nbuckets_alloc || carry_p > caps.pool_cap) atomicOr(&ctr->errors, kErrTableFull);
     }
+    if (over) { atomicOr(&ctr->errors, kErrTableFull); atomicOr(&ctr->err_where, kSiteChunkFull); }
 }
 
 // ---- pass B: build a chunk in shared memory and contract its chains ------------------------------------------
@@ -713,9 +727,12 @@ ct_build_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u32* _
     }
     // ---- 4. pointer jumping in shared memory: every k-mer learns its segment head and its distance from it ----
     // In place: a stale read is still a valid (ancestor, distance) pair.  A root's low half is its segment index, which a
-    // child never adds (it stops as soon as its ancestor is a root).  Chains are <= ~40 k-mers: ~6 passes, KH_CT_JUMPS of
-    // them between two barriers; a cycle without a head (no chain enters it: kmer_hash.cpp never visits it) never settles
-    // and is cut off after 14+ passes.
+    // child never adds (it stops as soon as its ancestor is a root).  KH_CT_JUMPS passes run between two barriers; a
+    // pass may read other threads' pairs as they stood at the last barrier, so a round is only sure to multiply a
+    // node's reach by KH_CT_JUMPS + 1.  B::kJumpRounds rounds therefore settle a chain through every record of a full
+    // chunk (a repeat can put thousands of k-mers in one chain; random sequence gives <= ~40).  The loop leaves at the
+    // first barrier where nothing is unsettled, so only a cycle without a head (no chain enters it: kmer_hash.cpp never
+    // visits it) runs all the rounds; it never settles and phases 5 and 6 skip it.
     // A thread keeps a bit per node of its own that has not settled yet: later rounds only touch those.
     u32 active = 0;
 #pragma unroll 1
@@ -723,7 +740,7 @@ ct_build_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u32* _
         const u32 pd = s_pd[node];
         active |= ((pd >> 16) != node) ? (1u << i) : 0u;            // heads and dead nodes are roots already
     }
-    for (int round = 0; round < (14 + KH_CT_JUMPS - 1) / KH_CT_JUMPS; ++round) {
+    for (int round = 0; round < B::kJumpRounds; ++round) {
 #pragma unroll 1
         for (int rep = 0; rep < KH_CT_JUMPS; ++rep) {
 #pragma unroll 1
@@ -817,7 +834,7 @@ ct_build_kernel(const typename Slot<W>::value_t* __restrict__ fine, const u32* _
     if (threadIdx.x == 0) {
         if (s_inserted) atomicAdd(&ctr->n_inserted, (u64)s_inserted);
         if (s_dups) atomicAdd(&ctr->n_duplicates, (u64)s_dups);
-        if (s_err) atomicOr(&ctr->errors, s_err);
+        if (s_err) { atomicOr(&ctr->errors, s_err); atomicOr(&ctr->err_where, kSiteChunkFull); }      // the only build error: the chunk is full
     }
 }
 
@@ -1031,7 +1048,8 @@ ct_gather_kernel(const CtPeers pe, const CtCaps caps, const u64* __restrict__ li
 // ---- ranking by walking: one lane per contig follows its segments (kmer_hash.cpp:38-55, a segment per step) ----------
 // Contigs are short (~100 k-mers = 4..30 segments), there are hundreds of thousands of them, and every array the walk
 // reads is local (own arrays + gathered copies), so a lane per contig keeps the memory system busy with ONE read per
-// segment.  A contig of more than max_steps segments sets need_jump: the whole step then falls back to pointer jumping.
+// segment.  A lane counts the links it follows from the contig's first chunk segment, so a contig of more than
+// max_steps + 1 chunk segments (its head stub not counted) sets need_jump: the whole step then falls back to pointer jumping.
 struct CtGathered {
     const u64* link[kMaxRanks];
     const u64* meta[kMaxRanks];

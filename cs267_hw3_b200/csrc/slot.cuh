@@ -458,8 +458,10 @@ constexpr u32 kLinkUnused = 0xFFFFFFFEu;    // id never walked
 constexpr u32 kLinkClaimed = 0xFFFFFFFDu;   // tail claimed by a contig; low word = contig id
 constexpr u32 kLinkPending = 0xFFFFFFFCu;   // sharded walk: successor lives on another GPU, link not resolved yet
 
-// where a kErrInternal came from (Counters::err_where)
-enum : u32 { kSiteBarrier = 1u, kSiteStarts = 2u, kSiteSegCap = 4u, kSiteInbox = 8u, kSiteStubOpen = 16u, kSiteOutCap = 32u };
+// where a kErrInternal came from (Counters::err_where); kSiteChunkFull: a kErrTableFull came from a chunk of the chunk
+// table that was offered more than CtBuild<W>::kMaxSlots records
+enum : u32 { kSiteBarrier = 1u, kSiteStarts = 2u, kSiteSegCap = 4u, kSiteInbox = 8u, kSiteStubOpen = 16u, kSiteOutCap = 32u,
+             kSiteChunkFull = 64u };
 
 struct Counters {
     u32 next_walker;
@@ -474,7 +476,7 @@ struct Counters {
     u32 n_outbox;         // plain table, chunked build: records the chunks could not place (the overflow list)
     u32 flags[40];
     u32 rank_done;        // ctable: no rank moved a link in the last pointer-jumping round (agreed on by all ranks)
-    u32 err_where;        // ctable: which capacity / wait raised kErrInternal (CtSite bits), for the error message
+    u32 err_where;        // ctable: which capacity / wait raised kErrInternal or kErrTableFull (kSite* bits), for the error message
     u64 n_starts_dev;     // both tables: start nodes registered so far (kept on the device: no host round trip per insert)
     u32 need_jump;        // ctable: a contig of this rank is too long for the bounded walk
     u32 use_jump;         // ctable: some rank said so (agreed on at a barrier): rank by pointer jumping instead
