@@ -49,6 +49,7 @@ struct kh_table {
     bool table_dirty = false;         // something was inserted since create/clear
     bool chunk_attr_set = false;
     int debug_cap_pct = 100;          // KH_DEBUG_CAP_PCT: scale the grouping buffers' capacities (tests force the overflow paths)
+    u32 walk_steps = kCtWalkMaxSteps; // KH_DEBUG_WALK_STEPS: links the bounded contig walk follows (tests force pointer jumping)
     bool part_attr_set = false;
     Counters* d_ctr = nullptr;
     Counters* h_ctr = nullptr;
@@ -755,9 +756,9 @@ int ct_seal_build(kh_table* t) {
 //   6 .. 6+R-1  one pointer-jumping round each | barrier that also agrees on "nobody moved"
 //   6+R  (slow path only) contig lengths, claims, offsets | barrier
 //   7+R  (slow path only) emit | barrier
-constexpr int kCtMaxRounds = 24;            // chains of up to 2^24 segments
+// kCtMaxRounds (ctable.cuh): chains of up to 2^24 segments.  kCtWalkMaxSteps (ctable.cuh): links a lane follows, so a
+// contig of more than 513 chunk segments falls back to pointer jumping (KH_DEBUG_WALK_STEPS lowers it, see kh_create).
 constexpr int kCtParts = 8 + kCtMaxRounds;
-constexpr u32 kCtWalkMaxSteps = 512;        // links a lane follows: a contig of more than 513 chunk segments falls back to pointer jumping
 
 template <int W>
 int ct_assemble_part(kh_table* t, int part) {
@@ -831,7 +832,7 @@ int ct_assemble_part(kh_table* t, int part) {
         KH_CUDA(t, cudaEventRecord(t->ev[EV_WALK], t->stream));
         return ct_barrier(t);
     case 4:
-        ct_walk_len_kernel<<<gb, 256, 0, t->stream>>>(gt, link, c.caps, t->k, kCtWalkMaxSteps, static_cast<u32*>(t->contig_len.p), t->d_ctr);
+        ct_walk_len_kernel<<<gb, 256, 0, t->stream>>>(gt, link, c.caps, t->k, t->walk_steps, static_cast<u32*>(t->contig_len.p), t->d_ctr);
         KH_CUDA(t, cudaGetLastError());
         ++t->n_launches;
         return ct_barrier(t, -2);
@@ -1051,6 +1052,9 @@ int kh_create(int k, uint64_t n_expected, double load_factor, int device, kh_tab
     int v = env_int("KH_SPLIT_BUCKETS", 0);
     if (v > 0 && set_option(t, "split_buckets", v) != KH_OK) fprintf(stderr, "libkh_b200: ignoring KH_SPLIT_BUCKETS=%d\n", v);
     t->debug_cap_pct = std::max(1, env_int("KH_DEBUG_CAP_PCT", 100));
+    // 0 sends every step with a contig of two or more chunk segments to pointer jumping.  The ranks of a sharded step
+    // agree on the path at a barrier, so ranks with different values stay consistent.
+    t->walk_steps = (u32)std::min(std::max(env_int("KH_DEBUG_WALK_STEPS", (int)kCtWalkMaxSteps), 0), (int)kCtWalkMaxSteps);
     v = env_int("KH_SEG_CHARS", 0);
     if (v > 0 && set_option(t, "seg_chars", v) != KH_OK) fprintf(stderr, "libkh_b200: ignoring KH_SEG_CHARS=%d\n", v);
     if (use_ct) {

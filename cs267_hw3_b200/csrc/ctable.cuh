@@ -1050,6 +1050,8 @@ ct_gather_kernel(const CtPeers pe, const CtCaps caps, const u64* __restrict__ li
 // reads is local (own arrays + gathered copies), so a lane per contig keeps the memory system busy with ONE read per
 // segment.  A lane counts the links it follows from the contig's first chunk segment, so a contig of more than
 // max_steps + 1 chunk segments (its head stub not counted) sets need_jump: the whole step then falls back to pointer jumping.
+// max_steps is kCtWalkMaxSteps unless KH_DEBUG_WALK_STEPS lowers it (tests send ordinary inputs down the fallback).
+constexpr u32 kCtWalkMaxSteps = 512;
 struct CtGathered {
     const u64* link[kMaxRanks];
     const u64* meta[kMaxRanks];
@@ -1157,12 +1159,29 @@ ct_walk_emit_kernel(const CtGathered gt, const u64* __restrict__ link, const typ
 
 // ---- pointer jumping over segment lists that span GPUs --------------------------------------------------------------
 // A link is FINAL (top bit of the distance word) once its pointer is the chain's last segment (high word a marker);
-// a link that is not final always moves when it is visited, so "nothing moved here" means this rank's links are final
-// for good and it only keeps the others company at the barriers.  The rounds of all ranks run in lockstep (a barrier
+// a link that is not final moves when it is visited unless it is already saturated on a self-looping cycle segment,
+// so "nothing moved here" means this rank's links will never change again and it only keeps the others company at
+// the barriers.  The rounds of all ranks run in lockstep (a barrier
 // after each, ct_barrier_kernel): jumping over a peer's link doubles the distance only if the peer jumps too --
 // ranks that ran their rounds on their own would walk a chain one remote segment per round.
+constexpr int kCtMaxRounds = 24;            // pointer-jumping rounds of a traverse: chains of up to 2^24 segments
 __device__ __forceinline__ u64* ct_peer_link(const CtPeers& pe, u32 gid) { return pe.link[gid >> kRankShift] + (gid & kLocalMask); }
-__device__ __forceinline__ bool ct_is_end_marker(u32 hi) { return hi == kLinkTail || hi == kLinkClaimed || hi == kLinkMissing || hi == kLinkConverge; }
+__host__ __device__ __forceinline__ bool ct_is_end_marker(u32 hi) { return hi == kLinkTail || hi == kLinkClaimed || hi == kLinkMissing || hi == kLinkConverge; }
+
+// One jump of an open link li (pointer not a marker, not final) over the link lp of the segment it points at.
+// The distance saturates at kLinkDistMask: on a cycle it roughly doubles every round, and a sum that carried into the
+// final bit would make a cycle's link "final" with a meaningless distance (a start-rooted cycle was then refused as
+// KH_ERR_CONVERGE by the claim instead of KH_ERR_CYCLE).  A saturated link is never final, so ct_lengths_kernel
+// reports the cycle.  A chain that ends is exact as long as it has fewer than kLinkDistMask characters (contig
+// lengths are 32-bit anyway).  Returns li itself when the target is pending or unused: left open, ct_lengths reports it.
+__host__ __device__ __forceinline__ u64 ct_jump_link(u64 li, u64 lp) {
+    const u32 pp = (u32)(lp >> 32), sp = (u32)lp;
+    if (ct_is_end_marker(pp)) return li | kLinkFinalBit;
+    if (pp >= kLinkCtFirstMarker) return li;
+    const u32 d = ((u32)li & kLinkDistMask) + (sp & kLinkDistMask);      // < 2^32: no wrap
+    if (d >= kLinkDistMask) return ((u64)pp << 32) | kLinkDistMask;
+    return ((u64)pp << 32) | (d | (sp & kLinkFinalBit));
+}
 
 __global__ void __launch_bounds__(256)
 ct_rank_round_kernel(const CtPeers pe, u64* __restrict__ link, const CtCaps caps, Counters* ctr, u32* __restrict__ moved, int round) {
@@ -1175,11 +1194,10 @@ ct_rank_round_kernel(const CtPeers pe, u64* __restrict__ link, const CtCaps caps
         if (pi >= kLinkCtFirstMarker) continue;               // ends here / unused / still pending (reported by ct_lengths)
         if (si & kLinkFinalBit) continue;
         const u64 lp = __ldcg(ct_peer_link(pe, pi));
-        const u32 pp = (u32)(lp >> 32), sp = (u32)lp;
-        if (ct_is_end_marker(pp)) { __stcg(link + i, li | kLinkFinalBit); continue; }
-        if (pp >= kLinkCtFirstMarker) continue;               // pending / unused target: left open, ct_lengths reports it
-        __stcg(link + i, ((u64)pp << 32) | (u32)((si + (sp & kLinkDistMask)) | (sp & kLinkFinalBit)));
-        any = true;
+        const u64 ln = ct_jump_link(li, lp);
+        if (ln == li) continue;
+        __stcg(link + i, ln);
+        any |= (u32)(lp >> 32) < kLinkCtFirstMarker;          // jumped (a link that only turned final did not move)
     }
     if (__any_sync(kFullMask, any) && lane_id() == 0) moved[round] = 1;
 }
